@@ -2,7 +2,7 @@
 """Benchmark of the per-timestep implicit advection-diffusion step (BASELINE.json metric:
 cell-timesteps/sec, fp64; solver HBM GB/s vs peak).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload 1m16|ohio|ens64|16m] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload 1m16|ohio|ens64|16m] [--impl reference] [--dump-outputs DIR]
 
 A "step" = one ClearwaterRiverine.update(): LHS assembly, RHS, solve, store, mass flux for all K
 constituents on the workload's mesh.  One cell-timestep = one real cell advanced one step for one
@@ -23,6 +23,10 @@ The same JSON line carries the other BASELINE configurations under "extra" (boun
 linalg.py + csr_matrix + spsolve + _mass_flux (the reference package cannot be imported here: no
 xarray/h5py) on the 1M-cell mesh, ONE constituent (the reference solves constituents one after another:
 its rate in cell-timesteps/s does not depend on K), min(steps, 3) timed steps of ~50 s each.
+
+--dump-outputs DIR (GPU arm, one GPU): after the timed steps, what the last of them handed its caller -- the
+concentrations and the three mass-flux arrays of every constituent, on the cells and edges where they are defined --
+as DIR/<name>.npy (float64, see dump_outputs).  The inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -183,6 +187,43 @@ def measured_peak():
     return 6650.0, "B200_PROFILING.md fallback 6.65 TB/s (of fallback)"
 
 
+DUMP_STATE_BYTES, DUMP_FLUX_BYTES = 32 << 20, 24 << 20     # 56 MiB in all: under 64 MB whatever K is
+
+
+def dump_outputs(be, t: int, out_dir, f2, inputs) -> dict:
+    """Step t's results as its caller receives them, written to out_dir as float64 .npy files:
+      concentration                                  (K, cells)  c[t + 1] of the real cells
+      advection / diffusion / total_mass_flux        (K, edges)  the three per-edge mass-flux arrays of step t
+    The fluxes are kept on the edges where they are defined: between two real cells, and into ghost cells that hold a
+    boundary value (inputs (K, T, F) nonzero at t + 1) for every constituent.  Into any other ghost cell the flux is
+    NaN by definition, as in the reference (the ghost concentration is NaN).  The edges are chosen from the mesh and the
+    inputs alone, so a NaN on a kept edge is a defect of the build, not dropped.  Cells and edges beyond what fits
+    DUMP_STATE_BYTES / DUMP_FLUX_BYTES are sampled at fixed, seeded indices (sorted), so the same mesh and inputs
+    always give the same sample.  Returns {name: shape}."""
+    out_dir = Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    rng = np.random.default_rng(12345)
+
+    def sample(candidates, cap):
+        return np.sort(rng.choice(candidates, cap, replace=False)) if len(candidates) > cap else candidates
+
+    K = be.K
+    cells = sample(np.arange(be.n_real), DUMP_STATE_BYTES // (8 * K))
+    arrays = {"concentration": be.get_state_all(t + 1)[:, cells]}
+    if be.options.mass_flux:
+        f2 = np.asarray(f2)
+        defined = f2 < be.n_real
+        ghost = np.flatnonzero(~defined)
+        defined[ghost] = (np.asarray(inputs)[:, t + 1, f2[ghost]] != 0).all(axis=0)
+        edges = sample(np.flatnonzero(defined), DUMP_FLUX_BYTES // (3 * 8 * K))
+        flux = [be.get_mass_flux(k, t) for k in range(K)]
+        for i, name in enumerate(("advection_mass_flux", "diffusion_mass_flux", "total_mass_flux")):
+            arrays[name] = np.stack([f[i][edges] for f in flux])
+    for name, a in arrays.items():
+        np.save(out_dir / f"{name}.npy", np.ascontiguousarray(a, dtype=np.float64))
+    return {name: list(a.shape) for name, a in arrays.items()}
+
+
 def pinned(a: np.ndarray) -> np.ndarray:
     import torch
     return torch.from_numpy(np.ascontiguousarray(a)).pin_memory().numpy()
@@ -341,8 +382,9 @@ def precond_kernel_name(o):
 
 
 def gpu_workload(name, ctx, args, steps, warmup, profile_steps, opts, *, dd=False, want_roofline=True, want_e2e=False,
-                 want_clocks=True):
-    """One workload on the GPU(s): device-timed rate, per-kernel-family times, mass-balance scalars."""
+                 want_clocks=True, dump_dir=None):
+    """One workload on the GPU(s): device-timed rate, per-kernel-family times, mass-balance scalars; with dump_dir, the
+    outputs of the last timed step (dump_outputs)."""
     import torch
     import torch.distributed as dist
     from clearwater_riverine_b200 import TransportBackend, ensemble, synthetic
@@ -421,6 +463,8 @@ def gpu_workload(name, ctx, args, steps, warmup, profile_steps, opts, *, dd=Fals
                       "fallbacks_to_bicgstab": int(fallbacks), "worst_status": worst_status, "max_relres": worst_relres,
                       "strips": n_strips, "max_strip_neighbours": max_nbr},
            "clocks": clocks}
+    if dump_dir is not None:     # before the profiled steps below overwrite the device's mass fluxes
+        out["dumped_outputs"] = dump_outputs(be, W + K_steps - 1, dump_dir, plan.f2, inputs)
 
     # ---- per-kernel device time (CUDA events between launches on the handle's stream) -> roofline -------------
     roofline = None
@@ -604,7 +648,11 @@ def dd_small_parity(ctx, opts):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed steps of the headline workload (its rate, ms_per_step and --dump-outputs); two legs time fewer "
+                         "and report their own count: --impl reference min(steps, 3) (a SuperLU step of the 1M-cell mesh "
+                         "takes ~50 s) and the e2e contract leg min(steps, 8) (it keeps the (T, E) mass-flux history of all "
+                         "16 constituents in page-locked host memory, ~0.8 GB per step)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="1m16", choices=["1m16", "ohio", "ens64", "ensw", "16m"])
@@ -617,10 +665,16 @@ def main():
     ap.add_argument("--profile-steps", type=int, default=2)
     ap.add_argument("--opt", action="append", default=[], metavar="KEY=VALUE",
                     help="cwr_options override, e.g. --opt precond_steps=8 --opt rtol=1e-12")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step to DIR/<name>.npy (GPU arm, one GPU)")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and (args.impl != "b200" or world > 1):
+        ap.error("--dump-outputs applies to the GPU arm on one GPU")
     args.warmup = max(3, args.warmup) if args.impl == "b200" else args.warmup
 
     if args.impl == "reference":
@@ -644,7 +698,7 @@ def main():
 
     dd_main = args.workload == "16m" and world > 1
     head = gpu_workload(args.workload, ctx, args, args.steps, args.warmup, args.profile_steps, opts, dd=dd_main,
-                        want_e2e=not args.no_e2e and not dd_main)
+                        want_e2e=not args.no_e2e and not dd_main, dump_dir=args.dump_outputs)
 
     # ---- the other BASELINE configurations, bounded ------------------------------------------------------------
     extra = {}
@@ -707,6 +761,8 @@ def main():
             "extra": extra or None,
             "wall_seconds": time.perf_counter() - T_START,
         }
+        if "dumped_outputs" in head:
+            line["dumped_outputs"] = {"dir": str(args.dump_outputs), "arrays": head["dumped_outputs"]}
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
