@@ -102,6 +102,8 @@ def load_library():
         "cwr_mass_totals_at": ([H, C.c_int, C.c_int, C.c_int, C.POINTER(CwrMassTotals)], C.c_int),
         "cwr_get_flux_sums": ([H, C.c_int, dp, dp, dp], C.c_int),
         "cwr_get_volume_sums": ([H, dp, dp, dp], C.c_int),
+        "cwr_set_kinetics": ([H, dp, dp, dp, C.c_int, C.c_double], C.c_int),
+        "cwr_get_reaction_mass": ([H, C.c_int, dp], C.c_int),
         "cwr_get_lhs": ([H, C.POINTER(C.c_int64), ip, ip, dp], C.c_int),
         "cwr_get_rhs": ([H, C.c_int, dp], C.c_int),
         "cwr_get_permutation": ([H, ip], C.c_int),
@@ -405,6 +407,30 @@ class TransportBackend:
         m = CwrMassTotals()
         self._check(self._lib.cwr_mass_totals_at(self._h, k, t_start, t_end, C.byref(m)))
         return m
+
+    # -- kinetics --------------------------------------------------------------------------------
+    def set_kinetics(self, decay_per_day=None, theta=None, yields=None, temperature_k: int = -1, temperature_c: float = 20.0):
+        """First-order decay / transformations applied on the device in every later step (cwr_set_kinetics):
+        decay_per_day (K,) or None = off; theta (K,) or None = all 1; yields (K, K), yields[j, k] = mass of j formed per
+        mass of k decayed, or None; temperature_k = temperature constituent or -1 for the constant temperature_c (deg C).
+        An invalid set raises ValueError.  kinetics.compile_kinetics builds the arrays from a by-name spec."""
+        if decay_per_day is None:
+            self._check(self._lib.cwr_set_kinetics(self._h, None, None, None, -1, 20.0))
+            return
+        d = _arr(decay_per_day, np.float64, (self.K,), "decay_per_day")
+        th = None if theta is None else _arr(theta, np.float64, (self.K,), "theta")
+        y = None if yields is None else _arr(yields, np.float64, (self.K, self.K), "yields")
+        rc = self._lib.cwr_set_kinetics(self._h, _ptr(d, C.c_double), _ptr(th, C.c_double), _ptr(y, C.c_double),
+                                        int(temperature_k), float(temperature_c))
+        if rc == CWR_EINVAL:
+            raise ValueError(self._lib.cwr_last_error(self._h).decode())
+        self._check(rc)
+
+    def reaction_mass(self, k: int) -> float:
+        """Sum over the steps taken of sum_i V[t]_i (c~'_ik - c~_ik): the mass the reactions added to constituent k."""
+        out = C.c_double()
+        self._check(self._lib.cwr_get_reaction_mass(self._h, k, C.byref(out)))
+        return out.value
 
     # -- domain decomposition (one TransportBackend per GPU/process; see domain.py) -----------------------
     def dd_export(self) -> bytes:

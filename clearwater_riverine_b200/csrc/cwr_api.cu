@@ -110,6 +110,12 @@ struct cwr_handle {
     int lhs_step = -1;
     bool have_geometry = false;
     int64_t launches = 0, iterations = 0;
+    // first-order kinetics (cwr_set_kinetics): the reacting constituents in topological order and their yields; k_react runs
+    // in every step while kin_on.  The buffers are allocated by the first call and kept (the reaction mass is a running sum).
+    bool kin_on = false;
+    int kin_steps = 0, kin_temp_k = -1, kin_grid_max = 0;   // kin_grid_max: resident CTAs of k_react (partials sized for it)
+    double kin_temp_c = 20.0;
+    KinStep* d_kin_steps = nullptr; KinYield* d_kin_yields = nullptr; KinState* d_kin_state = nullptr; double* d_kin_partials = nullptr;
     // optional per-kernel-family timing with CUDA events on the handle's stream (bench.py roofline)
     bool profiling = false;
     std::vector<cudaEvent_t> ev_pool;
@@ -1316,15 +1322,25 @@ static int patch_real_cells(cwr_handle* h, int t, int before_solve) {
     return CWR_OK;
 }
 
-// b and the warm start x0 = c~ of step t (after the LHS: b is row-scaled by the diagonal), then x0's boundary rows to
-// the ranks that gather them
-static int build_rhs(cwr_handle* h, int t) {
+// b and the warm start x0 = c~ of step t (after the LHS: b is row-scaled by the diagonal), reacted when kinetics is set,
+// then x0's boundary rows to the ranks that gather them.  accumulate = 0 (the defect-correction fallback forms the same
+// right-hand side again): the step's reaction mass is not added a second time.
+static int build_rhs(cwr_handle* h, int t, int accumulate) {
     DeviceModel& M = h->M;
     mark(h, CWR_FAM_RHS);
     KC_DISPATCH(h->KC, (launch_chain(h, k_rhs<KC, VEC>, h->grid_rows, kThreads, 0, M)));
     h->launches += 1;
     int rc = patch_real_cells(h, t, 1);
     if (rc) return rc;
+    if (h->kin_on) {
+        // one CTA per tile of the rows this rank owns now (the ordering, and with it the row range, may still be rebuilt
+        // after cwr_set_kinetics), at most the resident grid; the same rows give the same grid, hence the same sums
+        const int R = react_tile_rows(h->K);
+        const int grid = grid_for((M.row_hi - M.row_lo + R - 1) / R, 1, h->kin_grid_max);
+        CK(launch_chain(h, k_react, grid, kThreads, react_smem_bytes(h->K), M, (const KinStep*)h->d_kin_steps, h->kin_steps,
+                        (const KinYield*)h->d_kin_yields, h->kin_temp_k, h->kin_temp_c, h->d_kin_partials, h->d_kin_state, accumulate));
+        h->launches += 1;
+    }
     if (M.b_hi - M.b_lo > 0) {
         CK(launch_chain(h, k_boundary_rhs, h->grid_b, kThreads, 0, M));
         h->launches += 1;
@@ -1371,7 +1387,7 @@ int cwr_step(cwr_handle* h, int t, cwr_step_info* info) {
     CK(launch_chain(h, k_assemble, grid_for(M.row_hi - M.row_lo, kThreads, h->max_grid), kThreads, 0, M));
     h->launches += 2 + (nb_own > 0);
     h->lhs_step = t;
-    { int rc = build_rhs(h, t); if (rc) return rc; }
+    { int rc = build_rhs(h, t, 1); if (rc) return rc; }
     cwr_step_info local{};
     int status;
     if (h->small_path) status = solve_small(h, &local);
@@ -1384,7 +1400,7 @@ int cwr_step(cwr_handle* h, int t, cwr_step_info* info) {
             const int cycles = h->h_ctl->iter, sweeps = h->h_ctl->sweeps_done;
             CK(cudaMemsetAsync(&M.ctl->all_done, 0, 2 * sizeof(int), h->stream));   // all_done, iter
             h->last_iters = 0;
-            { int rc = build_rhs(h, t); if (rc) return rc; }
+            { int rc = build_rhs(h, t, 0); if (rc) return rc; }
             status = solve(h, &local);
             local.restarts += 1 + cycles;
             local.sweeps = sweeps;
@@ -1667,6 +1683,94 @@ int cwr_get_volume_sums(cwr_handle* h, double* total_sum, double* in_sum, double
         std::fill(outs[w], outs[w] + h->E, 0.0);
         for (int g = 0; g < Eg; ++g) outs[w][h->topo.eperm[Ei + g]] = host[(size_t)w * Eg + g];
     }
+    return CWR_OK;
+}
+
+int cwr_set_kinetics(cwr_handle* h, const double* decay, const double* theta, const double* yields, int temperature_k,
+                     double temperature_c) {
+    if (!h) return CWR_EINVAL;
+    const int K = h->K;
+    if (!decay) { h->kin_on = false; return CWR_OK; }
+    for (int k = 0; k < K; ++k) {
+        if (!std::isfinite(decay[k]) || decay[k] < 0.0) FAIL(CWR_EINVAL, "cwr_set_kinetics: decay rates must be finite and >= 0");
+        if (theta && (!std::isfinite(theta[k]) || theta[k] <= 0.0)) FAIL(CWR_EINVAL, "cwr_set_kinetics: theta must be finite and > 0");
+    }
+    if (yields)
+        for (int j = 0; j < K; ++j)
+            for (int k = 0; k < K; ++k) {
+                const double y = yields[(size_t)j * K + k];
+                if (!std::isfinite(y)) FAIL(CWR_EINVAL, "cwr_set_kinetics: yields must be finite");
+                if (j == k && y != 0.0) FAIL(CWR_EINVAL, "cwr_set_kinetics: a constituent cannot yield itself");
+            }
+    if (temperature_k < -1 || temperature_k >= K) FAIL(CWR_EINVAL, "cwr_set_kinetics: temperature constituent out of range");
+    if (temperature_k < 0 && !std::isfinite(temperature_c)) FAIL(CWR_EINVAL, "cwr_set_kinetics: temperature must be finite");
+    if (temperature_k >= 0) {
+        if (decay[temperature_k] != 0.0) FAIL(CWR_EINVAL, "cwr_set_kinetics: the temperature constituent cannot decay");
+        for (int k = 0; yields && k < K; ++k)
+            if (yields[(size_t)temperature_k * K + k] != 0.0) FAIL(CWR_EINVAL, "cwr_set_kinetics: the temperature constituent cannot receive a yield");
+    }
+    // topological order of the yield graph (k -> j where yields[j, k] != 0), smallest index first among the ready ones
+    std::vector<int> indeg(K, 0), order;
+    for (int j = 0; yields && j < K; ++j)
+        for (int k = 0; k < K; ++k) indeg[j] += yields[(size_t)j * K + k] != 0.0;
+    std::vector<uint8_t> done(K, 0);
+    for (int round = 0; round < K; ++round) {
+        int k = 0;
+        while (k < K && (done[k] || indeg[k] != 0)) ++k;
+        if (k == K) FAIL(CWR_EINVAL, "cwr_set_kinetics: the yield graph has a cycle");
+        done[k] = 1;
+        order.push_back(k);
+        for (int j = 0; yields && j < K; ++j) indeg[j] -= yields[(size_t)j * K + k] != 0.0;
+    }
+    // a constituent that does not decay forms no loss (and so yields nothing): only the decaying ones are steps
+    std::vector<KinStep> steps;
+    std::vector<KinYield> ylist;
+    for (int k : order) {
+        if (decay[k] == 0.0) continue;
+        KinStep s{};
+        s.col = k; s.decay = decay[k]; s.log_theta = theta ? std::log(theta[k]) : 0.0;
+        s.y_begin = (int)ylist.size();
+        for (int j = 0; yields && j < K; ++j) {
+            const double y = yields[(size_t)j * K + k];
+            if (y != 0.0) { KinYield e{}; e.col = j; e.y = y; ylist.push_back(e); }
+        }
+        s.y_end = (int)ylist.size();
+        steps.push_back(s);
+    }
+    CK(cudaSetDevice(h->device));
+    if (!h->d_kin_state) {
+        cudaFuncAttributes fa{};
+        CK(cudaFuncGetAttributes(&fa, k_react));
+        if (fa.sharedSizeBytes > kReactStaticSmem) FAIL(CWR_ECUDA, "k_react: static shared memory exceeds what its tile sizing reserves");
+        int occ = 0;
+        CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_react, kThreads, react_smem_bytes(K)));
+        h->kin_grid_max = h->num_sms * std::max(1, occ);
+        CK(dalloc(h, &h->d_kin_steps, (size_t)K));
+        CK(dalloc(h, &h->d_kin_yields, (size_t)K * K));
+        CK(dalloc(h, &h->d_kin_partials, (size_t)K * h->kin_grid_max));
+        CK(dalloc(h, &h->d_kin_state, 1));
+        CK(cudaMemsetAsync(h->d_kin_state, 0, sizeof(KinState), h->stream));
+    }
+    // stream-ordered: steps queued before this call still read the previous parameters (pageable sources: the copies
+    // have left the host vectors when the calls return)
+    if (!steps.empty()) CK(cudaMemcpyAsync(h->d_kin_steps, steps.data(), steps.size() * sizeof(KinStep), cudaMemcpyHostToDevice, h->stream));
+    if (!ylist.empty()) CK(cudaMemcpyAsync(h->d_kin_yields, ylist.data(), ylist.size() * sizeof(KinYield), cudaMemcpyHostToDevice, h->stream));
+    h->kin_steps = (int)steps.size();
+    h->kin_temp_k = temperature_k;
+    h->kin_temp_c = temperature_k < 0 ? temperature_c : 20.0;
+    h->kin_on = true;
+    return CWR_OK;
+}
+
+int cwr_get_reaction_mass(cwr_handle* h, int k, double* total) {
+    if (!h) return CWR_EINVAL;
+    if (!total) FAIL(CWR_EINVAL, "NULL output");
+    if (k < 0 || k >= h->K) FAIL(CWR_EINVAL, "constituent index out of range");
+    *total = 0.0;
+    if (!h->d_kin_state) return CWR_OK;
+    CK(cudaSetDevice(h->device));
+    CK(cudaMemcpyAsync(total, &h->d_kin_state->mass[k], sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
     return CWR_OK;
 }
 

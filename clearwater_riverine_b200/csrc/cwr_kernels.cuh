@@ -530,6 +530,142 @@ __device__ __forceinline__ void grid_totals(const double* partials, double* tot,
 }
 
 // ---------------------------------------------------------------------------------------------
+// First-order kinetics (cwr_set_kinetics): after c~ is formed (k_rhs, k_patch_rows), every owned real row is reacted
+//   for the reacting constituents k in topological order of the yield graph:
+//     r = decay_k * theta_k^(T - 20) / 86400,  loss = c~_k * (-expm1(-r dt)),  c~_k -= loss,  c~_j += yield[j,k] * loss
+// and the load term b = (vol c~' / dt) / D is rewritten with k_rhs's expression (k_boundary_rhs, which runs afterwards,
+// reads the reacted c~'), so a zero rate leaves every bit as it was.  The step's reaction mass sum_i vol_i (c~'_ik - c~_ik)
+// is reduced per column without atomics: per-thread sums over a fixed set of rows, per-CTA partials, and the last CTA adds
+// them in block order (grid_totals).
+// ---------------------------------------------------------------------------------------------
+struct KinStep { int col, y_begin, y_end, pad; double decay, log_theta; };   // a reacting constituent; its yields
+struct KinYield { int col, pad; double y; };                                 // [y_begin, y_end)
+struct KinState { unsigned ticket; int pad; double mass[kMaxK]; };           // last-CTA ticket, running reaction mass
+
+// Shared memory of k_react: st[kMaxK] and last_block_arrives' flag (static, kReactStaticSmem bounds them), then the dynamic
+// part: a tile of R rows x (K + 1) doubles (odd stride: the one-row-per-thread chain is free of bank conflicts), vol and D
+// of its rows, fac[kMaxK] and red[kThreads].  R is the largest multiple of 32 (at most kThreads) that keeps the whole within
+// the 48 KB a kernel may use without opting in, for every K <= kMaxK.
+constexpr size_t kReactSmemLimit = 48 * 1024;
+constexpr size_t kReactStaticSmem = sizeof(KinStep) * kMaxK + 64;
+__host__ __device__ constexpr int react_tile_rows(int K) {
+    return (int)((kReactSmemLimit - kReactStaticSmem - (kMaxK + kThreads) * sizeof(double)) / ((K + 3) * sizeof(double))) >= kThreads
+               ? kThreads
+               : (int)((kReactSmemLimit - kReactStaticSmem - (kMaxK + kThreads) * sizeof(double)) / ((K + 3) * sizeof(double))) / 32 * 32;
+}
+__host__ __device__ constexpr size_t react_smem_bytes(int K) {
+    return (size_t)react_tile_rows(K) * (K + 1 + 2) * sizeof(double) + (size_t)(kMaxK + kThreads) * sizeof(double);
+}
+constexpr bool react_smem_fits_every_k() {
+    for (int K = 1; K <= kMaxK; ++K)
+        if (react_tile_rows(K) < 32 || react_smem_bytes(K) + kReactStaticSmem > kReactSmemLimit) return false;
+    return true;
+}
+static_assert(react_smem_fits_every_k(), "k_react's shared memory must fit in 48 KB for every K <= kMaxK");
+
+// f(e) for the elements [0, cnt) of a tile of the interleaved state that starts at `base`: each thread takes pairs that
+// are 16-byte aligned there, the unpaired element at either end is taken by one thread.  (A state slot starts at an odd
+// element when n K is odd.)
+template <typename F>
+__device__ __forceinline__ void react_pairs(const double* base, int cnt, F f) {
+    const int head = (int)((reinterpret_cast<uintptr_t>(base) >> 3) & 1);
+    const int pairs = (cnt - head) >> 1;
+    for (int q = threadIdx.x; q < pairs; q += blockDim.x) f(head + 2 * q, true);
+    if (threadIdx.x == 0) {
+        if (head && cnt > 0) f(0, false);
+        if (cnt > head && ((cnt - head) & 1)) f(cnt - 1, false);
+    }
+}
+
+__global__ void __launch_bounds__(kThreads) k_react(DeviceModel M, const KinStep* __restrict__ steps, int n_steps,
+                                                    const KinYield* __restrict__ yl, int temp_k, double temp_c,
+                                                    double* __restrict__ partials, KinState* __restrict__ ks, int accumulate) {
+    extern __shared__ double rs[];
+    __shared__ KinStep st[kMaxK];
+    pdl_enter();
+    const StepParams& sp = *M.sp;
+    const int K = M.K, ld = K + 1, R = react_tile_rows(K);
+    double* tile = rs;                        // [R][K + 1]: c~, then c~', then vol * (c~' - c~)
+    double* svol = tile + (size_t)R * ld;     // [R] vol[t] of the tile's rows
+    double* sdg = svol + R;                   // [R] D
+    double* fac = sdg + R;                    // [kMaxK] constant temperature: 1 - exp(-r dt) of every step
+    double* red = fac + kMaxK;                // [kThreads] column sums
+    const double dt = sp.dt;
+    for (int p = threadIdx.x; p < n_steps; p += blockDim.x) {
+        const KinStep s = steps[p];
+        st[p] = s;
+        if (temp_k < 0) fac[p] = -expm1(-(s.decay * exp((temp_c - 20.0) * s.log_theta) / 86400.0) * dt);
+    }
+    __syncthreads();
+    // column sums: thread (g, k) adds rows g, g + G, ... of every tile the CTA takes, in that order
+    const int G = kThreads / K, kc = threadIdx.x % K, g = threadIdx.x / K;
+    double acc = 0.0;
+    const int nrows = M.row_hi - M.row_lo;
+    double* __restrict__ x = sp.state_t1;
+    for (int r0 = blockIdx.x * R; r0 < nrows; r0 += gridDim.x * R) {
+        const int rows = min(R, nrows - r0), row0 = M.row_lo + r0, cnt = rows * K;
+        const size_t g0 = (size_t)row0 * K;
+        const bool b_aligned = ((reinterpret_cast<uintptr_t>(M.b + g0) ^ reinterpret_cast<uintptr_t>(x + g0)) & 15) == 0;
+        react_pairs(x + g0, cnt, [&](int e, bool pair) {
+            const int r = e / K, k = e - r * K;
+            if (pair) {
+                const double2 v = *reinterpret_cast<const double2*>(x + g0 + e);
+                tile[r * ld + k] = v.x;
+                const int r1 = (e + 1) / K, k1 = e + 1 - r1 * K;
+                tile[r1 * ld + k1] = v.y;
+            } else tile[r * ld + k] = x[g0 + e];
+        });
+        for (int r = threadIdx.x; r < rows; r += blockDim.x) { svol[r] = (double)sp.vol_t[row0 + r]; sdg[r] = M.diag[row0 + r]; }
+        __syncthreads();
+        if (threadIdx.x < rows) {             // one row's chain per thread
+            double* c = tile + threadIdx.x * ld;
+            const double T = temp_k < 0 ? temp_c : c[temp_k];
+            for (int p = 0; p < n_steps; ++p) {
+                const KinStep& s = st[p];
+                const double f = temp_k < 0 ? fac[p] : -expm1(-(s.decay * exp((T - 20.0) * s.log_theta) / 86400.0) * dt);
+                const double loss = c[s.col] * f;
+                c[s.col] -= loss;
+                for (int q = s.y_begin; q < s.y_end; ++q) {
+                    const KinYield y = yl[q];
+                    c[y.col] += y.y * loss;
+                }
+            }
+        }
+        __syncthreads();
+        // c~' and b = (vol c~' / dt) / D out (k_rhs's expression); the tile keeps vol * (c~' - c~) (c~ re-read from L2)
+        react_pairs(x + g0, cnt, [&](int e, bool pair) {
+            double nv[2], bb[2];
+            const int m = pair ? 2 : 1;
+            for (int u = 0; u < m; ++u) {
+                const int r = (e + u) / K, k = e + u - r * K;
+                const double v = tile[r * ld + k], vol = svol[r];
+                nv[u] = v;
+                bb[u] = (vol * v / dt) / sdg[r];
+                tile[r * ld + k] = vol * (v - x[g0 + e + u]);
+            }
+            if (pair) *reinterpret_cast<double2*>(x + g0 + e) = make_double2(nv[0], nv[1]);
+            else x[g0 + e] = nv[0];
+            if (pair && b_aligned) *reinterpret_cast<double2*>(M.b + g0 + e) = make_double2(bb[0], bb[1]);
+            else for (int u = 0; u < m; ++u) M.b[g0 + e + u] = bb[u];
+        });
+        __syncthreads();
+        if (g < G)
+            for (int r = g; r < rows; r += G) acc += tile[r * ld + kc];
+        __syncthreads();
+    }
+    red[threadIdx.x] = acc;
+    __syncthreads();
+    if (threadIdx.x < K) {
+        double s = 0.0;
+        for (int q = 0; q < G; ++q) s += red[q * K + threadIdx.x];
+        partials[(size_t)threadIdx.x * gridDim.x + blockIdx.x] = s;
+    }
+    if (!last_block_arrives(&ks->ticket)) return;
+    grid_totals<1>(partials, red, K);
+    if (accumulate && threadIdx.x < K) ks->mass[threadIdx.x] += red[threadIdx.x];
+}
+
+// ---------------------------------------------------------------------------------------------
 // Domain decomposition over NVLink: one process per GPU, every rank holds the whole mesh's index space
 // (global row numbers everywhere) but computes only its rows [row_lo, row_hi).  The vectors other
 // ranks gather from (p^, s^, x) live in a symmetric slab that every rank maps from every peer (CUDA

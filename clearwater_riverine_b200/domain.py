@@ -79,3 +79,8 @@ class DomainDecomposedBackend(TransportBackend):
         m = self.mass_totals(k, t_start, t_end)
         v = merge_owned(np.array([m.vol_start, m.mass_start, m.vol_end, m.mass_end]), np.ones(4, bool), group=self.group)
         return tuple(float(x) for x in v)
+
+    def gather_reaction_mass(self, k: int) -> float:
+        """Reaction mass of constituent k over the whole mesh: the sum of the ranks' partial sums."""
+        v = merge_owned(np.array([self.reaction_mass(k)]), np.ones(1, bool), group=self.group)
+        return float(v[0])

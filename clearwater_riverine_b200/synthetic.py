@@ -296,3 +296,29 @@ def ohio_like(n_time: int = 913, seed: int = 2) -> SyntheticPlan:
 def square_mesh(n_side: int, n_time: int, seed: int, **kw) -> SyntheticPlan:
     kw.setdefault("tri_fraction", 0.1)
     return make_plan(n_side, n_side, n_time, seed=seed, **kw)
+
+
+def make_kinetics(inputs: np.ndarray, *, seed: int = 0, decay_range=(20.0, 200.0)):
+    """A seeded first-order network over the K constituents of `inputs` ((K,T,F), make_inputs): every constituent
+    decays (decay_range in 1/day, theta in 1.02..1.08) and constituent k yields to k + 1 with +0.8 for even k and -0.4 for
+    odd k (a chain with negative yields).  K >= 4: the last constituent is the temperature instead (its values rescaled to
+    10..30 deg C; it neither decays nor receives); K < 4: a constant 24 deg C (13 deg C for K = 1).
+    Returns (inputs', dict of TransportBackend.set_kinetics arguments)."""
+    rng = np.random.default_rng(seed + 104729)
+    inputs = np.array(inputs, dtype=np.float64, copy=True)
+    K = inputs.shape[0]
+    temperature_k = K - 1 if K >= 4 else -1
+    n_react = K - 1 if temperature_k >= 0 else K
+    lo, hi = decay_range
+    decay = np.zeros(K)
+    decay[:n_react] = lo + (hi - lo) * rng.random(n_react)
+    theta = np.ones(K)
+    theta[:n_react] = 1.02 + 0.06 * rng.random(n_react)
+    yields = np.zeros((K, K))
+    for k in range(n_react - 1):
+        yields[k + 1, k] = 0.8 if k % 2 == 0 else -0.4
+    if temperature_k >= 0:
+        a = inputs[temperature_k]
+        inputs[temperature_k] = np.where(a != 0, 10.0 + 0.2 * a, 0.0)
+    return inputs, dict(decay_per_day=decay, theta=theta, yields=yields, temperature_k=temperature_k,
+                        temperature_c=13.0 if K == 1 else 24.0)

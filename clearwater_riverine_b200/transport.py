@@ -91,6 +91,8 @@ class ClearwaterRiverine:
         verbose: Optional[bool] = False,
         datetime_range: Optional[Tuple[int, int]] = None,
         mesh_file_path: Optional[str | Path] = None,
+        kinetics: Optional[Dict[str, Dict[str, Any]]] = None,
+        temperature: Optional[str | float] = None,
         **backend_options,
     ) -> None:
         from .io import ras
@@ -108,6 +110,11 @@ class ClearwaterRiverine:
             if not flow_field_file_path:
                 flow_field_file_path = cfg["flow_field_filepath"]
             constituent_dict = cfg["constituents"]
+            if kinetics is None:                                   # optional `kinetics:` block per constituent
+                kinetics = {name: c["kinetics"] for name, c in constituent_dict.items()
+                            if isinstance(c, dict) and c.get("kinetics") is not None} or None
+            if temperature is None:
+                temperature = cfg.get("temperature")
         if not flow_field_file_path or not isinstance(constituent_dict, dict):
             raise TypeError("Missing a `config_filepath` or a `constituent_dict` and `flow_field_file_path` to run the model.")
         plan = ras.read_ras_plan(flow_field_file_path, datetime_range)
@@ -120,23 +127,24 @@ class ClearwaterRiverine:
             units[name] = cfg_c.get("units", "Unknown")
         self._setup(plan.f1, plan.f2, plan.face_x, plan.face_y, plan.time_seconds, plan.face_flow, plan.edge_velocity,
                     plan.volume, float(diffusion_coefficient_input), inputs, units, time=plan.time,
-                    backend_options=backend_options)
+                    backend_options=backend_options, kinetics=kinetics, temperature=temperature)
         self.boundary_data = plan.boundary_data
         self.mesh.attrs["boundary_data"] = plan.boundary_data
 
     @classmethod
     def from_arrays(cls, f1, f2, face_x, face_y, time_seconds, face_flow, edge_velocity, volume,
                     diffusion_coefficient: float, inputs: Dict[str, np.ndarray], units: Optional[Dict[str, str]] = None,
+                    kinetics: Optional[Dict[str, Dict[str, Any]]] = None, temperature: Optional[str | float] = None,
                     **backend_options) -> "ClearwaterRiverine":
         self = cls.__new__(cls)
         self._setup(f1, f2, face_x, face_y, time_seconds, face_flow, edge_velocity, volume, float(diffusion_coefficient),
-                    inputs, units or {}, time=None, backend_options=backend_options)
+                    inputs, units or {}, time=None, backend_options=backend_options, kinetics=kinetics, temperature=temperature)
         self.boundary_data = None
         return self
 
     # ------------------------------------------------------------------------------------------
     def _setup(self, f1, f2, face_x, face_y, time_seconds, face_flow, edge_velocity, volume, D, inputs, units, time,
-               backend_options):
+               backend_options, kinetics=None, temperature=None):
         store_mass_flux = backend_options.pop("store_mass_flux", True)
         # 'eager': update() returns with the results in the host arrays; 'pipelined': the copies overlap the next
         # update() (sync() before reading); 'none': results stay on the device (read them through self.backend)
@@ -184,6 +192,9 @@ class ClearwaterRiverine:
         for k, name in enumerate(self.constituents):
             self.backend.set_inputs(k, self.constituent_dict[name].input_array)
         self._index = {name: k for k, name in enumerate(self.constituents)}
+        self.kinetics = None
+        if kinetics is not None:
+            self.set_kinetics(kinetics, 20.0 if temperature is None else temperature)
         # update() copies c[t+1] of every constituent straight into row t+1 of its output array; page-locking
         # those arrays lets the copies run at the full PCIe rate with no intermediate host buffer
         outputs = [self.mesh[name] for name in self.constituents]
@@ -266,6 +277,19 @@ class ClearwaterRiverine:
         if self.output == "eager":
             self.backend.fetch_wait()
 
+    def set_kinetics(self, spec: Optional[Dict[str, Dict[str, Any]]], temperature: str | float = 20.0):
+        """First-order kinetics applied on the device in every later step, after the update_concentration override and
+        before transport (kinetics.py: spec format; temperature is a constituent name or a constant in deg C).
+        None switches kinetics off.  History rows are not rewritten: the reaction of step t shows in row t + 1."""
+        from .kinetics import compile_kinetics
+        if spec is None:
+            self.backend.set_kinetics(None)
+            self.kinetics = None
+            return
+        kin = compile_kinetics(spec, self.constituents, temperature)
+        self.backend.set_kinetics(kin.decay_per_day, kin.theta, kin.yields, kin.temperature_k, kin.temperature_c)
+        self.kinetics = kin
+
     def sync(self):
         """Wait for the output copies of the updates issued so far (output='pipelined')."""
         self.backend.fetch_wait()
@@ -306,6 +330,9 @@ class ClearwaterRiverine:
         out["bcTotalMassInOutAll"], out["bcTotalMassInAll"], out["bcTotalMassOutAll"] = tm, tm_in, tm_out
         out["vol_end_calc"] = out["Vol_start"] - tv_in - tv_out
         out["mass_end_calc"] = out["Mass_start"] - tm_in - tm_out
+        if self.kinetics is not None:                         # mass the reactions formed (< 0: lost) since the start
+            out["reaction_mass"] = self.backend.reaction_mass(k)
+            out["mass_end_calc"] += out["reaction_mass"]
         out["error_vol"] = out["vol_end_calc"] - out["Vol_end"]
         out["error_mass"] = out["mass_end_calc"] - out["Mass_end"]
         out["prct_error_vol"] = out["error_vol"] / tv_in * 100 if tv_in else float("nan")

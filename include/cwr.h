@@ -201,6 +201,30 @@ int cwr_get_flux_sums(cwr_handle* h, int k, double* total_sum, double* in_sum, d
  * internal edges.  (With cwr_set_hydro, which is not given the raw face flow, advection_coeff stands in for it.) */
 int cwr_get_volume_sums(cwr_handle* h, double* total_sum, double* in_sum, double* out_sum);
 
+/* --- first-order kinetics (decay with temperature correction, transformation chains) ---------------------------------
+ * Step t first forms c~ as without kinetics: c[t], or the cwr_set_state override, with the non-zero real-cell entries of
+ * input_array[t] merged in.  With kinetics set, every real cell i is then reacted before the load term V[t] c~ / dt is formed:
+ *     T_i = temperature_c, or c~ of constituent temperature_k in cell i
+ *     for k in topological order of the yield graph:
+ *         r = decay_k * theta_k^(T_i - 20) / 86400          (decay in 1/day; theta^x = exp(x log theta))
+ *         loss = c~_k * (-expm1(-r dt[t]));  c~_k -= loss;  c~_j += yields[j, k] * loss for every j
+ * and the rest of the step (ghost terms, warm start, solve, BC re-imposition, mass flux) takes the reacted c~'.  History
+ * rows are not rewritten: c[t] stays what transport or the override produced; the reaction of step t shows in c[t+1].
+ * Ghost cells and BC values are not reacted; nothing is clamped.  Rates are per column (a scenario ensemble may sweep them).
+ *
+ * decay_per_day (K) or NULL = kinetics off; theta (K) or NULL = all 1; yields (K,K) row-major,
+ * yields[j*K + k] = mass of j formed per mass of k decayed, or NULL = none; temperature_k = index of the
+ * temperature constituent or -1 for the constant temperature_c.  Takes effect for steps queued after the call
+ * (stream-ordered upload).  CWR_EINVAL for a negative or non-finite decay, theta <= 0 or non-finite, a non-finite yield
+ * or yields[k*K + k] != 0, a cycle in the yield graph, a temperature constituent that decays or receives a yield, an
+ * index out of range.  Domain decomposition: every rank makes the same call. */
+int cwr_set_kinetics(cwr_handle* h, const double* decay_per_day, const double* theta, const double* yields,
+                     int temperature_k, double temperature_c);
+/* Reaction mass of constituent k, sum over the steps taken of sum_i V[t]_i (c~'_ik - c~_ik), reduced on the device in a fixed
+ * order (the same bits every run): a running sum since cwr_create, 0 while kinetics was never set.  Domain decomposition:
+ * the partial sum over the rows the rank owns (as cwr_mass_totals_at). */
+int cwr_get_reaction_mass(cwr_handle* h, int k, double* total);
+
 /* --- domain decomposition over NVLink (SURVEY.md 8e-ii; BASELINE configs[4]) ----------------------------
  * One process per GPU creates a handle with options.dd_rank / dd_world set, every rank with the SAME mesh,
  * hydrodynamics and inputs (the mesh is replicated, the rows are not: a rank assembles, solves and stores

@@ -2,12 +2,14 @@
 """Parity of the domain-decomposed path (one process per GPU, NVLink peer memory) -- run under torchrun:
 
   python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 --master-port 29511 \
-      tools/dd_check.py [--side 160] [--K 3] [--steps 6]
+      tools/dd_check.py [--side 160] [--K 3] [--steps 6] [--kinetics]
 
 Every rank builds the same synthetic mesh, owns one strip of it and steps; the merged concentrations are
 compared with (a) the oracle (reference arithmetic incl. SuperLU, on rank 0; rtol 1e-9 per step as in
 tests/test_gpu_parity.py) and (b) a single-GPU run of the same library on rank 0's GPU.  Mass totals and
-boundary flux sums are checked as sums of the per-rank partial values.  Prints one JSON line per case on
+boundary flux sums are checked as sums of the per-rank partial values.  --kinetics: the same with a first-order
+network (synthetic.make_kinetics) reacted on the device, the oracle being oracle.kinetics.KineticsRiverine, and the
+ranks' reaction masses summed against the single-GPU ones.  Prints one JSON line per case on
 rank 0; exit code 0 only if every check passed on every rank.
 """
 from __future__ import annotations
@@ -30,12 +32,14 @@ def main():
     ap.add_argument("--K", type=int, default=3)
     ap.add_argument("--steps", type=int, default=6)
     ap.add_argument("--no-oracle", action="store_true")
+    ap.add_argument("--kinetics", action="store_true", help="react a first-order network on the device in every step")
     args = ap.parse_args()
     import torch
     import torch.distributed as dist
     from clearwater_riverine_b200 import TransportBackend, synthetic
     from clearwater_riverine_b200.domain import DomainDecomposedBackend, merge_owned
     from oracle import reference_step as ref
+    from oracle.kinetics import KineticsRiverine
 
     rank, world, local = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"]), int(os.environ["LOCAL_RANK"])
     torch.cuda.set_device(local)
@@ -53,11 +57,16 @@ def main():
         adv, _, _, cdiff, dt = ref.derive_coefficients(plan.face_flow, plan.edge_velocity, plan.face_x, plan.face_y,
                                                        plan.f1, plan.f2, D, plan.time_seconds)
         inputs = synthetic.make_inputs(plan, K, seed=40 + ci)
+        kin = None
+        if args.kinetics:
+            inputs, kin = synthetic.make_kinetics(inputs, seed=40 + ci)
         be = DomainDecomposedBackend(plan.f1, plan.f2, plan.n_face, T, K, D, rank, world, device=local, **opts)
         be.set_hydro(0, adv, cdiff, plan.edge_velocity, plan.volume, dt)
         info = be.attach()
         for k in range(K):
             be.set_inputs(k, inputs[k])
+        if kin is not None:
+            be.set_kinetics(**kin)
         single = oracle = None
         if rank == 0:
             single = TransportBackend(plan.f1, plan.f2, plan.n_face, T, K, D, device=local, solver_path=1,
@@ -65,9 +74,16 @@ def main():
             single.set_hydro(0, adv, cdiff, plan.edge_velocity, plan.volume, dt)
             for k in range(K):
                 single.set_inputs(k, inputs[k])
+            if kin is not None:
+                single.set_kinetics(**kin)
             if not args.no_oracle:
                 mesh = ref.HydroMesh(plan.f1, plan.f2, plan.n_face, adv, cdiff, plan.edge_velocity, plan.volume, dt, D)
-                oracle = ref.OracleRiverine(mesh, {f"c{k}": inputs[k] for k in range(K)})
+                named = {f"c{k}": inputs[k] for k in range(K)}
+                if kin is None:
+                    oracle = ref.OracleRiverine(mesh, named)
+                else:
+                    temperature = f"c{kin['temperature_k']}" if kin["temperature_k"] >= 0 else kin["temperature_c"]
+                    oracle = KineticsRiverine(mesh, named, kin["decay_per_day"], kin["theta"], kin["yields"], temperature)
         worst_oracle = worst_single = 0.0
         iters = []
         status = 0
@@ -89,6 +105,7 @@ def main():
         m_dd = be.gather_mass_totals(0, 0, args.steps)
         fsum = np.nansum(np.stack(be.flux_sums(0)), axis=1)
         fsum = merge_owned(fsum, np.ones(3, bool))
+        rmass = np.array([be.gather_reaction_mass(k) for k in range(K)]) if kin is not None else None   # collective
         ok = status == 0
         line = None
         if rank == 0:
@@ -97,11 +114,18 @@ def main():
             mass_err = abs(m_dd[3] - m1.mass_end) / abs(m1.mass_end)
             flux_err = float(np.abs(fsum - f1).max() / max(1e-300, np.abs(f1).max()))
             ok = ok and worst_single < 1e-9 and (oracle is None or worst_oracle < 1e-9) and mass_err < 1e-9 and flux_err < 1e-9
+            rmass_err = None
+            if kin is not None:
+                r1 = np.array([single.reaction_mass(k) for k in range(K)])
+                rmass_err = float(np.abs(rmass - r1).max() / max(1e-300, np.abs(r1).max()))
+                ok = ok and rmass_err < 1e-9
             line = {"case": opts, "world": world, "cells": n, "K": K, "steps": args.steps, "rows_owned_rank0": info.rows_owned,
                     "rows_sent_rank0": info.rows_sent, "colors": info.n_colors, "levels": info.n_levels,
                     "iterations_per_step": iters, "single_gpu_iterations_last_step": s1.iterations,
                     "max_rel_diff_vs_single_gpu": worst_single, "max_rel_diff_vs_oracle": worst_oracle if oracle is not None else None,
                     "mass_end_rel_diff": mass_err, "boundary_flux_sums_rel_diff": flux_err, "ok": bool(ok)}
+            if kin is not None:
+                line["reaction_mass_rel_diff"] = rmass_err
             single.close()
         flag = torch.tensor([1 if ok else 0], device="cuda")
         dist.all_reduce(flag, op=dist.ReduceOp.MIN)

@@ -1,0 +1,189 @@
+#!/usr/bin/env python
+"""What first-order kinetics on the device costs and what it saves (cwr_set_kinetics, k_react).
+
+  python tools/kinetics_bench.py [--reps 20] [--out profiles/kinetics_bench.json]
+
+1M x 16 (bench.py's 1m16 plan; a 16-constituent network with the last constituent as the temperature,
+synthetic.make_kinetics): the step time with kinetics off and on, measured alternately on the same handle (the same step
+t is taken again and again, so both see the same system) with CUDA events; k_react's time as the delta of the
+CWR_FAM_RHS profile family (k_rhs + k_boundary_rhs + k_react), also with the same network at a constant temperature
+(no per-row exp); its bytes 3V + 12n (read c~, vol, D; write c~' and b)
+over that time against a device-to-device copy's rate.  Ohio-shaped mesh, K = 1 and 64 scenarios with 64 decay rates:
+the time kinetics adds per step in cwr_run.  The coupled loop both ways at both sizes: the same reactions on the host
+(every constituent copied down, reacted in numpy, pushed back through the update_concentration override) against the
+device kinetics.  Prints one JSON object and writes it to --out.
+"""
+from __future__ import annotations
+
+import argparse
+import json
+import subprocess
+import sys
+import time
+from pathlib import Path
+
+import numpy as np
+
+ROOT = Path(__file__).resolve().parent.parent
+sys.path.insert(0, str(ROOT))
+
+
+def gpu_name_and_power():
+    try:
+        out = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
+                             capture_output=True, text=True, timeout=30).stdout.strip().splitlines()
+        return out[0] if out else None
+    except Exception:
+        return None
+
+
+def copy_rate_gbs(torch):
+    """Device-to-device copy of 4 GiB (larger than L2): bytes read + written over the time, best of 5."""
+    a = torch.empty(1 << 29, dtype=torch.float64, device="cuda")
+    b = torch.empty_like(a)
+    best = float("inf")
+    for _ in range(6):
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record(); b.copy_(a); e1.record(); e1.synchronize()
+        best = min(best, e0.elapsed_time(e1))
+    del a, b
+    return 2 * 8 * (1 << 29) / (best * 1e-3) / 1e9
+
+
+def build(plan, inputs, torch, **opt):
+    from clearwater_riverine_b200 import TransportBackend
+    K = inputs.shape[0]
+    be = TransportBackend(plan.f1, plan.f2, plan.n_face, plan.n_time, K, 0.1, **opt)
+    be.set_geometry(plan.face_x, plan.face_y)
+    be.set_hydro_raw(0, plan.face_flow, plan.edge_velocity, plan.volume, np.append(np.diff(plan.time_seconds), np.nan))
+    for k in range(K):
+        be.set_inputs(k, inputs[k])
+    return be
+
+
+def timed(torch, be, fn, n):
+    """ms per call of fn over n calls, CUDA events on the handle's stream."""
+    s = torch.cuda.ExternalStream(be.stream())
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    e0.record(s)
+    for _ in range(n):
+        fn()
+    e1.record(s)
+    e1.synchronize()
+    return e0.elapsed_time(e1) / n
+
+
+def alternate(torch, be, kin, fn, reps, n):
+    """fn timed with kinetics off and on, alternately, reps times each: medians (ms)."""
+    off, on = [], []
+    for _ in range(reps):
+        be.set_kinetics(None)
+        off.append(timed(torch, be, fn, n))
+        be.set_kinetics(**kin)
+        on.append(timed(torch, be, fn, n))
+    return float(np.median(off)), float(np.median(on))
+
+
+def host_loop(be, kin, t0, steps, dt):
+    """The coupled loop with the reactions on the host: c[t] down, numpy reactions, override up, step.  s per step."""
+    from oracle.kinetics import react
+    be.set_kinetics(None)
+    t_start = time.perf_counter()
+    for t in range(t0, t0 + steps):
+        c = be.get_state_all(t)
+        temp = kin["temperature_k"] if kin["temperature_k"] >= 0 else kin["temperature_c"]
+        c = react(c, dt, kin["decay_per_day"], kin["theta"], kin["yields"], temp, kin["temperature_k"] >= 0)
+        be.set_state_all(t, c)
+        be.step(t)
+    be.get_state_all(t0 + steps)
+    return (time.perf_counter() - t_start) / steps
+
+
+def device_loop(torch, be, kin, t0, steps):
+    be.set_kinetics(**kin)
+    t_start = time.perf_counter()
+    be.run(t0, t0 + steps)
+    be.get_state_all(t0 + steps)
+    return (time.perf_counter() - t_start) / steps
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--reps", type=int, default=15)
+    ap.add_argument("--scale", type=float, default=1.0, help="1m16 mesh side scale (1.0 = 1M cells)")
+    ap.add_argument("--out", default=None)
+    args = ap.parse_args()
+    import torch
+    import bench
+    from clearwater_riverine_b200 import synthetic
+    if not torch.cuda.is_available():
+        raise SystemExit("kinetics_bench needs a CUDA device")
+    res = {"gpu": gpu_name_and_power(), "d2d_copy_gbs": copy_rate_gbs(torch)}
+
+    # --- 1M x 16 ------------------------------------------------------------------------------------------------
+    T = 14
+    plan, K = bench.workload_plan("1m16", T, seed=0, scale=args.scale)
+    inputs, kin = synthetic.make_kinetics(synthetic.make_inputs(plan, K, seed=0), seed=0, decay_range=(0.05, 2.0))
+    be = build(plan, inputs, torch)
+    n = be.n_real
+    for t in range(3):
+        be.step(t)
+    t = 3
+    step = lambda: be.step(t)
+    be.set_kinetics(**kin)
+    for _ in range(3):
+        step()
+    off, on = alternate(torch, be, kin, step, args.reps, 5)
+    fam = {}
+    # "const": the same network at a constant temperature -- the per-row exp of theta^(T - 20) is gone (one factor per
+    # constituent per CTA), what is left is the tile's load / chain / store
+    kin_const = dict(kin, temperature_k=-1, temperature_c=24.0)
+    for mode in ("off", "on", "const"):
+        be.set_kinetics(None) if mode == "off" else be.set_kinetics(**(kin if mode == "on" else kin_const))
+        step()
+        be.profile(1)
+        for _ in range(10):
+            step()
+        fam[mode] = be.profile(-1)["rhs"][0] / 10
+        be.profile(0)
+    react_ms = fam["on"] - fam["off"]
+    react_const_ms = fam["const"] - fam["off"]
+    nbytes = 3 * 8 * n * K + 12 * n
+    res["1m16"] = {"cells": n, "K": K, "step_ms_off": off, "step_ms_on": on, "added_ms": on - off,
+                   "added_fraction": (on - off) / off, "rhs_family_ms_off": fam["off"], "rhs_family_ms_on": fam["on"],
+                   "k_react_ms": react_ms, "k_react_bytes": nbytes, "k_react_gbs": nbytes / (react_ms * 1e-3) / 1e9,
+                   "k_react_of_copy_rate": nbytes / (react_ms * 1e-3) / 1e9 / res["d2d_copy_gbs"],
+                   "k_react_ms_constant_temperature": react_const_ms,
+                   "k_react_of_copy_rate_constant_temperature": nbytes / (react_const_ms * 1e-3) / 1e9 / res["d2d_copy_gbs"]}
+    steps = 8
+    res["1m16"]["coupled_host_ms_per_step"] = 1e3 * host_loop(be, kin, 4, steps, 30.0)
+    res["1m16"]["coupled_device_ms_per_step"] = 1e3 * device_loop(torch, be, kin, 4, steps)
+    be.close()
+    del inputs, plan
+
+    # --- Ohio-shaped mesh ---------------------------------------------------------------------------------------
+    T = 202
+    plan = synthetic.ohio_like(T, seed=2)
+    for K in (1, 64):
+        inputs = synthetic.make_inputs(plan, K, seed=2)
+        kin = dict(decay_per_day=np.linspace(0.05, 3.0, K), theta=np.full(K, 1.047), yields=None, temperature_k=-1,
+                   temperature_c=17.0)
+        be = build(plan, inputs, torch)
+        be.set_kinetics(**kin)
+        be.run(0, 200)
+        off, on = alternate(torch, be, kin, lambda: be.run(0, 200), max(3, args.reps // 3), 1)
+        key = "ohio" if K == 1 else "ohio_ens64"
+        res[key] = {"cells": be.n_real, "K": K, "solver_path": be.options.solver_path, "step_ms_off": off / 200,
+                    "step_ms_on": on / 200, "added_us_per_step": 1e3 * (on - off) / 200}
+        res[key]["coupled_host_ms_per_step"] = 1e3 * host_loop(be, kin, 0, 100, 3600.0)
+        res[key]["coupled_device_ms_per_step"] = 1e3 * device_loop(torch, be, kin, 0, 100)
+        be.close()
+    line = json.dumps(res)
+    print(line)
+    if args.out:
+        Path(args.out).parent.mkdir(parents=True, exist_ok=True)
+        Path(args.out).write_text(json.dumps(res, indent=1) + "\n")
+
+
+if __name__ == "__main__":
+    main()
