@@ -103,6 +103,7 @@ def load_library():
         "cwr_get_flux_sums": ([H, C.c_int, dp, dp, dp], C.c_int),
         "cwr_get_volume_sums": ([H, dp, dp, dp], C.c_int),
         "cwr_set_kinetics": ([H, dp, dp, dp, C.c_int, C.c_double], C.c_int),
+        "cwr_set_kinetics_sources": ([H, dp, dp, dp, dp, dp, ip], C.c_int),
         "cwr_get_reaction_mass": ([H, C.c_int, dp], C.c_int),
         "cwr_get_lhs": ([H, C.POINTER(C.c_int64), ip, ip, dp], C.c_int),
         "cwr_get_rhs": ([H, C.c_int, dp], C.c_int),
@@ -413,7 +414,8 @@ class TransportBackend:
         """First-order decay / transformations applied on the device in every later step (cwr_set_kinetics):
         decay_per_day (K,) or None = off; theta (K,) or None = all 1; yields (K, K), yields[j, k] = mass of j formed per
         mass of k decayed, or None; temperature_k = temperature constituent or -1 for the constant temperature_c (deg C).
-        An invalid set raises ValueError.  kinetics.compile_kinetics builds the arrays from a by-name spec."""
+        An invalid set raises ValueError; any call clears set_kinetics_sources.  kinetics.compile_kinetics builds the
+        arrays from a by-name spec."""
         if decay_per_day is None:
             self._check(self._lib.cwr_set_kinetics(self._h, None, None, None, -1, 20.0))
             return
@@ -422,6 +424,23 @@ class TransportBackend:
         y = None if yields is None else _arr(yields, np.float64, (self.K, self.K), "yields")
         rc = self._lib.cwr_set_kinetics(self._h, _ptr(d, C.c_double), _ptr(th, C.c_double), _ptr(y, C.c_double),
                                         int(temperature_k), float(temperature_c))
+        if rc == CWR_EINVAL:
+            raise ValueError(self._lib.cwr_last_error(self._h).decode())
+        self._check(rc)
+
+    def set_kinetics_sources(self, source_per_day=None, source_theta=None, exchange_per_day=None, exchange_theta=None,
+                             equilibrium=None, equilibrium_kind=None):
+        """Zero-order sources and relaxation toward an equilibrium, applied after the first-order chain of the kinetics set
+        last (cwr_set_kinetics_sources): dc/dt = s + r (ceq - c) per column, solved exactly over each step.
+        source_per_day (K,) or None; exchange_per_day (K,) 1/day or None (both None: sources off); a theta (K,) or None =
+        all 1; equilibrium (K,) the constant targets; equilibrium_kind (K,) 0 = constant, 1 = oxygen saturation at T, or
+        None = all 0.  set_kinetics clears them.  An invalid set raises ValueError."""
+        K = (self.K,)
+        f = lambda a, name: None if a is None else _arr(a, np.float64, K, name)
+        arrs = [f(source_per_day, "source_per_day"), f(source_theta, "source_theta"), f(exchange_per_day, "exchange_per_day"),
+                f(exchange_theta, "exchange_theta"), f(equilibrium, "equilibrium")]
+        kind = None if equilibrium_kind is None else _arr(equilibrium_kind, np.int32, K, "equilibrium_kind")
+        rc = self._lib.cwr_set_kinetics_sources(self._h, *[_ptr(a, C.c_double) for a in arrs], _ptr(kind, C.c_int32))
         if rc == CWR_EINVAL:
             raise ValueError(self._lib.cwr_last_error(self._h).decode())
         self._check(rc)

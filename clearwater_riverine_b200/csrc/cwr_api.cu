@@ -116,6 +116,9 @@ struct cwr_handle {
     int kin_steps = 0, kin_temp_k = -1, kin_grid_max = 0;   // kin_grid_max: resident CTAs of k_react (partials sized for it)
     double kin_temp_c = 20.0;
     KinStep* d_kin_steps = nullptr; KinYield* d_kin_yields = nullptr; KinState* d_kin_state = nullptr; double* d_kin_partials = nullptr;
+    // sources and exchange (cwr_set_kinetics_sources): the listed columns in ascending order; kin_src_o2: one is kind 1
+    int kin_srcs = 0, kin_src_o2 = 0;
+    KinSrc* d_kin_srcs = nullptr;
     // optional per-kernel-family timing with CUDA events on the handle's stream (bench.py roofline)
     bool profiling = false;
     std::vector<cudaEvent_t> ev_pool;
@@ -1337,8 +1340,9 @@ static int build_rhs(cwr_handle* h, int t, int accumulate) {
         // after cwr_set_kinetics), at most the resident grid; the same rows give the same grid, hence the same sums
         const int R = react_tile_rows(h->K);
         const int grid = grid_for((M.row_hi - M.row_lo + R - 1) / R, 1, h->kin_grid_max);
-        CK(launch_chain(h, k_react, grid, kThreads, react_smem_bytes(h->K), M, (const KinStep*)h->d_kin_steps, h->kin_steps,
-                        (const KinYield*)h->d_kin_yields, h->kin_temp_k, h->kin_temp_c, h->d_kin_partials, h->d_kin_state, accumulate));
+        CK(launch_chain(h, k_react, grid, kThreads, react_smem_bytes(h->K) + react_src_smem_bytes(h->kin_srcs, h->kin_temp_k), M,
+                        (const KinStep*)h->d_kin_steps, h->kin_steps, (const KinYield*)h->d_kin_yields, h->kin_temp_k, h->kin_temp_c,
+                        (const KinSrc*)h->d_kin_srcs, h->kin_srcs, h->kin_src_o2, h->d_kin_partials, h->d_kin_state, accumulate));
         h->launches += 1;
     }
     if (M.b_hi - M.b_lo > 0) {
@@ -1690,7 +1694,7 @@ int cwr_set_kinetics(cwr_handle* h, const double* decay, const double* theta, co
                      double temperature_c) {
     if (!h) return CWR_EINVAL;
     const int K = h->K;
-    if (!decay) { h->kin_on = false; return CWR_OK; }
+    if (!decay) { h->kin_on = false; h->kin_srcs = 0; return CWR_OK; }
     for (int k = 0; k < K; ++k) {
         if (!std::isfinite(decay[k]) || decay[k] < 0.0) FAIL(CWR_EINVAL, "cwr_set_kinetics: decay rates must be finite and >= 0");
         if (theta && (!std::isfinite(theta[k]) || theta[k] <= 0.0)) FAIL(CWR_EINVAL, "cwr_set_kinetics: theta must be finite and > 0");
@@ -1749,6 +1753,7 @@ int cwr_set_kinetics(cwr_handle* h, const double* decay, const double* theta, co
         CK(dalloc(h, &h->d_kin_yields, (size_t)K * K));
         CK(dalloc(h, &h->d_kin_partials, (size_t)K * h->kin_grid_max));
         CK(dalloc(h, &h->d_kin_state, 1));
+        CK(dalloc(h, &h->d_kin_srcs, (size_t)K));
         CK(cudaMemsetAsync(h->d_kin_state, 0, sizeof(KinState), h->stream));
     }
     // stream-ordered: steps queued before this call still read the previous parameters (pageable sources: the copies
@@ -1759,6 +1764,56 @@ int cwr_set_kinetics(cwr_handle* h, const double* decay, const double* theta, co
     h->kin_temp_k = temperature_k;
     h->kin_temp_c = temperature_k < 0 ? temperature_c : 20.0;
     h->kin_on = true;
+    h->kin_srcs = 0;
+    return CWR_OK;
+}
+
+int cwr_set_kinetics_sources(cwr_handle* h, const double* source_per_day, const double* source_theta, const double* exchange_per_day,
+                             const double* exchange_theta, const double* equilibrium, const int* equilibrium_kind) {
+    if (!h) return CWR_EINVAL;
+    const int K = h->K;
+    if (!h->kin_on) FAIL(CWR_EINVAL, "cwr_set_kinetics_sources: call cwr_set_kinetics first");
+    if (!source_per_day && !exchange_per_day) { h->kin_srcs = 0; return CWR_OK; }
+    if (exchange_per_day && !equilibrium) FAIL(CWR_EINVAL, "cwr_set_kinetics_sources: exchange needs an equilibrium array");
+    for (int k = 0; k < K; ++k) {
+        const double s = source_per_day ? source_per_day[k] : 0.0, e = exchange_per_day ? exchange_per_day[k] : 0.0;
+        const int kind = equilibrium_kind ? equilibrium_kind[k] : 0;
+        if (!std::isfinite(s)) FAIL(CWR_EINVAL, "cwr_set_kinetics_sources: sources must be finite");
+        if (source_theta && (!std::isfinite(source_theta[k]) || source_theta[k] <= 0.0))
+            FAIL(CWR_EINVAL, "cwr_set_kinetics_sources: source_theta must be finite and > 0");
+        if (exchange_theta && (!std::isfinite(exchange_theta[k]) || exchange_theta[k] <= 0.0))
+            FAIL(CWR_EINVAL, "cwr_set_kinetics_sources: exchange_theta must be finite and > 0");
+        if (!std::isfinite(e) || e < 0.0) FAIL(CWR_EINVAL, "cwr_set_kinetics_sources: exchange rates must be finite and >= 0");
+        if (kind != 0 && kind != 1) FAIL(CWR_EINVAL, "cwr_set_kinetics_sources: equilibrium_kind must be 0 (constant) or 1 (oxygen saturation)");
+        if (kind == 0 && e > 0.0 && !std::isfinite(equilibrium[k]))
+            FAIL(CWR_EINVAL, "cwr_set_kinetics_sources: a constant equilibrium must be finite");
+        if (kind == 1 && k == h->kin_temp_k)
+            FAIL(CWR_EINVAL, "cwr_set_kinetics_sources: the temperature constituent cannot relax toward oxygen saturation");
+    }
+    // only the columns with a term are listed; the equilibrium of a column without exchange is never read
+    std::vector<KinSrc> list;
+    int o2 = 0;
+    for (int k = 0; k < K; ++k) {
+        const double s = source_per_day ? source_per_day[k] : 0.0, e = exchange_per_day ? exchange_per_day[k] : 0.0;
+        if (s == 0.0 && e == 0.0) continue;
+        KinSrc c{};
+        c.col = k;
+        c.kind = e > 0.0 && equilibrium_kind ? equilibrium_kind[k] : 0;
+        c.source = s; c.log_source_theta = source_theta ? std::log(source_theta[k]) : 0.0;
+        c.exchange = e; c.log_exchange_theta = exchange_theta ? std::log(exchange_theta[k]) : 0.0;
+        c.equilibrium = e > 0.0 && c.kind == 0 ? equilibrium[k] : 0.0;
+        o2 |= c.kind;
+        list.push_back(c);
+    }
+    CK(cudaSetDevice(h->device));
+    // at a constant temperature the coefficients take shared memory beyond the tile's 48 KB (react_src_smem_bytes); the
+    // limit is the same for every handle (the attribute is the kernel's, not the handle's)
+    if (h->kin_temp_k < 0 && !list.empty())
+        CK(cudaFuncSetAttribute(k_react, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                (int)(kReactSmemLimit - kReactStaticSmem + react_src_smem_bytes(kMaxK, -1))));
+    if (!list.empty()) CK(cudaMemcpyAsync(h->d_kin_srcs, list.data(), list.size() * sizeof(KinSrc), cudaMemcpyHostToDevice, h->stream));
+    h->kin_srcs = (int)list.size();
+    h->kin_src_o2 = o2;
     return CWR_OK;
 }
 

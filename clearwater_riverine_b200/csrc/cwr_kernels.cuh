@@ -537,15 +537,36 @@ __device__ __forceinline__ void grid_totals(const double* partials, double* tot,
 // reads the reacted c~'), so a zero rate leaves every bit as it was.  The step's reaction mass sum_i vol_i (c~'_ik - c~_ik)
 // is reduced per column without atomics: per-thread sums over a fixed set of rows, per-CTA partials, and the last CTA adds
 // them in block order (grid_totals).
+// Sources and exchange (cwr_set_kinetics_sources) follow the chain in the same row, for the listed columns in ascending k:
+//     s = source_k theta_s^(T - 20) / 86400,  r = exchange_k theta_e^(T - 20) / 86400,  ceq = equilibrium_k | O2sat(T)
+//     phi = -expm1(-r dt) / r (dt when r == 0),  c~_k += (s + r ceq - r c~_k) phi
+// the exact solution of dc/dt = s + r (ceq - c) over dt.  T is the value before any of the step's reactions.
 // ---------------------------------------------------------------------------------------------
 struct KinStep { int col, y_begin, y_end, pad; double decay, log_theta; };   // a reacting constituent; its yields
 struct KinYield { int col, pad; double y; };                                 // [y_begin, y_end)
 struct KinState { unsigned ticket; int pad; double mass[kMaxK]; };           // last-CTA ticket, running reaction mass
+// a column with a source or exchange term; kind 1: ceq = O2sat(T) (listed only with exchange > 0), kind 0: ceq = equilibrium
+struct KinSrc { int col, kind; double source, log_source_theta, exchange, log_exchange_theta, equilibrium; };
+
+// Dissolved-oxygen saturation (mg/L) of fresh water at 1 atm, T in deg C (APHA / Benson-Krause), as written: no clamp
+__device__ __forceinline__ double o2_saturation(double T) {
+    const double x = 1.0 / (T + 273.15);
+    return exp(-139.34411 + x * (1.575701e5 + x * (-6.642308e7 + x * (1.243800e10 + x * -8.621949e11))));
+}
+
+// s + r ceq, r and phi of one source column at temperature T (o2 = O2sat(T), read only for kind 1)
+__device__ __forceinline__ void kin_src_coef(const KinSrc& s, double T, double o2, double dt, double& sr, double& r, double& phi) {
+    const double dT = T - 20.0;
+    r = s.exchange * exp(dT * s.log_exchange_theta) / 86400.0;
+    sr = s.source * exp(dT * s.log_source_theta) / 86400.0 + r * (s.kind ? o2 : s.equilibrium);
+    phi = r > 0.0 ? -expm1(-r * dt) / r : dt;
+}
 
 // Shared memory of k_react: st[kMaxK] and last_block_arrives' flag (static, kReactStaticSmem bounds them), then the dynamic
 // part: a tile of R rows x (K + 1) doubles (odd stride: the one-row-per-thread chain is free of bank conflicts), vol and D
 // of its rows, fac[kMaxK] and red[kThreads].  R is the largest multiple of 32 (at most kThreads) that keeps the whole within
-// the 48 KB a kernel may use without opting in, for every K <= kMaxK.
+// the 48 KB a kernel may use without opting in, for every K <= kMaxK.  With source columns at a constant temperature, their
+// coefficients follow (react_src_smem_bytes, opted in); the tile does not shrink for them, so R is the same with or without.
 constexpr size_t kReactSmemLimit = 48 * 1024;
 constexpr size_t kReactStaticSmem = sizeof(KinStep) * kMaxK + 64;
 __host__ __device__ constexpr int react_tile_rows(int K) {
@@ -562,6 +583,10 @@ constexpr bool react_smem_fits_every_k() {
     return true;
 }
 static_assert(react_smem_fits_every_k(), "k_react's shared memory must fit in 48 KB for every K <= kMaxK");
+// [3 n_src] s + r ceq, r, phi per source column; only at a constant temperature (a temperature constituent: per row)
+__host__ __device__ constexpr size_t react_src_smem_bytes(int n_src, int temp_k) {
+    return temp_k < 0 ? (size_t)3 * n_src * sizeof(double) : 0;
+}
 
 // f(e) for the elements [0, cnt) of a tile of the interleaved state that starts at `base`: each thread takes pairs that
 // are 16-byte aligned there, the unpaired element at either end is taken by one thread.  (A state slot starts at an odd
@@ -579,6 +604,7 @@ __device__ __forceinline__ void react_pairs(const double* base, int cnt, F f) {
 
 __global__ void __launch_bounds__(kThreads) k_react(DeviceModel M, const KinStep* __restrict__ steps, int n_steps,
                                                     const KinYield* __restrict__ yl, int temp_k, double temp_c,
+                                                    const KinSrc* __restrict__ srcs, int n_src, int src_o2,
                                                     double* __restrict__ partials, KinState* __restrict__ ks, int accumulate) {
     extern __shared__ double rs[];
     __shared__ KinStep st[kMaxK];
@@ -590,12 +616,18 @@ __global__ void __launch_bounds__(kThreads) k_react(DeviceModel M, const KinStep
     double* sdg = svol + R;                   // [R] D
     double* fac = sdg + R;                    // [kMaxK] constant temperature: 1 - exp(-r dt) of every step
     double* red = fac + kMaxK;                // [kThreads] column sums
+    double* sco = red + kThreads;             // [3 n_src] constant temperature: s + r ceq, r, phi (react_src_smem_bytes)
     const double dt = sp.dt;
     for (int p = threadIdx.x; p < n_steps; p += blockDim.x) {
         const KinStep s = steps[p];
         st[p] = s;
         if (temp_k < 0) fac[p] = -expm1(-(s.decay * exp((temp_c - 20.0) * s.log_theta) / 86400.0) * dt);
     }
+    if (temp_k < 0)
+        for (int p = threadIdx.x; p < n_src; p += blockDim.x) {
+            const KinSrc s = srcs[p];
+            kin_src_coef(s, temp_c, s.kind ? o2_saturation(temp_c) : 0.0, dt, sco[3 * p], sco[3 * p + 1], sco[3 * p + 2]);
+        }
     __syncthreads();
     // column sums: thread (g, k) adds rows g, g + G, ... of every tile the CTA takes, in that order
     const int G = kThreads / K, kc = threadIdx.x % K, g = threadIdx.x / K;
@@ -628,6 +660,22 @@ __global__ void __launch_bounds__(kThreads) k_react(DeviceModel M, const KinStep
                 for (int q = s.y_begin; q < s.y_end; ++q) {
                     const KinYield y = yl[q];
                     c[y.col] += y.y * loss;
+                }
+            }
+            if (temp_k < 0) {
+                for (int p = 0; p < n_src; ++p) {
+                    const double* q = sco + 3 * p;
+                    double& v = c[srcs[p].col];
+                    v += (q[0] - q[1] * v) * q[2];
+                }
+            } else if (n_src > 0) {
+                const double o2 = src_o2 ? o2_saturation(T) : 0.0;
+                for (int p = 0; p < n_src; ++p) {
+                    const KinSrc s = srcs[p];
+                    double sr, r, phi;
+                    kin_src_coef(s, T, o2, dt, sr, r, phi);
+                    double& v = c[s.col];
+                    v += (sr - r * v) * phi;
                 }
             }
         }

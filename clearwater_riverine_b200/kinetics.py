@@ -1,22 +1,39 @@
-"""First-order kinetics by constituent name -> the arrays of `cwr_set_kinetics` (include/cwr.h), validated.
+"""Kinetics by constituent name -> the arrays of `cwr_set_kinetics` and `cwr_set_kinetics_sources` (include/cwr.h),
+validated.
 
     {"BOD": {"decay_per_day": 0.23, "theta": 1.047, "yields": {"DO": -1.0}},
-     "NH4": {"decay_per_day": 0.10, "theta": 1.083, "yields": {"NO3": 1.0, "DO": -4.57}}}
+     "NH4": {"decay_per_day": 0.10, "theta": 1.083, "yields": {"NO3": 1.0, "DO": -4.57}},
+     "DO":  {"source_per_day": -1.5, "source_theta": 1.065,                       # sediment oxygen demand
+             "exchange_per_day": 0.7, "exchange_theta": 1.024, "equilibrium": "oxygen_saturation"},
+     "T":   {"exchange_per_day": 0.3, "equilibrium": 18.0}}                       # equilibrium temperature
 
 Every step, each real cell is reacted before the load term is formed: for the decaying constituents k in topological
 order of the yield graph, loss = c_k (1 - exp(-decay_k theta_k^(T - 20) dt / 86400)) leaves k and yield * loss is added
-to every constituent k yields.  The temperature T (deg C) is a constant or another constituent's value in the cell.
+to every constituent k yields.  Then every constituent with a zero-order source s (per day) or an exchange rate r
+(1/day) toward an equilibrium ceq follows dc/dt = s + r (ceq - c), solved exactly over the step, with s and r corrected
+by their own theta^(T - 20); ceq is a constant or the oxygen saturation at T (`oxygen_saturation`).  The temperature T
+(deg C) is a constant or another constituent's value in the cell before the step's reactions.
 The library checks the same conditions; checking them here names the constituents in the error.
 """
 from __future__ import annotations
 
 import math
 from dataclasses import dataclass
-from typing import Mapping, Sequence, Tuple, Union
+from typing import Mapping, Optional, Sequence, Tuple, Union
 
 import numpy as np
 
-_KEYS = {"decay_per_day", "theta", "yields"}
+_KEYS = {"decay_per_day", "theta", "yields", "source_per_day", "source_theta", "exchange_per_day", "exchange_theta",
+         "equilibrium"}
+OXYGEN_SATURATION = "oxygen_saturation"
+
+
+def oxygen_saturation(T):
+    """Dissolved-oxygen saturation (mg/L) of fresh water at 1 atm, T in deg C: the APHA / Benson-Krause formula
+    ln O2sat = -139.34411 + 1.575701e5/Ta - 6.642308e7/Ta^2 + 1.243800e10/Ta^3 - 8.621949e11/Ta^4, Ta = T + 273.15,
+    evaluated as the device evaluates it, with no clamp."""
+    x = 1.0 / (np.asarray(T, np.float64) + 273.15)
+    return np.exp(-139.34411 + x * (1.575701e5 + x * (-6.642308e7 + x * (1.243800e10 + x * -8.621949e11))))
 
 
 @dataclass(frozen=True)
@@ -27,6 +44,22 @@ class Kinetics:
     temperature_k: int            # temperature constituent, or -1
     temperature_c: float          # the constant temperature when temperature_k == -1
     order: Tuple[int, ...]        # topological order of the yield graph (the order the reactions are applied in)
+    source_per_day: Optional[np.ndarray] = None     # (K,) zero-order source, concentration units per day (< 0: a sink)
+    source_theta: Optional[np.ndarray] = None       # (K,)
+    exchange_per_day: Optional[np.ndarray] = None   # (K,) 1/day, relaxation toward the equilibrium
+    exchange_theta: Optional[np.ndarray] = None     # (K,)
+    equilibrium: Optional[np.ndarray] = None        # (K,) the constant target of kind 0
+    equilibrium_kind: Optional[np.ndarray] = None   # (K,) int32: 0 = constant, 1 = oxygen saturation at T
+
+    @property
+    def has_sources(self) -> bool:
+        """Whether any constituent has a source or an exchange term (otherwise cwr_set_kinetics_sources is not needed)."""
+        return any(a is not None and (a != 0).any() for a in (self.source_per_day, self.exchange_per_day))
+
+    def sources_arguments(self) -> dict:
+        """The arguments of TransportBackend.set_kinetics_sources."""
+        return dict(source_per_day=self.source_per_day, source_theta=self.source_theta, exchange_per_day=self.exchange_per_day,
+                    exchange_theta=self.exchange_theta, equilibrium=self.equilibrium, equilibrium_kind=self.equilibrium_kind)
 
 
 def topological_order(yields: np.ndarray) -> Tuple[int, ...]:
@@ -48,8 +81,11 @@ def topological_order(yields: np.ndarray) -> Tuple[int, ...]:
     return tuple(order)
 
 
-def validate(decay_per_day, theta, yields, temperature_k: int, temperature_c: float, names: Sequence[str] = ()) -> None:
-    """The conditions cwr_set_kinetics rejects with CWR_EINVAL, as ValueError."""
+def validate(decay_per_day, theta, yields, temperature_k: int, temperature_c: float, names: Sequence[str] = (), *,
+             source_per_day=None, source_theta=None, exchange_per_day=None, exchange_theta=None, equilibrium=None,
+             equilibrium_kind=None) -> None:
+    """The conditions cwr_set_kinetics and cwr_set_kinetics_sources reject with CWR_EINVAL, as ValueError.  The source
+    arrays follow the ABI: None = none / all 1 / all 0 as there."""
     d, th, y = np.asarray(decay_per_day, np.float64), np.asarray(theta, np.float64), np.asarray(yields, np.float64)
     K = d.shape[0]
     nm = (lambda k: repr(names[k])) if len(names) == K else (lambda k: f"#{k}")
@@ -73,16 +109,42 @@ def validate(decay_per_day, theta, yields, temperature_k: int, temperature_c: fl
         if (y[temperature_k] != 0).any():
             raise ValueError(f"the temperature constituent {nm(temperature_k)} cannot receive a yield")
     topological_order(y)
+    if source_per_day is None and exchange_per_day is None:
+        return
+    if exchange_per_day is not None and equilibrium is None:
+        raise ValueError("an exchange rate needs an equilibrium")
+    col = lambda a, fill: np.full(K, fill, np.float64) if a is None else np.asarray(a, np.float64)
+    s, sth, e, eth = col(source_per_day, 0.0), col(source_theta, 1.0), col(exchange_per_day, 0.0), col(exchange_theta, 1.0)
+    eq = col(equilibrium, 0.0)
+    kind = np.zeros(K, np.int64) if equilibrium_kind is None else np.asarray(equilibrium_kind)
+    for k in range(K):
+        if not math.isfinite(s[k]):
+            raise ValueError(f"source_per_day of {nm(k)} must be finite, got {s[k]}")
+        for what, v in (("source_theta", sth[k]), ("exchange_theta", eth[k])):
+            if not math.isfinite(v) or v <= 0:
+                raise ValueError(f"{what} of {nm(k)} must be finite and > 0, got {v}")
+        if not math.isfinite(e[k]) or e[k] < 0:
+            raise ValueError(f"exchange_per_day of {nm(k)} must be finite and >= 0, got {e[k]}")
+        if kind[k] not in (0, 1):
+            raise ValueError(f"equilibrium kind of {nm(k)} must be 0 (constant) or 1 ({OXYGEN_SATURATION}), got {kind[k]}")
+        if kind[k] == 0 and e[k] > 0 and not math.isfinite(eq[k]):
+            raise ValueError(f"equilibrium of {nm(k)} must be finite, got {eq[k]}")
+        if kind[k] == 1 and k == temperature_k:
+            raise ValueError(f"the temperature constituent {nm(k)} cannot relax toward {OXYGEN_SATURATION}")
 
 
 def compile_kinetics(spec: Mapping[str, Mapping], constituents: Sequence[str],
                      temperature: Union[str, float] = 20.0) -> Kinetics:
-    """spec: {constituent: {"decay_per_day": float, "theta": float (default 1), "yields": {constituent: float}}};
+    """spec: {constituent: {"decay_per_day": float, "theta": float (default 1), "yields": {constituent: float},
+    "source_per_day": float, "source_theta": float (default 1), "exchange_per_day": float, "exchange_theta": float
+    (default 1), "equilibrium": float or "oxygen_saturation" (required when exchange_per_day > 0)}};
     temperature: a constituent name, or a constant in deg C."""
     names = list(constituents)
     index = {n: k for k, n in enumerate(names)}
     K = len(names)
     decay, theta, yields = np.zeros(K), np.ones(K), np.zeros((K, K))
+    source, source_theta, exchange, exchange_theta = np.zeros(K), np.ones(K), np.zeros(K), np.ones(K)
+    equilibrium, kind = np.zeros(K), np.zeros(K, np.int32)
     for name, block in spec.items():
         if name not in index:
             raise ValueError(f"kinetics given for {name!r}, which is not a constituent of the model")
@@ -98,11 +160,26 @@ def compile_kinetics(spec: Mapping[str, Mapping], constituents: Sequence[str],
             if target not in index:
                 raise ValueError(f"kinetics of {name!r}: yield to {target!r}, which is not a constituent of the model")
             yields[index[target], k] = float(y)
+        source[k] = float(block.get("source_per_day", 0.0))
+        source_theta[k] = float(block.get("source_theta", 1.0))
+        exchange[k] = float(block.get("exchange_per_day", 0.0))
+        exchange_theta[k] = float(block.get("exchange_theta", 1.0))
+        eq = block.get("equilibrium")
+        if isinstance(eq, str):
+            if eq != OXYGEN_SATURATION:
+                raise ValueError(f"kinetics of {name!r}: equilibrium must be a number or {OXYGEN_SATURATION!r}, got {eq!r}")
+            kind[k] = 1
+        elif eq is not None:
+            equilibrium[k] = float(eq)
+        elif exchange[k] > 0:
+            raise ValueError(f"kinetics of {name!r}: exchange_per_day > 0 needs an equilibrium")
     if isinstance(temperature, str):
         if temperature not in index:
             raise ValueError(f"temperature constituent {temperature!r} is not a constituent of the model")
         temperature_k, temperature_c = index[temperature], 20.0
     else:
         temperature_k, temperature_c = -1, float(temperature)
-    validate(decay, theta, yields, temperature_k, temperature_c, names)
-    return Kinetics(decay, theta, yields, temperature_k, temperature_c, topological_order(yields))
+    validate(decay, theta, yields, temperature_k, temperature_c, names, source_per_day=source, source_theta=source_theta,
+             exchange_per_day=exchange, exchange_theta=exchange_theta, equilibrium=equilibrium, equilibrium_kind=kind)
+    return Kinetics(decay, theta, yields, temperature_k, temperature_c, topological_order(yields), source, source_theta,
+                    exchange, exchange_theta, equilibrium, kind)

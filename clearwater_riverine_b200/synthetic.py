@@ -322,3 +322,34 @@ def make_kinetics(inputs: np.ndarray, *, seed: int = 0, decay_range=(20.0, 200.0
         inputs[temperature_k] = np.where(a != 0, 10.0 + 0.2 * a, 0.0)
     return inputs, dict(decay_per_day=decay, theta=theta, yields=yields, temperature_k=temperature_k,
                         temperature_c=13.0 if K == 1 else 24.0)
+
+
+def make_kinetics_sources(kin: dict, *, seed: int = 0, rate_range=(20.0, 200.0)) -> dict:
+    """Seeded zero-order sources and exchange for a network of make_kinetics (kin: its set_kinetics arguments), in the
+    manner of a BOD-DO model: every reacting constituent k has a source of 5..50 x rate_range per day (a sink for odd k,
+    like sediment oxygen demand) and, for even k, an exchange rate in rate_range (1/day) toward oxygen saturation
+    (k = 2 mod 4, reaeration) or a constant 5..45 (k = 0 mod 4); thetas in 1.0..1.08.  The temperature constituent, if
+    any, relaxes toward a constant 18 deg C with a small source (the equilibrium-temperature model).
+    Returns a dict of TransportBackend.set_kinetics_sources arguments."""
+    rng = np.random.default_rng(seed + 130363)
+    K = len(kin["decay_per_day"])
+    temperature_k = kin["temperature_k"]
+    lo, hi = rate_range
+    source, exchange = np.zeros(K), np.zeros(K)
+    source_theta, exchange_theta = 1.0 + 0.08 * rng.random(K), 1.0 + 0.08 * rng.random(K)
+    equilibrium, kind = np.zeros(K), np.zeros(K, np.int32)
+    for k in range(K):
+        if k == temperature_k:
+            exchange[k] = lo + (hi - lo) * rng.random()
+            equilibrium[k] = 18.0
+            source[k] = 0.5 * lo * (rng.random() - 0.5)
+            continue
+        source[k] = (5.0 + 45.0 * rng.random()) * (lo + (hi - lo) * rng.random()) * (-1.0 if k % 2 else 1.0)
+        if k % 2 == 0:
+            exchange[k] = lo + (hi - lo) * rng.random()
+            if k % 4 == 2 or K == 1:
+                kind[k] = 1
+            else:
+                equilibrium[k] = 5.0 + 40.0 * rng.random()
+    return dict(source_per_day=source, source_theta=source_theta, exchange_per_day=exchange, exchange_theta=exchange_theta,
+                equilibrium=equilibrium, equilibrium_kind=kind)

@@ -278,9 +278,10 @@ class ClearwaterRiverine:
             self.backend.fetch_wait()
 
     def set_kinetics(self, spec: Optional[Dict[str, Dict[str, Any]]], temperature: str | float = 20.0):
-        """First-order kinetics applied on the device in every later step, after the update_concentration override and
-        before transport (kinetics.py: spec format; temperature is a constituent name or a constant in deg C).
-        None switches kinetics off.  History rows are not rewritten: the reaction of step t shows in row t + 1."""
+        """Kinetics applied on the device in every later step, after the update_concentration override and before
+        transport: first-order decay and yields, then zero-order sources and relaxation toward an equilibrium such as
+        reaeration toward oxygen saturation (kinetics.py: spec format; temperature is a constituent name or a constant
+        in deg C).  None switches kinetics off.  History rows are not rewritten: the reaction of step t shows in row t + 1."""
         from .kinetics import compile_kinetics
         if spec is None:
             self.backend.set_kinetics(None)
@@ -288,6 +289,8 @@ class ClearwaterRiverine:
             return
         kin = compile_kinetics(spec, self.constituents, temperature)
         self.backend.set_kinetics(kin.decay_per_day, kin.theta, kin.yields, kin.temperature_k, kin.temperature_c)
+        if kin.has_sources:
+            self.backend.set_kinetics_sources(**kin.sources_arguments())
         self.kinetics = kin
 
     def sync(self):
@@ -299,8 +302,9 @@ class ClearwaterRiverine:
         of the reference's `_mass_bal_global` (postproc_util.py:21-166) under the same names -- Vol/Mass at the start and
         now, per boundary line the water volume and constituent mass that crossed it (total, in <= 0, out >= 0), the
         totals over all lines and the closure errors.  Nothing of it needs the (T,E) flux history on the host: the
-        per-face running sums are kept by the mass-flux kernel.  boundary_faces: {line name: face (edge) ids}; default:
-        the lines of the HEC-RAS plan the model was built from."""
+        per-face running sums are kept by the mass-flux kernel.  While kinetics is set, `reaction_mass` (what decay,
+        yields, sources and exchange formed) is reported and counted in mass_end_calc.  boundary_faces: {line name:
+        face (edge) ids}; default: the lines of the HEC-RAS plan the model was built from."""
         if boundary_faces is None:
             bd = getattr(self, "boundary_data", None)
             if bd is None:
@@ -330,7 +334,7 @@ class ClearwaterRiverine:
         out["bcTotalMassInOutAll"], out["bcTotalMassInAll"], out["bcTotalMassOutAll"] = tm, tm_in, tm_out
         out["vol_end_calc"] = out["Vol_start"] - tv_in - tv_out
         out["mass_end_calc"] = out["Mass_start"] - tm_in - tm_out
-        if self.kinetics is not None:                         # mass the reactions formed (< 0: lost) since the start
+        if self.kinetics is not None:                         # mass the reactions, sources and exchange formed (< 0: lost)
             out["reaction_mass"] = self.backend.reaction_mass(k)
             out["mass_end_calc"] += out["reaction_mass"]
         out["error_vol"] = out["vol_end_calc"] - out["Vol_end"]

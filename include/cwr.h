@@ -204,22 +204,42 @@ int cwr_get_volume_sums(cwr_handle* h, double* total_sum, double* in_sum, double
 /* --- first-order kinetics (decay with temperature correction, transformation chains) ---------------------------------
  * Step t first forms c~ as without kinetics: c[t], or the cwr_set_state override, with the non-zero real-cell entries of
  * input_array[t] merged in.  With kinetics set, every real cell i is then reacted before the load term V[t] c~ / dt is formed:
- *     T_i = temperature_c, or c~ of constituent temperature_k in cell i
+ *     T_i = temperature_c, or c~ of constituent temperature_k in cell i before any reaction of the step
  *     for k in topological order of the yield graph:
  *         r = decay_k * theta_k^(T_i - 20) / 86400          (decay in 1/day; theta^x = exp(x log theta))
  *         loss = c~_k * (-expm1(-r dt[t]));  c~_k -= loss;  c~_j += yields[j, k] * loss for every j
+ *     then, with cwr_set_kinetics_sources, for every column k with a source or exchange term, in ascending k:
+ *         s   = source_k * source_theta_k^(T_i - 20) / 86400        (concentration units per second; may be < 0)
+ *         r   = exchange_k * exchange_theta_k^(T_i - 20) / 86400    (1/s, >= 0)
+ *         ceq = equilibrium_k (kind 0) | O2sat(T_i) (kind 1, mg/L)
+ *         phi = -expm1(-r dt[t]) / r, or dt[t] when r == 0
+ *         c~_k += (s + r (ceq - c~_k)) * phi                        (exact solution of dc/dt = s + r (ceq - c) over dt)
  * and the rest of the step (ghost terms, warm start, solve, BC re-imposition, mass flux) takes the reacted c~'.  History
  * rows are not rewritten: c[t] stays what transport or the override produced; the reaction of step t shows in c[t+1].
  * Ghost cells and BC values are not reacted; nothing is clamped.  Rates are per column (a scenario ensemble may sweep them).
+ * O2sat is the APHA / Benson-Krause freshwater saturation at 1 atm, Ta = T + 273.15 K:
+ *     ln O2sat = -139.34411 + 1.575701e5/Ta - 6.642308e7/Ta^2 + 1.243800e10/Ta^3 - 8.621949e11/Ta^4
  *
  * decay_per_day (K) or NULL = kinetics off; theta (K) or NULL = all 1; yields (K,K) row-major,
  * yields[j*K + k] = mass of j formed per mass of k decayed, or NULL = none; temperature_k = index of the
  * temperature constituent or -1 for the constant temperature_c.  Takes effect for steps queued after the call
- * (stream-ordered upload).  CWR_EINVAL for a negative or non-finite decay, theta <= 0 or non-finite, a non-finite yield
- * or yields[k*K + k] != 0, a cycle in the yield graph, a temperature constituent that decays or receives a yield, an
- * index out of range.  Domain decomposition: every rank makes the same call. */
+ * (stream-ordered upload) and clears the sources.  CWR_EINVAL for a negative or non-finite decay, theta <= 0 or
+ * non-finite, a non-finite yield or yields[k*K + k] != 0, a cycle in the yield graph, a temperature constituent that
+ * decays or receives a yield, an index out of range.  Domain decomposition: every rank makes the same call. */
 int cwr_set_kinetics(cwr_handle* h, const double* decay_per_day, const double* theta, const double* yields,
                      int temperature_k, double temperature_c);
+/* Zero-order sources and relaxation toward an equilibrium (reaeration, equilibrium temperature), applied after the
+ * first-order chain of the kinetics set last (see above); all arrays (K).  source_per_day (concentration units per day)
+ * or NULL = none; exchange_per_day (1/day) or NULL = none; both NULL = sources off; a theta NULL = all 1; equilibrium
+ * (the constant target of kind 0); equilibrium_kind 0 = constant, 1 = O2sat(T), or NULL = all 0.  Acts only while
+ * kinetics is set (all-zero decay rates are allowed); cwr_set_kinetics clears it.  Stream-ordered upload.  CWR_EINVAL
+ * when kinetics is not set, for a non-finite source, a theta <= 0 or non-finite, a negative or non-finite exchange, a kind
+ * other than 0 or 1, exchange without equilibrium, a non-finite equilibrium of a kind-0 column with exchange > 0, or kind 1
+ * on the temperature constituent.  The reaction mass includes these terms.  Domain decomposition: every rank makes the
+ * same call. */
+int cwr_set_kinetics_sources(cwr_handle* h, const double* source_per_day, const double* source_theta,
+                             const double* exchange_per_day, const double* exchange_theta,
+                             const double* equilibrium, const int* equilibrium_kind);
 /* Reaction mass of constituent k, sum over the steps taken of sum_i V[t]_i (c~'_ik - c~_ik), reduced on the device in a fixed
  * order (the same bits every run): a running sum since cwr_create, 0 while kinetics was never set.  Domain decomposition:
  * the partial sum over the rows the rank owns (as cwr_mass_totals_at). */

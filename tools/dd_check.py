@@ -8,8 +8,9 @@ Every rank builds the same synthetic mesh, owns one strip of it and steps; the m
 compared with (a) the oracle (reference arithmetic incl. SuperLU, on rank 0; rtol 1e-9 per step as in
 tests/test_gpu_parity.py) and (b) a single-GPU run of the same library on rank 0's GPU.  Mass totals and
 boundary flux sums are checked as sums of the per-rank partial values.  --kinetics: the same with a first-order
-network (synthetic.make_kinetics) reacted on the device, the oracle being oracle.kinetics.KineticsRiverine, and the
-ranks' reaction masses summed against the single-GPU ones.  Prints one JSON line per case on
+network (synthetic.make_kinetics) reacted on the device, in every other case with sources and exchange as well
+(synthetic.make_kinetics_sources), the oracle being oracle.kinetics_sources.KineticsRiverine, and the ranks' reaction
+masses summed against the single-GPU ones.  Prints one JSON line per case on
 rank 0; exit code 0 only if every check passed on every rank.
 """
 from __future__ import annotations
@@ -32,14 +33,15 @@ def main():
     ap.add_argument("--K", type=int, default=3)
     ap.add_argument("--steps", type=int, default=6)
     ap.add_argument("--no-oracle", action="store_true")
-    ap.add_argument("--kinetics", action="store_true", help="react a first-order network on the device in every step")
+    ap.add_argument("--kinetics", action="store_true",
+                    help="react a first-order network on the device in every step, with sources and exchange in every other case")
     args = ap.parse_args()
     import torch
     import torch.distributed as dist
     from clearwater_riverine_b200 import TransportBackend, synthetic
     from clearwater_riverine_b200.domain import DomainDecomposedBackend, merge_owned
     from oracle import reference_step as ref
-    from oracle.kinetics import KineticsRiverine
+    from oracle.kinetics_sources import KineticsRiverine
 
     rank, world, local = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"]), int(os.environ["LOCAL_RANK"])
     torch.cuda.set_device(local)
@@ -57,9 +59,11 @@ def main():
         adv, _, _, cdiff, dt = ref.derive_coefficients(plan.face_flow, plan.edge_velocity, plan.face_x, plan.face_y,
                                                        plan.f1, plan.f2, D, plan.time_seconds)
         inputs = synthetic.make_inputs(plan, K, seed=40 + ci)
-        kin = None
+        kin = src = None
         if args.kinetics:
             inputs, kin = synthetic.make_kinetics(inputs, seed=40 + ci)
+            if ci % 2:
+                src = synthetic.make_kinetics_sources(kin, seed=40 + ci)
         be = DomainDecomposedBackend(plan.f1, plan.f2, plan.n_face, T, K, D, rank, world, device=local, **opts)
         be.set_hydro(0, adv, cdiff, plan.edge_velocity, plan.volume, dt)
         info = be.attach()
@@ -67,6 +71,8 @@ def main():
             be.set_inputs(k, inputs[k])
         if kin is not None:
             be.set_kinetics(**kin)
+        if src is not None:
+            be.set_kinetics_sources(**src)
         single = oracle = None
         if rank == 0:
             single = TransportBackend(plan.f1, plan.f2, plan.n_face, T, K, D, device=local, solver_path=1,
@@ -76,6 +82,8 @@ def main():
                 single.set_inputs(k, inputs[k])
             if kin is not None:
                 single.set_kinetics(**kin)
+            if src is not None:
+                single.set_kinetics_sources(**src)
             if not args.no_oracle:
                 mesh = ref.HydroMesh(plan.f1, plan.f2, plan.n_face, adv, cdiff, plan.edge_velocity, plan.volume, dt, D)
                 named = {f"c{k}": inputs[k] for k in range(K)}
@@ -83,7 +91,8 @@ def main():
                     oracle = ref.OracleRiverine(mesh, named)
                 else:
                     temperature = f"c{kin['temperature_k']}" if kin["temperature_k"] >= 0 else kin["temperature_c"]
-                    oracle = KineticsRiverine(mesh, named, kin["decay_per_day"], kin["theta"], kin["yields"], temperature)
+                    oracle = KineticsRiverine(mesh, named, kin["decay_per_day"], kin["theta"], kin["yields"], temperature,
+                                              **(src or {}))
         worst_oracle = worst_single = 0.0
         iters = []
         status = 0
@@ -126,6 +135,7 @@ def main():
                     "mass_end_rel_diff": mass_err, "boundary_flux_sums_rel_diff": flux_err, "ok": bool(ok)}
             if kin is not None:
                 line["reaction_mass_rel_diff"] = rmass_err
+                line["sources"] = src is not None
             single.close()
         flag = torch.tensor([1 if ok else 0], device="cuda")
         dist.all_reduce(flag, op=dist.ReduceOp.MIN)

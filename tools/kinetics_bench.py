@@ -11,7 +11,11 @@ CWR_FAM_RHS profile family (k_rhs + k_boundary_rhs + k_react), also with the sam
 over that time against a device-to-device copy's rate.  Ohio-shaped mesh, K = 1 and 64 scenarios with 64 decay rates:
 the time kinetics adds per step in cwr_run.  The coupled loop both ways at both sizes: the same reactions on the host
 (every constituent copied down, reacted in numpy, pushed back through the update_concentration override) against the
-device kinetics.  Prints one JSON object and writes it to --out.
+device kinetics.  With sources (cwr_set_kinetics_sources), 1M x 16: the same network with the zero-order sources and
+exchange of synthetic.make_kinetics_sources (sediment-oxygen-demand-like sinks, reaeration toward oxygen saturation, an
+equilibrium temperature), with the temperature constituent and at a constant temperature, each against the same network
+without its sources, alternately on the same handle: the step time and k_react's time (the CWR_FAM_RHS delta).
+Prints one JSON object and writes it to --out.
 """
 from __future__ import annotations
 
@@ -82,6 +86,25 @@ def alternate(torch, be, kin, fn, reps, n):
         be.set_kinetics(**kin)
         on.append(timed(torch, be, fn, n))
     return float(np.median(off)), float(np.median(on))
+
+
+def alternate_sources(torch, be, kin, src, step, reps):
+    """The network without and with its sources, alternately, reps times each: medians of the step time (ms, CUDA events)
+    and of the CWR_FAM_RHS family time (ms per step, in separate profiled steps)."""
+    out = {"step_ms": ([], []), "rhs_family_ms": ([], [])}
+    for _ in range(reps):
+        for i, with_src in enumerate((False, True)):
+            be.set_kinetics(**kin)
+            if with_src:
+                be.set_kinetics_sources(**src)
+            step()
+            out["step_ms"][i].append(timed(torch, be, step, 5))
+            be.profile(1)
+            for _ in range(5):
+                step()
+            out["rhs_family_ms"][i].append(be.profile(-1)["rhs"][0] / 5)
+            be.profile(0)
+    return {f"{key}_{name}": float(np.median(v[i])) for key, v in out.items() for i, name in enumerate(("without", "with"))}
 
 
 def host_loop(be, kin, t0, steps, dt):
@@ -155,6 +178,16 @@ def main():
                    "k_react_of_copy_rate": nbytes / (react_ms * 1e-3) / 1e9 / res["d2d_copy_gbs"],
                    "k_react_ms_constant_temperature": react_const_ms,
                    "k_react_of_copy_rate_constant_temperature": nbytes / (react_const_ms * 1e-3) / 1e9 / res["d2d_copy_gbs"]}
+    # the same network with its sources, and at a constant temperature (s, r ceq and phi once per CTA)
+    src = synthetic.make_kinetics_sources(kin, seed=0, rate_range=(0.05, 2.0))
+    for key, k in (("1m16_sources", kin), ("1m16_sources_constant_temperature", kin_const)):
+        r = alternate_sources(torch, be, k, src, step, args.reps)
+        r["k_react_added_ms"] = r["rhs_family_ms_with"] - r["rhs_family_ms_without"]
+        r["step_added_ms"] = r["step_ms_with"] - r["step_ms_without"]
+        r["k_react_ms_without_sources"] = r["rhs_family_ms_without"] - fam["off"]
+        r["k_react_ms_with_sources"] = r["rhs_family_ms_with"] - fam["off"]
+        r["source_columns"] = int(np.count_nonzero((src["source_per_day"] != 0) | (src["exchange_per_day"] != 0)))
+        res[key] = r
     steps = 8
     res["1m16"]["coupled_host_ms_per_step"] = 1e3 * host_loop(be, kin, 4, steps, 30.0)
     res["1m16"]["coupled_device_ms_per_step"] = 1e3 * device_loop(torch, be, kin, 4, steps)
