@@ -104,6 +104,7 @@ def load_library():
         "cwr_get_volume_sums": ([H, dp, dp, dp], C.c_int),
         "cwr_set_kinetics": ([H, dp, dp, dp, C.c_int, C.c_double], C.c_int),
         "cwr_set_kinetics_sources": ([H, dp, dp, dp, dp, dp, ip], C.c_int),
+        "cwr_set_kinetics_limits": ([H, C.c_int, ip, ip, ip, ip, dp], C.c_int),
         "cwr_get_reaction_mass": ([H, C.c_int, dp], C.c_int),
         "cwr_get_lhs": ([H, C.POINTER(C.c_int64), ip, ip, dp], C.c_int),
         "cwr_get_rhs": ([H, C.c_int, dp], C.c_int),
@@ -414,8 +415,8 @@ class TransportBackend:
         """First-order decay / transformations applied on the device in every later step (cwr_set_kinetics):
         decay_per_day (K,) or None = off; theta (K,) or None = all 1; yields (K, K), yields[j, k] = mass of j formed per
         mass of k decayed, or None; temperature_k = temperature constituent or -1 for the constant temperature_c (deg C).
-        An invalid set raises ValueError; any call clears set_kinetics_sources.  kinetics.compile_kinetics builds the
-        arrays from a by-name spec."""
+        An invalid set raises ValueError; any call clears set_kinetics_sources and set_kinetics_limits.
+        kinetics.compile_kinetics builds the arrays from a by-name spec."""
         if decay_per_day is None:
             self._check(self._lib.cwr_set_kinetics(self._h, None, None, None, -1, 20.0))
             return
@@ -434,13 +435,31 @@ class TransportBackend:
         last (cwr_set_kinetics_sources): dc/dt = s + r (ceq - c) per column, solved exactly over each step.
         source_per_day (K,) or None; exchange_per_day (K,) 1/day or None (both None: sources off); a theta (K,) or None =
         all 1; equilibrium (K,) the constant targets; equilibrium_kind (K,) 0 = constant, 1 = oxygen saturation at T, or
-        None = all 0.  set_kinetics clears them.  An invalid set raises ValueError."""
+        None = all 0.  set_kinetics clears them; any call clears set_kinetics_limits.  An invalid set raises ValueError."""
         K = (self.K,)
         f = lambda a, name: None if a is None else _arr(a, np.float64, K, name)
         arrs = [f(source_per_day, "source_per_day"), f(source_theta, "source_theta"), f(exchange_per_day, "exchange_per_day"),
                 f(exchange_theta, "exchange_theta"), f(equilibrium, "equilibrium")]
         kind = None if equilibrium_kind is None else _arr(equilibrium_kind, np.int32, K, "equilibrium_kind")
         rc = self._lib.cwr_set_kinetics_sources(self._h, *[_ptr(a, C.c_double) for a in arrs], _ptr(kind, C.c_int32))
+        if rc == CWR_EINVAL:
+            raise ValueError(self._lib.cwr_last_error(self._h).decode())
+        self._check(rc)
+
+    def set_kinetics_limits(self, process=None, column=None, factor_column=None, factor_kind=None, half_saturation=None):
+        """Monod limitation and inhibition of the kinetics and sources set last (cwr_set_kinetics_limits); (n,) arrays:
+        factor i scales process[i] (0 = the decay of column[i], 1 = its source) by c+/(K + c+) (factor_kind 0) or
+        K/(K + c+) (1) of constituent factor_column[i], K = half_saturation[i], c+ = max(c, 0).  process None = limits
+        off.  set_kinetics and set_kinetics_sources clear them.  An invalid set raises ValueError."""
+        if process is None:
+            self._check(self._lib.cwr_set_kinetics_limits(self._h, 0, None, None, None, None, None))
+            return
+        pr = _arr(process, np.int32).reshape(-1)
+        n = (pr.shape[0],)
+        ints = [pr] + [_arr(a, np.int32, n, name) for a, name in ((column, "column"), (factor_column, "factor_column"),
+                                                                  (factor_kind, "factor_kind"))]
+        hs = _arr(half_saturation, np.float64, n, "half_saturation")
+        rc = self._lib.cwr_set_kinetics_limits(self._h, n[0], *[_ptr(a, C.c_int32) for a in ints], _ptr(hs, C.c_double))
         if rc == CWR_EINVAL:
             raise ValueError(self._lib.cwr_last_error(self._h).decode())
         self._check(rc)

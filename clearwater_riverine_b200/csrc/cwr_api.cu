@@ -119,6 +119,13 @@ struct cwr_handle {
     // sources and exchange (cwr_set_kinetics_sources): the listed columns in ascending order; kin_src_o2: one is kind 1
     int kin_srcs = 0, kin_src_o2 = 0;
     KinSrc* d_kin_srcs = nullptr;
+    // what cwr_set_kinetics_limits validates against: the decay rates and yields of the kinetics set last, the step of
+    // each decaying column and the list position of each source column (-1: none)
+    std::vector<double> kin_decay_h, kin_yields_h, kin_source_h;
+    std::vector<int> kin_step_of, kin_src_of;
+    // Monod factors (cwr_set_kinetics_limits): kin_facs entries, grouped per process by d_kin_fptr (n_steps + n_src + 1)
+    int kin_facs = 0;
+    KinFac* d_kin_facs = nullptr; int* d_kin_fptr = nullptr;
     // optional per-kernel-family timing with CUDA events on the handle's stream (bench.py roofline)
     bool profiling = false;
     std::vector<cudaEvent_t> ev_pool;
@@ -1340,9 +1347,10 @@ static int build_rhs(cwr_handle* h, int t, int accumulate) {
         // after cwr_set_kinetics), at most the resident grid; the same rows give the same grid, hence the same sums
         const int R = react_tile_rows(h->K);
         const int grid = grid_for((M.row_hi - M.row_lo + R - 1) / R, 1, h->kin_grid_max);
-        CK(launch_chain(h, k_react, grid, kThreads, react_smem_bytes(h->K) + react_src_smem_bytes(h->kin_srcs, h->kin_temp_k), M,
+        CK(launch_chain(h, h->kin_facs ? k_react<true> : k_react<false>, grid, kThreads, react_smem_bytes(h->K) + react_src_smem_bytes(h->kin_srcs, h->kin_temp_k), M,
                         (const KinStep*)h->d_kin_steps, h->kin_steps, (const KinYield*)h->d_kin_yields, h->kin_temp_k, h->kin_temp_c,
-                        (const KinSrc*)h->d_kin_srcs, h->kin_srcs, h->kin_src_o2, h->d_kin_partials, h->d_kin_state, accumulate));
+                        (const KinSrc*)h->d_kin_srcs, h->kin_srcs, h->kin_src_o2, (const KinFac*)h->d_kin_facs,
+                        (const int*)h->d_kin_fptr, h->d_kin_partials, h->d_kin_state, accumulate));
         h->launches += 1;
     }
     if (M.b_hi - M.b_lo > 0) {
@@ -1694,7 +1702,7 @@ int cwr_set_kinetics(cwr_handle* h, const double* decay, const double* theta, co
                      double temperature_c) {
     if (!h) return CWR_EINVAL;
     const int K = h->K;
-    if (!decay) { h->kin_on = false; h->kin_srcs = 0; return CWR_OK; }
+    if (!decay) { h->kin_on = false; h->kin_srcs = 0; h->kin_facs = 0; return CWR_OK; }
     for (int k = 0; k < K; ++k) {
         if (!std::isfinite(decay[k]) || decay[k] < 0.0) FAIL(CWR_EINVAL, "cwr_set_kinetics: decay rates must be finite and >= 0");
         if (theta && (!std::isfinite(theta[k]) || theta[k] <= 0.0)) FAIL(CWR_EINVAL, "cwr_set_kinetics: theta must be finite and > 0");
@@ -1743,17 +1751,22 @@ int cwr_set_kinetics(cwr_handle* h, const double* decay, const double* theta, co
     }
     CK(cudaSetDevice(h->device));
     if (!h->d_kin_state) {
-        cudaFuncAttributes fa{};
-        CK(cudaFuncGetAttributes(&fa, k_react));
-        if (fa.sharedSizeBytes > kReactStaticSmem) FAIL(CWR_ECUDA, "k_react: static shared memory exceeds what its tile sizing reserves");
+        cudaFuncAttributes fa{}, fl{};
+        CK(cudaFuncGetAttributes(&fa, k_react<false>));
+        CK(cudaFuncGetAttributes(&fl, k_react<true>));
+        if (std::max(fa.sharedSizeBytes, fl.sharedSizeBytes) > kReactStaticSmem)
+            FAIL(CWR_ECUDA, "k_react: static shared memory exceeds what its tile sizing reserves");
+        // the grid of both instantiations (k_react<true> may hold fewer CTAs per SM; its CTAs need not be co-resident)
         int occ = 0;
-        CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_react, kThreads, react_smem_bytes(K)));
+        CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_react<false>, kThreads, react_smem_bytes(K)));
         h->kin_grid_max = h->num_sms * std::max(1, occ);
         CK(dalloc(h, &h->d_kin_steps, (size_t)K));
         CK(dalloc(h, &h->d_kin_yields, (size_t)K * K));
         CK(dalloc(h, &h->d_kin_partials, (size_t)K * h->kin_grid_max));
         CK(dalloc(h, &h->d_kin_state, 1));
         CK(dalloc(h, &h->d_kin_srcs, (size_t)K));
+        CK(dalloc(h, &h->d_kin_facs, (size_t)4 * K * K));      // at most (decay | source) x column x factor column x kind
+        CK(dalloc(h, &h->d_kin_fptr, (size_t)2 * K + 1));
         CK(cudaMemsetAsync(h->d_kin_state, 0, sizeof(KinState), h->stream));
     }
     // stream-ordered: steps queued before this call still read the previous parameters (pageable sources: the copies
@@ -1765,6 +1778,14 @@ int cwr_set_kinetics(cwr_handle* h, const double* decay, const double* theta, co
     h->kin_temp_c = temperature_k < 0 ? temperature_c : 20.0;
     h->kin_on = true;
     h->kin_srcs = 0;
+    h->kin_facs = 0;
+    h->kin_decay_h.assign(decay, decay + K);
+    h->kin_yields_h.assign((size_t)K * K, 0.0);
+    if (yields) h->kin_yields_h.assign(yields, yields + (size_t)K * K);
+    h->kin_step_of.assign(K, -1);
+    for (size_t p = 0; p < steps.size(); ++p) h->kin_step_of[steps[p].col] = (int)p;
+    h->kin_source_h.assign(K, 0.0);
+    h->kin_src_of.assign(K, -1);
     return CWR_OK;
 }
 
@@ -1773,7 +1794,11 @@ int cwr_set_kinetics_sources(cwr_handle* h, const double* source_per_day, const 
     if (!h) return CWR_EINVAL;
     const int K = h->K;
     if (!h->kin_on) FAIL(CWR_EINVAL, "cwr_set_kinetics_sources: call cwr_set_kinetics first");
-    if (!source_per_day && !exchange_per_day) { h->kin_srcs = 0; return CWR_OK; }
+    if (!source_per_day && !exchange_per_day) {
+        h->kin_srcs = 0; h->kin_facs = 0;
+        h->kin_source_h.assign(K, 0.0); h->kin_src_of.assign(K, -1);
+        return CWR_OK;
+    }
     if (exchange_per_day && !equilibrium) FAIL(CWR_EINVAL, "cwr_set_kinetics_sources: exchange needs an equilibrium array");
     for (int k = 0; k < K; ++k) {
         const double s = source_per_day ? source_per_day[k] : 0.0, e = exchange_per_day ? exchange_per_day[k] : 0.0;
@@ -1809,11 +1834,66 @@ int cwr_set_kinetics_sources(cwr_handle* h, const double* source_per_day, const 
     // at a constant temperature the coefficients take shared memory beyond the tile's 48 KB (react_src_smem_bytes); the
     // limit is the same for every handle (the attribute is the kernel's, not the handle's)
     if (h->kin_temp_k < 0 && !list.empty())
-        CK(cudaFuncSetAttribute(k_react, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                (int)(kReactSmemLimit - kReactStaticSmem + react_src_smem_bytes(kMaxK, -1))));
+        for (auto* fn : {k_react<false>, k_react<true>})
+            CK(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                    (int)(kReactSmemLimit - kReactStaticSmem + react_src_smem_bytes(kMaxK, -1))));
     if (!list.empty()) CK(cudaMemcpyAsync(h->d_kin_srcs, list.data(), list.size() * sizeof(KinSrc), cudaMemcpyHostToDevice, h->stream));
     h->kin_srcs = (int)list.size();
     h->kin_src_o2 = o2;
+    h->kin_facs = 0;
+    h->kin_source_h.assign(K, 0.0);
+    h->kin_src_of.assign(K, -1);
+    for (size_t p = 0; p < list.size(); ++p) {
+        h->kin_source_h[list[p].col] = list[p].source;
+        h->kin_src_of[list[p].col] = (int)p;
+    }
+    return CWR_OK;
+}
+
+int cwr_set_kinetics_limits(cwr_handle* h, int n, const int* process, const int* column, const int* factor_column,
+                            const int* factor_kind, const double* half_saturation) {
+    if (!h) return CWR_EINVAL;
+    const int K = h->K;
+    if (!h->kin_on) FAIL(CWR_EINVAL, "cwr_set_kinetics_limits: call cwr_set_kinetics first");
+    if (n < 0) FAIL(CWR_EINVAL, "cwr_set_kinetics_limits: n must be >= 0");
+    if (n == 0 || !process || !column || !factor_column || !factor_kind || !half_saturation) { h->kin_facs = 0; return CWR_OK; }
+    std::vector<long long> seen;
+    for (int i = 0; i < n; ++i) {
+        const int pr = process[i], k = column[i], j = factor_column[i], kind = factor_kind[i];
+        const double half = half_saturation[i];
+        if (pr != 0 && pr != 1) FAIL(CWR_EINVAL, "cwr_set_kinetics_limits: process must be 0 (decay) or 1 (source)");
+        if (kind != 0 && kind != 1) FAIL(CWR_EINVAL, "cwr_set_kinetics_limits: factor_kind must be 0 (limitation) or 1 (inhibition)");
+        if (k < 0 || k >= K || j < 0 || j >= K) FAIL(CWR_EINVAL, "cwr_set_kinetics_limits: column index out of range");
+        if (!std::isfinite(half) || half <= 0.0) FAIL(CWR_EINVAL, "cwr_set_kinetics_limits: half-saturations must be finite and > 0");
+        if (pr == 0 && h->kin_decay_h[k] == 0.0) FAIL(CWR_EINVAL, "cwr_set_kinetics_limits: a decay factor on a column that does not decay");
+        if (pr == 1 && h->kin_source_h[k] == 0.0) FAIL(CWR_EINVAL, "cwr_set_kinetics_limits: a source factor on a column without a source");
+        if (pr == 0 && j == k) FAIL(CWR_EINVAL, "cwr_set_kinetics_limits: a decay cannot be limited or inhibited by its own column");
+        if (pr == 1 && j == k && (kind != 0 || h->kin_source_h[k] >= 0.0))
+            FAIL(CWR_EINVAL, "cwr_set_kinetics_limits: only a sink (source < 0) can be limited by its own column");
+        seen.push_back((((long long)pr * K + k) * K + j) * 2 + kind);
+    }
+    std::sort(seen.begin(), seen.end());
+    if (std::adjacent_find(seen.begin(), seen.end()) != seen.end())
+        FAIL(CWR_EINVAL, "cwr_set_kinetics_limits: the same (process, column, factor column, kind) given twice");
+    // grouped per process (the decay steps in their order, then the source columns in theirs), each in the order given
+    const int n_proc = h->kin_steps + h->kin_srcs;
+    std::vector<std::vector<KinFac>> per(n_proc);
+    for (int i = 0; i < n; ++i) {
+        const int k = column[i], j = factor_column[i];
+        const int q = process[i] == 0 ? h->kin_step_of[k] : h->kin_steps + h->kin_src_of[k];
+        KinFac a{};
+        a.col = j; a.kind = factor_kind[i]; a.half = half_saturation[i];
+        const double y = h->kin_yields_h[(size_t)j * K + k];
+        a.use = process[i] == 0 && a.kind == 0 && y < 0.0 ? -y : 0.0;
+        per[q].push_back(a);
+    }
+    std::vector<KinFac> list;
+    std::vector<int> ptr(1, 0);
+    for (const auto& v : per) { list.insert(list.end(), v.begin(), v.end()); ptr.push_back((int)list.size()); }
+    CK(cudaSetDevice(h->device));
+    CK(cudaMemcpyAsync(h->d_kin_facs, list.data(), list.size() * sizeof(KinFac), cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(h->d_kin_fptr, ptr.data(), ptr.size() * sizeof(int), cudaMemcpyHostToDevice, h->stream));
+    h->kin_facs = (int)list.size();
     return CWR_OK;
 }
 

@@ -541,12 +541,34 @@ __device__ __forceinline__ void grid_totals(const double* partials, double* tot,
 //     s = source_k theta_s^(T - 20) / 86400,  r = exchange_k theta_e^(T - 20) / 86400,  ceq = equilibrium_k | O2sat(T)
 //     phi = -expm1(-r dt) / r (dt when r == 0),  c~_k += (s + r ceq - r c~_k) phi
 // the exact solution of dc/dt = s + r (ceq - c) over dt.  T is the value before any of the step's reactions.
+// Monod factors (cwr_set_kinetics_limits) scale a process -- the decay of step p or the source of source column p -- by
+// M = prod f in the order given, f = c+_j / (K + c+_j) (limitation) or K / (K + c+_j) (inhibition), c+ = max(c, 0), with
+// c_j as the row holds it when the process is applied:
+//     decay:   loss = c~_k * (-expm1(-r M dt)), then loss = min(loss, c+_j / -yield[j,k]) for every limitation on a j the
+//              process consumes (KinFac.use > 0), the quotient rounded toward -inf so that c~_j + yield[j,k] * loss >= 0
+//              holds in floating point for any yield; c~_k and the yields as above
+//     source:  s M in place of s; a limitation on the column itself (a sink only) is the first-order sink
+//              a = -s M' / (K + c+_k) (M': the other factors), c~_k += (r ceq - (r + a) c~_k) phi(r + a)
+// Process q's factors are fl[fptr[q], fptr[q + 1]), q = p for step p and n_steps + p for source column p.  A process with
+// factors is evaluated per row (at a constant temperature too); the others take exactly the unfactored code.  Only
+// k_react<true> (launched while factors are set) has the factored code: k_react<false> keeps the registers, hence the
+// occupancy and the grid (kin_grid_max), that it has without it, and both take that grid, so the column sums of the
+// reaction mass are added in the same order with or without factors.
 // ---------------------------------------------------------------------------------------------
 struct KinStep { int col, y_begin, y_end, pad; double decay, log_theta; };   // a reacting constituent; its yields
 struct KinYield { int col, pad; double y; };                                 // [y_begin, y_end)
 struct KinState { unsigned ticket; int pad; double mass[kMaxK]; };           // last-CTA ticket, running reaction mass
 // a column with a source or exchange term; kind 1: ceq = O2sat(T) (listed only with exchange > 0), kind 0: ceq = equilibrium
 struct KinSrc { int col, kind; double source, log_source_theta, exchange, log_exchange_theta, equilibrium; };
+// a Monod factor on column col: kind 0 limitation, 1 inhibition; half: K > 0; use: -yield[col, k] of a decay process that
+// consumes col and is limited by it (the cap), else 0
+struct KinFac { int col, kind; double half, use; };
+
+// c+_j / (K + c+_j) or K / (K + c+_j)
+__device__ __forceinline__ double monod(const KinFac& a, double cj) {
+    const double cp = fmax(cj, 0.0);
+    return (a.kind ? a.half : cp) / (a.half + cp);
+}
 
 // Dissolved-oxygen saturation (mg/L) of fresh water at 1 atm, T in deg C (APHA / Benson-Krause), as written: no clamp
 __device__ __forceinline__ double o2_saturation(double T) {
@@ -560,6 +582,48 @@ __device__ __forceinline__ void kin_src_coef(const KinSrc& s, double T, double o
     r = s.exchange * exp(dT * s.log_exchange_theta) / 86400.0;
     sr = s.source * exp(dT * s.log_source_theta) / 86400.0 + r * (s.kind ? o2 : s.equilibrium);
     phi = r > 0.0 ? -expm1(-r * dt) / r : dt;
+}
+
+// The loss of decay step s with its nf factors a[] (the row c as it is now)
+__device__ __forceinline__ double kin_decay_limited(const double* c, const KinStep& s, const KinFac* __restrict__ a, int nf,
+                                                 double T, double dt) {
+    const double r = s.decay * exp((T - 20.0) * s.log_theta) / 86400.0;
+    double m = 1.0;
+    for (int q = 0; q < nf; ++q) {
+        const KinFac f = a[q];
+        m *= monod(f, c[f.col]);
+    }
+    double loss = c[s.col] * (-expm1(-(r * m) * dt));
+    for (int q = 0; q < nf; ++q) {
+        const KinFac f = a[q];
+        if (f.use > 0.0) loss = fmin(loss, __ddiv_rd(fmax(c[f.col], 0.0), f.use));   // rounded down: use * cap <= c+_j
+    }
+    return loss;
+}
+
+// Source column *sp with its nf factors a[] applied to the row c (o2 = O2sat(T), read only for kind 1)
+__device__ __forceinline__ void kin_src_limited(double* c, const KinSrc* __restrict__ sp, const KinFac* __restrict__ a, int nf,
+                                             double T, double o2, double dt) {
+    const KinSrc s = *sp;
+    const double dT = T - 20.0;
+    const double r = s.exchange * exp(dT * s.log_exchange_theta) / 86400.0;
+    const double src = s.source * exp(dT * s.log_source_theta) / 86400.0;
+    const double req = r * (s.kind ? o2 : s.equilibrium);
+    double m = 1.0, self_half = 0.0;
+    for (int q = 0; q < nf; ++q) {
+        const KinFac f = a[q];
+        if (f.col == s.col) self_half = f.half;   // the self-limitation of a sink (K > 0)
+        else m *= monod(f, c[f.col]);
+    }
+    double& v = c[s.col];
+    if (self_half > 0.0) {
+        const double rr = r + -src * m / (self_half + fmax(v, 0.0));
+        const double phi = rr > 0.0 ? -expm1(-rr * dt) / rr : dt;
+        v += (req - rr * v) * phi;
+    } else {
+        const double phi = r > 0.0 ? -expm1(-r * dt) / r : dt;
+        v += (src * m + req - r * v) * phi;
+    }
 }
 
 // Shared memory of k_react: st[kMaxK] and last_block_arrives' flag (static, kReactStaticSmem bounds them), then the dynamic
@@ -602,9 +666,11 @@ __device__ __forceinline__ void react_pairs(const double* base, int cnt, F f) {
     }
 }
 
+template <bool kLimited>
 __global__ void __launch_bounds__(kThreads) k_react(DeviceModel M, const KinStep* __restrict__ steps, int n_steps,
                                                     const KinYield* __restrict__ yl, int temp_k, double temp_c,
                                                     const KinSrc* __restrict__ srcs, int n_src, int src_o2,
+                                                    const KinFac* __restrict__ fl, const int* __restrict__ fptr,
                                                     double* __restrict__ partials, KinState* __restrict__ ks, int accumulate) {
     extern __shared__ double rs[];
     __shared__ KinStep st[kMaxK];
@@ -654,15 +720,36 @@ __global__ void __launch_bounds__(kThreads) k_react(DeviceModel M, const KinStep
             const double T = temp_k < 0 ? temp_c : c[temp_k];
             for (int p = 0; p < n_steps; ++p) {
                 const KinStep& s = st[p];
-                const double f = temp_k < 0 ? fac[p] : -expm1(-(s.decay * exp((T - 20.0) * s.log_theta) / 86400.0) * dt);
-                const double loss = c[s.col] * f;
+                const int fb = kLimited ? fptr[p] : 0, fe = kLimited ? fptr[p + 1] : 0;
+                double loss;
+                if (fb == fe) {
+                    const double f = temp_k < 0 ? fac[p] : -expm1(-(s.decay * exp((T - 20.0) * s.log_theta) / 86400.0) * dt);
+                    loss = c[s.col] * f;
+                } else loss = kin_decay_limited(c, s, fl + fb, fe - fb, T, dt);
                 c[s.col] -= loss;
                 for (int q = s.y_begin; q < s.y_end; ++q) {
                     const KinYield y = yl[q];
                     c[y.col] += y.y * loss;
                 }
             }
-            if (temp_k < 0) {
+            if (kLimited) {                   // factored source columns per row; the others as below
+                const double o2 = src_o2 ? o2_saturation(T) : 0.0;
+                for (int p = 0; p < n_src; ++p) {
+                    const int fb = fptr[n_steps + p], fe = fptr[n_steps + p + 1];
+                    if (fb != fe) {
+                        kin_src_limited(c, srcs + p, fl + fb, fe - fb, T, o2, dt);
+                    } else if (temp_k < 0) {
+                        const double* q = sco + 3 * p;
+                        double& v = c[srcs[p].col];
+                        v += (q[0] - q[1] * v) * q[2];
+                    } else {
+                        double sr, r, phi;
+                        kin_src_coef(srcs[p], T, o2, dt, sr, r, phi);
+                        double& v = c[srcs[p].col];
+                        v += (sr - r * v) * phi;
+                    }
+                }
+            } else if (temp_k < 0) {
                 for (int p = 0; p < n_src; ++p) {
                     const double* q = sco + 3 * p;
                     double& v = c[srcs[p].col];

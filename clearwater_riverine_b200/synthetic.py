@@ -353,3 +353,35 @@ def make_kinetics_sources(kin: dict, *, seed: int = 0, rate_range=(20.0, 200.0))
                 equilibrium[k] = 5.0 + 40.0 * rng.random()
     return dict(source_per_day=source, source_theta=source_theta, exchange_per_day=exchange, exchange_theta=exchange_theta,
                 equilibrium=equilibrium, equilibrium_kind=kind)
+
+
+def make_kinetics_limits(kin: dict, src: Optional[dict] = None, *, seed: int = 0) -> dict:
+    """Seeded Monod factors for a network of make_kinetics (kin) and make_kinetics_sources (src, or None), in the manner
+    of a BOD-DO-nitrogen model: every decay that consumes a constituent (a negative yield) is limited by it (K in
+    0.05..0.5, so that the decay is capped where the consumed constituent runs out), every sink is limited by its own
+    constituent (sediment-oxygen-demand-like, K in 0.5..2), the decay of every reacting k = 1 mod 3 is inhibited by
+    constituent k + 1 (denitrification-like, K in 5..50) and the positive source of every k = 0 mod 4 by constituent
+    k + 2, when they exist.  A network without a consuming decay or a sink (K = 1 with a positive source) gets no factor.
+    Returns a dict of TransportBackend.set_kinetics_limits arguments."""
+    rng = np.random.default_rng(seed + 160183)
+    decay, yields = np.asarray(kin["decay_per_day"]), np.asarray(kin["yields"])
+    K = len(decay)
+    source = np.zeros(K) if src is None or src.get("source_per_day") is None else np.asarray(src["source_per_day"])
+    rows = []                                   # (process, column, factor column, kind, half-saturation)
+    for k in range(K):
+        if decay[k] == 0.0:
+            continue
+        for j in np.nonzero(yields[:, k] < 0.0)[0]:
+            rows.append((0, k, int(j), 0, 0.05 + 0.45 * rng.random()))
+    for k in range(K):
+        if source[k] < 0.0:
+            rows.append((1, k, k, 0, 0.5 + 1.5 * rng.random()))
+    for k in range(K):
+        if decay[k] != 0.0 and k % 3 == 1 and k + 1 < K:
+            rows.append((0, k, k + 1, 1, 5.0 + 45.0 * rng.random()))
+        if source[k] > 0.0 and k % 4 == 0 and k + 2 < K:
+            rows.append((1, k, k + 2, 1, 5.0 + 45.0 * rng.random()))
+    cols = list(zip(*rows)) if rows else [()] * 5
+    return dict(process=np.array(cols[0], np.int32), column=np.array(cols[1], np.int32),
+                factor_column=np.array(cols[2], np.int32), factor_kind=np.array(cols[3], np.int32),
+                half_saturation=np.array(cols[4], np.float64))

@@ -280,7 +280,8 @@ class ClearwaterRiverine:
     def set_kinetics(self, spec: Optional[Dict[str, Dict[str, Any]]], temperature: str | float = 20.0):
         """Kinetics applied on the device in every later step, after the update_concentration override and before
         transport: first-order decay and yields, then zero-order sources and relaxation toward an equilibrium such as
-        reaeration toward oxygen saturation (kinetics.py: spec format; temperature is a constituent name or a constant
+        reaeration toward oxygen saturation, each optionally scaled by Monod limitation and inhibition factors such as
+        oxygen limitation of BOD oxidation (kinetics.py: spec format; temperature is a constituent name or a constant
         in deg C).  None switches kinetics off.  History rows are not rewritten: the reaction of step t shows in row t + 1."""
         from .kinetics import compile_kinetics
         if spec is None:
@@ -291,6 +292,8 @@ class ClearwaterRiverine:
         self.backend.set_kinetics(kin.decay_per_day, kin.theta, kin.yields, kin.temperature_k, kin.temperature_c)
         if kin.has_sources:
             self.backend.set_kinetics_sources(**kin.sources_arguments())
+        if kin.has_limits:
+            self.backend.set_kinetics_limits(**kin.limits_arguments())
         self.kinetics = kin
 
     def sync(self):

@@ -216,14 +216,31 @@ int cwr_get_volume_sums(cwr_handle* h, double* total_sum, double* in_sum, double
  *         c~_k += (s + r (ceq - c~_k)) * phi                        (exact solution of dc/dt = s + r (ceq - c) over dt)
  * and the rest of the step (ghost terms, warm start, solve, BC re-imposition, mass flux) takes the reacted c~'.  History
  * rows are not rewritten: c[t] stays what transport or the override produced; the reaction of step t shows in c[t+1].
- * Ghost cells and BC values are not reacted; nothing is clamped.  Rates are per column (a scenario ensemble may sweep them).
+ * Ghost cells and BC values are not reacted; without Monod factors nothing is clamped.  Rates are per column (a scenario
+ * ensemble may sweep them).
+ * With cwr_set_kinetics_limits, a process (the decay of column k, or the source of column k) carries Monod factors on
+ * constituents j with half-saturations K > 0, c+ = max(c, 0):
+ *         limitation f = c+_j / (K + c+_j),  inhibition f = K / (K + c+_j),  M = product of the process's factors in the
+ *         order given, from 1.0
+ *     c_j is read as the row holds it when the process is applied (decays in the topological order above -- factors add no
+ *     edges to the yield graph --, then the source columns in ascending k); T is still the value before the reactions.
+ *     decay:  r_eff = r M;  loss = c~_k * (-expm1(-r_eff dt[t]));  for every limitation on a j the decay consumes
+ *             (yields[j, k] < 0): loss = min(loss, c+_j / -yields[j, k]), the quotient rounded toward -inf;  then c~_k
+ *             and the yields as above
+ *     source: a factor on another column: s M in place of s.  A limitation on the column itself (a sink, s < 0) is the
+ *             first-order sink a = -s M' / (K + c+_k) (M': the other factors), frozen at the value before the term:
+ *             c~_k += (r ceq - (r + a) c~_k) * phi, phi = -expm1(-(r + a) dt[t]) / (r + a), or dt[t] when r + a == 0
+ *     So a constituent stays >= 0 at every step size when it starts >= 0, every process that consumes it is limited by
+ *     it, its own sink is self-limited and its equilibrium is >= 0.  The cap holds exactly in floating point for any
+ *     yield: the rounded-down quotient keeps -yields[j, k] * loss <= c+_j.  This covers the reaction; transport adds
+ *     only solver-tolerance noise.  Processes without factors are computed exactly as without cwr_set_kinetics_limits.
  * O2sat is the APHA / Benson-Krause freshwater saturation at 1 atm, Ta = T + 273.15 K:
  *     ln O2sat = -139.34411 + 1.575701e5/Ta - 6.642308e7/Ta^2 + 1.243800e10/Ta^3 - 8.621949e11/Ta^4
  *
  * decay_per_day (K) or NULL = kinetics off; theta (K) or NULL = all 1; yields (K,K) row-major,
  * yields[j*K + k] = mass of j formed per mass of k decayed, or NULL = none; temperature_k = index of the
  * temperature constituent or -1 for the constant temperature_c.  Takes effect for steps queued after the call
- * (stream-ordered upload) and clears the sources.  CWR_EINVAL for a negative or non-finite decay, theta <= 0 or
+ * (stream-ordered upload) and clears the sources and the limits.  CWR_EINVAL for a negative or non-finite decay, theta <= 0 or
  * non-finite, a non-finite yield or yields[k*K + k] != 0, a cycle in the yield graph, a temperature constituent that
  * decays or receives a yield, an index out of range.  Domain decomposition: every rank makes the same call. */
 int cwr_set_kinetics(cwr_handle* h, const double* decay_per_day, const double* theta, const double* yields,
@@ -232,7 +249,8 @@ int cwr_set_kinetics(cwr_handle* h, const double* decay_per_day, const double* t
  * first-order chain of the kinetics set last (see above); all arrays (K).  source_per_day (concentration units per day)
  * or NULL = none; exchange_per_day (1/day) or NULL = none; both NULL = sources off; a theta NULL = all 1; equilibrium
  * (the constant target of kind 0); equilibrium_kind 0 = constant, 1 = O2sat(T), or NULL = all 0.  Acts only while
- * kinetics is set (all-zero decay rates are allowed); cwr_set_kinetics clears it.  Stream-ordered upload.  CWR_EINVAL
+ * kinetics is set (all-zero decay rates are allowed); cwr_set_kinetics clears it; it clears the limits.  Stream-ordered
+ * upload.  CWR_EINVAL
  * when kinetics is not set, for a non-finite source, a theta <= 0 or non-finite, a negative or non-finite exchange, a kind
  * other than 0 or 1, exchange without equilibrium, a non-finite equilibrium of a kind-0 column with exchange > 0, or kind 1
  * on the temperature constituent.  The reaction mass includes these terms.  Domain decomposition: every rank makes the
@@ -240,6 +258,17 @@ int cwr_set_kinetics(cwr_handle* h, const double* decay_per_day, const double* t
 int cwr_set_kinetics_sources(cwr_handle* h, const double* source_per_day, const double* source_theta,
                              const double* exchange_per_day, const double* exchange_theta,
                              const double* equilibrium, const int* equilibrium_kind);
+/* Monod limitation and inhibition of the kinetics and sources set last (see above); arrays (n): factor i scales process
+ * process[i] (0 = the decay of column[i], 1 = its source) by a factor of kind factor_kind[i] (0 = limitation, 1 =
+ * inhibition) on constituent factor_column[i] with half-saturation half_saturation[i].  n == 0 or a NULL array = limits
+ * off.  Acts only while kinetics is set; cwr_set_kinetics and cwr_set_kinetics_sources clear it, so the order is kinetics,
+ * sources, limits.  Stream-ordered upload.  CWR_EINVAL when kinetics is not set, for n < 0, a process or kind other than 0
+ * or 1, a column index out of range, a half-saturation <= 0 or non-finite, a decay factor on a column whose decay is 0 or
+ * a source factor on a column whose source is 0, a decay factor on its own column, a source factor on its own column that
+ * is an inhibition or whose source is >= 0, or the same (process, column, factor column, kind) twice.  Domain
+ * decomposition: every rank makes the same call. */
+int cwr_set_kinetics_limits(cwr_handle* h, int n, const int* process, const int* column, const int* factor_column,
+                            const int* factor_kind, const double* half_saturation);
 /* Reaction mass of constituent k, sum over the steps taken of sum_i V[t]_i (c~'_ik - c~_ik), reduced on the device in a fixed
  * order (the same bits every run): a running sum since cwr_create, 0 while kinetics was never set.  Domain decomposition:
  * the partial sum over the rows the rank owns (as cwr_mass_totals_at). */

@@ -9,8 +9,8 @@ compared with (a) the oracle (reference arithmetic incl. SuperLU, on rank 0; rto
 tests/test_gpu_parity.py) and (b) a single-GPU run of the same library on rank 0's GPU.  Mass totals and
 boundary flux sums are checked as sums of the per-rank partial values.  --kinetics: the same with a first-order
 network (synthetic.make_kinetics) reacted on the device, in every other case with sources and exchange as well
-(synthetic.make_kinetics_sources), the oracle being oracle.kinetics_sources.KineticsRiverine, and the ranks' reaction
-masses summed against the single-GPU ones.  Prints one JSON line per case on
+(synthetic.make_kinetics_sources) and in every fourth with Monod factors (synthetic.make_kinetics_limits), the oracle
+being oracle.kinetics_limits.KineticsRiverine, and the ranks' reaction masses summed against the single-GPU ones.  Prints one JSON line per case on
 rank 0; exit code 0 only if every check passed on every rank.
 """
 from __future__ import annotations
@@ -34,14 +34,15 @@ def main():
     ap.add_argument("--steps", type=int, default=6)
     ap.add_argument("--no-oracle", action="store_true")
     ap.add_argument("--kinetics", action="store_true",
-                    help="react a first-order network on the device in every step, with sources and exchange in every other case")
+                    help="react a first-order network on the device in every step, with sources and exchange in every other case "
+                         "and Monod factors in every fourth")
     args = ap.parse_args()
     import torch
     import torch.distributed as dist
     from clearwater_riverine_b200 import TransportBackend, synthetic
     from clearwater_riverine_b200.domain import DomainDecomposedBackend, merge_owned
     from oracle import reference_step as ref
-    from oracle.kinetics_sources import KineticsRiverine
+    from oracle.kinetics_limits import KineticsRiverine, limit_terms
 
     rank, world, local = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"]), int(os.environ["LOCAL_RANK"])
     torch.cuda.set_device(local)
@@ -59,11 +60,13 @@ def main():
         adv, _, _, cdiff, dt = ref.derive_coefficients(plan.face_flow, plan.edge_velocity, plan.face_x, plan.face_y,
                                                        plan.f1, plan.f2, D, plan.time_seconds)
         inputs = synthetic.make_inputs(plan, K, seed=40 + ci)
-        kin = src = None
+        kin = src = lim = None
         if args.kinetics:
             inputs, kin = synthetic.make_kinetics(inputs, seed=40 + ci)
             if ci % 2:
                 src = synthetic.make_kinetics_sources(kin, seed=40 + ci)
+            if ci % 4 == 3:
+                lim = synthetic.make_kinetics_limits(kin, src, seed=40 + ci)
         be = DomainDecomposedBackend(plan.f1, plan.f2, plan.n_face, T, K, D, rank, world, device=local, **opts)
         be.set_hydro(0, adv, cdiff, plan.edge_velocity, plan.volume, dt)
         info = be.attach()
@@ -73,6 +76,8 @@ def main():
             be.set_kinetics(**kin)
         if src is not None:
             be.set_kinetics_sources(**src)
+        if lim is not None:
+            be.set_kinetics_limits(**lim)
         single = oracle = None
         if rank == 0:
             single = TransportBackend(plan.f1, plan.f2, plan.n_face, T, K, D, device=local, solver_path=1,
@@ -84,6 +89,8 @@ def main():
                 single.set_kinetics(**kin)
             if src is not None:
                 single.set_kinetics_sources(**src)
+            if lim is not None:
+                single.set_kinetics_limits(**lim)
             if not args.no_oracle:
                 mesh = ref.HydroMesh(plan.f1, plan.f2, plan.n_face, adv, cdiff, plan.edge_velocity, plan.volume, dt, D)
                 named = {f"c{k}": inputs[k] for k in range(K)}
@@ -92,7 +99,7 @@ def main():
                 else:
                     temperature = f"c{kin['temperature_k']}" if kin["temperature_k"] >= 0 else kin["temperature_c"]
                     oracle = KineticsRiverine(mesh, named, kin["decay_per_day"], kin["theta"], kin["yields"], temperature,
-                                              **(src or {}))
+                                              **(src or {}), **limit_terms(**(lim or {})))
         worst_oracle = worst_single = 0.0
         iters = []
         status = 0
@@ -136,6 +143,7 @@ def main():
             if kin is not None:
                 line["reaction_mass_rel_diff"] = rmass_err
                 line["sources"] = src is not None
+                line["limits"] = lim is not None
             single.close()
         flag = torch.tensor([1 if ok else 0], device="cuda")
         dist.all_reduce(flag, op=dist.ReduceOp.MIN)

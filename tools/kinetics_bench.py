@@ -15,6 +15,12 @@ device kinetics.  With sources (cwr_set_kinetics_sources), 1M x 16: the same net
 exchange of synthetic.make_kinetics_sources (sediment-oxygen-demand-like sinks, reaeration toward oxygen saturation, an
 equilibrium temperature), with the temperature constituent and at a constant temperature, each against the same network
 without its sources, alternately on the same handle: the step time and k_react's time (the CWR_FAM_RHS delta).
+With Monod factors (cwr_set_kinetics_limits), 1M x 16: the network with its sources and the factors of
+synthetic.make_kinetics_limits against the same network without the factors, alternately on the same handle, with the
+temperature constituent and at a constant temperature (--limits-only: this leg alone).  --parent-root DIR: the
+kinetics-only and the sources-only network timed in this tree's build and in DIR's (another checkout with its library
+built), one process per measurement, alternating, --parent-rounds times each; every process also reports the spread of
+its own repetitions.
 Prints one JSON object and writes it to --out.
 """
 from __future__ import annotations
@@ -30,6 +36,8 @@ import numpy as np
 
 ROOT = Path(__file__).resolve().parent.parent
 sys.path.insert(0, str(ROOT))
+if "--regression-child" in sys.argv:          # the package and its library from the tree named by --root
+    sys.path.insert(0, sys.argv[sys.argv.index("--root") + 1])
 
 
 def gpu_name_and_power():
@@ -107,6 +115,125 @@ def alternate_sources(torch, be, kin, src, step, reps):
     return {f"{key}_{name}": float(np.median(v[i])) for key, v in out.items() for i, name in enumerate(("without", "with"))}
 
 
+def alternate_limits(torch, be, kin, src, lim, step, reps):
+    """The network with its sources, without and with its Monod factors, alternately, reps times each: medians of the step
+    time (ms, CUDA events) and of the CWR_FAM_RHS family time (ms per step, in separate profiled steps)."""
+    out = {"step_ms": ([], []), "rhs_family_ms": ([], [])}
+    for _ in range(reps):
+        for i, with_lim in enumerate((False, True)):
+            be.set_kinetics(**kin)
+            be.set_kinetics_sources(**src)
+            if with_lim:
+                be.set_kinetics_limits(**lim)
+            step()
+            out["step_ms"][i].append(timed(torch, be, step, 5))
+            be.profile(1)
+            for _ in range(5):
+                step()
+            out["rhs_family_ms"][i].append(be.profile(-1)["rhs"][0] / 5)
+            be.profile(0)
+    return {f"{key}_{name}": float(np.median(v[i])) for key, v in out.items() for i, name in enumerate(("without", "with"))}
+
+
+def limits_leg(torch, res, reps, scale):
+    """1M x 16 with sources: without and with Monod factors, with the temperature constituent and at a constant one."""
+    import bench
+    from clearwater_riverine_b200 import synthetic
+    plan, K = bench.workload_plan("1m16", 14, seed=0, scale=scale)
+    inputs, kin = synthetic.make_kinetics(synthetic.make_inputs(plan, K, seed=0), seed=0, decay_range=(0.05, 2.0))
+    src = synthetic.make_kinetics_sources(kin, seed=0, rate_range=(0.05, 2.0))
+    lim = synthetic.make_kinetics_limits(kin, src, seed=0)
+    be = build(plan, inputs, torch)
+    for t in range(3):
+        be.step(t)
+    step = lambda: be.step(3)
+    be.profile(1)
+    for _ in range(10):
+        step()
+    fam_off = be.profile(-1)["rhs"][0] / 10
+    be.profile(0)
+    kin_const = dict(kin, temperature_k=-1, temperature_c=24.0)
+    for key, k in (("1m16_limits", kin), ("1m16_limits_constant_temperature", kin_const)):
+        r = alternate_limits(torch, be, k, src, lim, step, reps)
+        r["k_react_ms_without_limits"] = r["rhs_family_ms_without"] - fam_off
+        r["k_react_ms_with_limits"] = r["rhs_family_ms_with"] - fam_off
+        r["k_react_added_ms"] = r["rhs_family_ms_with"] - r["rhs_family_ms_without"]
+        r["step_added_ms"] = r["step_ms_with"] - r["step_ms_without"]
+        r["factors"] = int(len(lim["process"]))
+        r["limited_processes"] = int(len({(int(p), int(c)) for p, c in zip(lim["process"], lim["column"])}))
+        res[key] = r
+    be.close()
+
+
+def regression_child(reps, scale):
+    """One process of --parent-root: kinetics off, the kinetics-only and the sources-only 1M x 16 network (temperature
+    constituent) on one handle; medians and spreads (min, max) of the step time and of k_react's time (CWR_FAM_RHS
+    delta).  Uses only calls both builds have."""
+    import os
+    import torch
+    import bench
+    from clearwater_riverine_b200 import synthetic
+    from clearwater_riverine_b200.backend import library_path
+    plan, K = bench.workload_plan("1m16", 14, seed=0, scale=scale)
+    inputs, kin = synthetic.make_kinetics(synthetic.make_inputs(plan, K, seed=0), seed=0, decay_range=(0.05, 2.0))
+    src = synthetic.make_kinetics_sources(kin, seed=0, rate_range=(0.05, 2.0))
+    be = build(plan, inputs, torch)
+    for t in range(3):
+        be.step(t)
+    step = lambda: be.step(3)
+    modes = {"off": None, "kinetics": (kin, None), "sources": (kin, src)}
+    samples = {m: {"step_ms": [], "rhs_family_ms": []} for m in modes}
+    for _ in range(reps):
+        for m, v in modes.items():
+            if v is None:
+                be.set_kinetics(None)
+            else:
+                be.set_kinetics(**v[0])
+                if v[1] is not None:
+                    be.set_kinetics_sources(**v[1])
+            step()
+            samples[m]["step_ms"].append(timed(torch, be, step, 5))
+            be.profile(1)
+            for _ in range(5):
+                step()
+            samples[m]["rhs_family_ms"].append(be.profile(-1)["rhs"][0] / 5)
+            be.profile(0)
+    be.close()
+    lib = Path(os.environ.get("CWR_B200_LIB", library_path())).resolve()   # what load_library actually loaded
+    out = {"library": str(lib.relative_to(Path.cwd().resolve())) if lib.is_relative_to(Path.cwd().resolve()) else str(lib)}
+    off = np.array(samples["off"]["rhs_family_ms"])
+    for m in ("kinetics", "sources"):
+        st, fam = np.array(samples[m]["step_ms"]), np.array(samples[m]["rhs_family_ms"])
+        react = fam - np.median(off)
+        out[m] = {"step_ms": float(np.median(st)), "step_ms_min": float(st.min()), "step_ms_max": float(st.max()),
+                  "k_react_ms": float(np.median(react)), "k_react_ms_min": float(react.min()),
+                  "k_react_ms_max": float(react.max())}
+    print(json.dumps(out))
+
+
+def parent_comparison(parent_root: str, rounds: int, reps: int, scale: float) -> dict:
+    """regression_child in this tree and in parent_root, alternately (one process each), `rounds` times each."""
+    import os
+    runs = {"this": [], "parent": []}
+    for _ in range(rounds):
+        for name, root in (("parent", parent_root), ("this", str(ROOT))):
+            env = dict(os.environ, CWR_B200_LIB=str(Path(root) / "clearwater_riverine_b200" / "libcwr_b200.so"))
+            out = subprocess.run([sys.executable, str(Path(__file__).resolve()), "--regression-child", "--root", root,
+                                  "--reps", str(reps), "--scale", str(scale)], capture_output=True, text=True, env=env,
+                                 timeout=1800)
+            if out.returncode != 0:
+                raise SystemExit(f"regression child failed ({name}):\n{out.stderr[-3000:]}")
+            runs[name].append(json.loads(out.stdout.strip().splitlines()[-1]))
+    res = {"rounds": rounds, "reps_per_round": reps, "runs": runs}
+    for m in ("kinetics", "sources"):
+        for key in ("step_ms", "k_react_ms"):
+            a = [r[m][key] for r in runs["this"]]
+            b = [r[m][key] for r in runs["parent"]]
+            res[f"{m}_{key}_this_median"], res[f"{m}_{key}_parent_median"] = float(np.median(a)), float(np.median(b))
+            res[f"{m}_{key}_this_range"], res[f"{m}_{key}_parent_range"] = [min(a), max(a)], [min(b), max(b)]
+    return res
+
+
 def host_loop(be, kin, t0, steps, dt):
     """The coupled loop with the reactions on the host: c[t] down, numpy reactions, override up, step.  s per step."""
     from oracle.kinetics import react
@@ -135,13 +262,29 @@ def main():
     ap.add_argument("--reps", type=int, default=15)
     ap.add_argument("--scale", type=float, default=1.0, help="1m16 mesh side scale (1.0 = 1M cells)")
     ap.add_argument("--out", default=None)
+    ap.add_argument("--limits-only", action="store_true", help="only the Monod-factor leg (and --parent-root)")
+    ap.add_argument("--parent-root", default=None,
+                    help="another checkout with its library built: the no-factor networks timed in both builds, alternately")
+    ap.add_argument("--parent-rounds", type=int, default=3)
+    ap.add_argument("--regression-child", action="store_true", help=argparse.SUPPRESS)
+    ap.add_argument("--root", default=None, help=argparse.SUPPRESS)
     args = ap.parse_args()
+    if args.regression_child:
+        regression_child(args.reps, args.scale)
+        return
     import torch
     import bench
     from clearwater_riverine_b200 import synthetic
     if not torch.cuda.is_available():
         raise SystemExit("kinetics_bench needs a CUDA device")
-    res = {"gpu": gpu_name_and_power(), "d2d_copy_gbs": copy_rate_gbs(torch)}
+    res = {"gpu": gpu_name_and_power()}
+    if args.limits_only:
+        limits_leg(torch, res, args.reps, args.scale)
+        if args.parent_root:
+            res["no_factor_paths_vs_parent"] = parent_comparison(args.parent_root, args.parent_rounds, max(3, args.reps // 3),
+                                                                 args.scale)
+        return emit(res, args.out)
+    res["d2d_copy_gbs"] = copy_rate_gbs(torch)
 
     # --- 1M x 16 ------------------------------------------------------------------------------------------------
     T = 14
@@ -211,11 +354,18 @@ def main():
         res[key]["coupled_host_ms_per_step"] = 1e3 * host_loop(be, kin, 0, 100, 3600.0)
         res[key]["coupled_device_ms_per_step"] = 1e3 * device_loop(torch, be, kin, 0, 100)
         be.close()
-    line = json.dumps(res)
-    print(line)
-    if args.out:
-        Path(args.out).parent.mkdir(parents=True, exist_ok=True)
-        Path(args.out).write_text(json.dumps(res, indent=1) + "\n")
+    limits_leg(torch, res, args.reps, args.scale)
+    if args.parent_root:
+        res["no_factor_paths_vs_parent"] = parent_comparison(args.parent_root, args.parent_rounds, max(3, args.reps // 3),
+                                                             args.scale)
+    emit(res, args.out)
+
+
+def emit(res: dict, out) -> None:
+    print(json.dumps(res))
+    if out:
+        Path(out).parent.mkdir(parents=True, exist_ok=True)
+        Path(out).write_text(json.dumps(res, indent=1) + "\n")
 
 
 if __name__ == "__main__":
