@@ -13,6 +13,8 @@ from typing import Optional, Sequence
 
 import numpy as np
 
+from .kinetics import DEFAULT_MIN_DEPTH
+
 _LIB_NAME = "libcwr_b200.so"
 _lib = None
 
@@ -105,6 +107,7 @@ def load_library():
         "cwr_set_kinetics": ([H, dp, dp, dp, C.c_int, C.c_double], C.c_int),
         "cwr_set_kinetics_sources": ([H, dp, dp, dp, dp, dp, ip], C.c_int),
         "cwr_set_kinetics_limits": ([H, C.c_int, ip, ip, ip, ip, dp], C.c_int),
+        "cwr_set_kinetics_depth": ([H, dp, C.c_double, ip, ip, ip], C.c_int),
         "cwr_get_reaction_mass": ([H, C.c_int, dp], C.c_int),
         "cwr_get_lhs": ([H, C.POINTER(C.c_int64), ip, ip, dp], C.c_int),
         "cwr_get_rhs": ([H, C.c_int, dp], C.c_int),
@@ -415,7 +418,7 @@ class TransportBackend:
         """First-order decay / transformations applied on the device in every later step (cwr_set_kinetics):
         decay_per_day (K,) or None = off; theta (K,) or None = all 1; yields (K, K), yields[j, k] = mass of j formed per
         mass of k decayed, or None; temperature_k = temperature constituent or -1 for the constant temperature_c (deg C).
-        An invalid set raises ValueError; any call clears set_kinetics_sources and set_kinetics_limits.
+        An invalid set raises ValueError; any call clears set_kinetics_sources, set_kinetics_limits and set_kinetics_depth.
         kinetics.compile_kinetics builds the arrays from a by-name spec."""
         if decay_per_day is None:
             self._check(self._lib.cwr_set_kinetics(self._h, None, None, None, -1, 20.0))
@@ -435,7 +438,8 @@ class TransportBackend:
         last (cwr_set_kinetics_sources): dc/dt = s + r (ceq - c) per column, solved exactly over each step.
         source_per_day (K,) or None; exchange_per_day (K,) 1/day or None (both None: sources off); a theta (K,) or None =
         all 1; equilibrium (K,) the constant targets; equilibrium_kind (K,) 0 = constant, 1 = oxygen saturation at T, or
-        None = all 0.  set_kinetics clears them; any call clears set_kinetics_limits.  An invalid set raises ValueError."""
+        None = all 0.  set_kinetics clears them; any call clears set_kinetics_limits and set_kinetics_depth.  An invalid
+        set raises ValueError."""
         K = (self.K,)
         f = lambda a, name: None if a is None else _arr(a, np.float64, K, name)
         arrs = [f(source_per_day, "source_per_day"), f(source_theta, "source_theta"), f(exchange_per_day, "exchange_per_day"),
@@ -460,6 +464,24 @@ class TransportBackend:
                                                                   (factor_kind, "factor_kind"))]
         hs = _arr(half_saturation, np.float64, n, "half_saturation")
         rc = self._lib.cwr_set_kinetics_limits(self._h, n[0], *[_ptr(a, C.c_int32) for a in ints], _ptr(hs, C.c_double))
+        if rc == CWR_EINVAL:
+            raise ValueError(self._lib.cwr_last_error(self._h).decode())
+        self._check(rc)
+
+    def set_kinetics_depth(self, cell_area=None, min_depth: float = DEFAULT_MIN_DEPTH, decay_per_depth=None, source_per_depth=None,
+                           exchange_per_depth=None):
+        """Depth-scaled processes of the kinetics and sources set last (cwr_set_kinetics_depth): a flag (K,) of 1 divides
+        that process's rate of column k by the cell's depth h = max(V[t] / cell_area, min_depth), making the decay a
+        settling velocity, the source an areal flux and the exchange a transfer velocity (mesh length units).  cell_area
+        (F,) plan areas; every flag None or 0 = depth off.  set_kinetics and set_kinetics_sources clear it;
+        set_kinetics_limits does not.  An invalid set raises ValueError."""
+        K = (self.K,)
+        flags = [None if a is None else _arr(a, np.int32, K, name) for a, name in
+                 ((decay_per_depth, "decay_per_depth"), (source_per_depth, "source_per_depth"),
+                  (exchange_per_depth, "exchange_per_depth"))]
+        area = None if cell_area is None else _arr(cell_area, np.float64, (self.n_face,), "cell_area")
+        rc = self._lib.cwr_set_kinetics_depth(self._h, _ptr(area, C.c_double), float(min_depth),
+                                              *[_ptr(a, C.c_int32) for a in flags])
         if rc == CWR_EINVAL:
             raise ValueError(self._lib.cwr_last_error(self._h).decode())
         self._check(rc)

@@ -121,11 +121,19 @@ struct cwr_handle {
     KinSrc* d_kin_srcs = nullptr;
     // what cwr_set_kinetics_limits validates against: the decay rates and yields of the kinetics set last, the step of
     // each decaying column and the list position of each source column (-1: none)
-    std::vector<double> kin_decay_h, kin_yields_h, kin_source_h;
+    std::vector<double> kin_decay_h, kin_yields_h, kin_source_h, kin_exchange_h;
     std::vector<int> kin_step_of, kin_src_of;
     // Monod factors (cwr_set_kinetics_limits): kin_facs entries, grouped per process by d_kin_fptr (n_steps + n_src + 1)
     int kin_facs = 0;
     KinFac* d_kin_facs = nullptr; int* d_kin_fptr = nullptr;
+    // depth-scaled processes (cwr_set_kinetics_depth): flags per process (n_steps + n_src, numbered as d_kin_fptr; bit 0 the
+    // decay or source, bit 1 the exchange), the plan areas in reference numbering (kin_area_h, F) and per device row
+    // (d_kin_area, n; uploaded again when the ordering is rebuilt); k_react<true, true> runs while kin_depth, with the
+    // all-zero d_kin_fptr0 when there are no factors
+    bool kin_depth = false;
+    double kin_min_depth = 0.0;
+    std::vector<double> kin_area_h;
+    double* d_kin_area = nullptr; int* d_kin_dflag = nullptr; int* d_kin_fptr0 = nullptr;
     // optional per-kernel-family timing with CUDA events on the handle's stream (bench.py roofline)
     bool profiling = false;
     std::vector<cudaEvent_t> ev_pool;
@@ -291,6 +299,14 @@ static cudaError_t put(cwr_handle* h, T* d, const std::vector<T>& v) {
     return v.empty() ? cudaSuccess : cudaMemcpyAsync(d, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice, h->stream);
 }
 
+// the plan areas of cwr_set_kinetics_depth in the device order (stream-ordered; pageable source)
+static int upload_kin_area(cwr_handle* h) {
+    std::vector<double> a(h->n);
+    for (int i = 0; i < h->n; ++i) a[i] = h->kin_area_h[h->topo.old_of_new[i]];
+    CK(cudaMemcpyAsync(h->d_kin_area, a.data(), a.size() * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+    return CWR_OK;
+}
+
 static int upload_topology(cwr_handle* h) {
     const Topology& tp = h->topo;
     CK(put(h, h->d_ell_col, tp.ell_col)); CK(put(h, h->d_ell_code, tp.ell_code));
@@ -314,6 +330,10 @@ static int upload_topology(cwr_handle* h) {
         }
         CK(put(h, h->d_strip_nbr, tp.strip_nbr));
         CK(put(h, h->d_strip_peers, tp.strip_peers));
+    }
+    if (!h->kin_area_h.empty()) {
+        const int rc = upload_kin_area(h);
+        if (rc) return rc;
     }
     CK(cudaStreamSynchronize(h->stream));
     return CWR_OK;
@@ -1347,10 +1367,13 @@ static int build_rhs(cwr_handle* h, int t, int accumulate) {
         // after cwr_set_kinetics), at most the resident grid; the same rows give the same grid, hence the same sums
         const int R = react_tile_rows(h->K);
         const int grid = grid_for((M.row_hi - M.row_lo + R - 1) / R, 1, h->kin_grid_max);
-        CK(launch_chain(h, h->kin_facs ? k_react<true> : k_react<false>, grid, kThreads, react_smem_bytes(h->K) + react_src_smem_bytes(h->kin_srcs, h->kin_temp_k), M,
+        auto* fn = h->kin_depth ? k_react<true, true> : h->kin_facs ? k_react<true> : k_react<false>;
+        const int* fptr = h->kin_depth && !h->kin_facs ? h->d_kin_fptr0 : h->d_kin_fptr;
+        CK(launch_chain(h, fn, grid, kThreads, react_smem_bytes(h->K) + react_src_smem_bytes(h->kin_srcs, h->kin_temp_k), M,
                         (const KinStep*)h->d_kin_steps, h->kin_steps, (const KinYield*)h->d_kin_yields, h->kin_temp_k, h->kin_temp_c,
                         (const KinSrc*)h->d_kin_srcs, h->kin_srcs, h->kin_src_o2, (const KinFac*)h->d_kin_facs,
-                        (const int*)h->d_kin_fptr, h->d_kin_partials, h->d_kin_state, accumulate));
+                        fptr, h->d_kin_partials, h->d_kin_state, accumulate, (const double*)h->d_kin_area,
+                        (const int*)h->d_kin_dflag, h->kin_min_depth));
         h->launches += 1;
     }
     if (M.b_hi - M.b_lo > 0) {
@@ -1702,7 +1725,7 @@ int cwr_set_kinetics(cwr_handle* h, const double* decay, const double* theta, co
                      double temperature_c) {
     if (!h) return CWR_EINVAL;
     const int K = h->K;
-    if (!decay) { h->kin_on = false; h->kin_srcs = 0; h->kin_facs = 0; return CWR_OK; }
+    if (!decay) { h->kin_on = false; h->kin_srcs = 0; h->kin_facs = 0; h->kin_depth = false; return CWR_OK; }
     for (int k = 0; k < K; ++k) {
         if (!std::isfinite(decay[k]) || decay[k] < 0.0) FAIL(CWR_EINVAL, "cwr_set_kinetics: decay rates must be finite and >= 0");
         if (theta && (!std::isfinite(theta[k]) || theta[k] <= 0.0)) FAIL(CWR_EINVAL, "cwr_set_kinetics: theta must be finite and > 0");
@@ -1751,12 +1774,13 @@ int cwr_set_kinetics(cwr_handle* h, const double* decay, const double* theta, co
     }
     CK(cudaSetDevice(h->device));
     if (!h->d_kin_state) {
-        cudaFuncAttributes fa{}, fl{};
+        cudaFuncAttributes fa{}, fl{}, fd{};
         CK(cudaFuncGetAttributes(&fa, k_react<false>));
         CK(cudaFuncGetAttributes(&fl, k_react<true>));
-        if (std::max(fa.sharedSizeBytes, fl.sharedSizeBytes) > kReactStaticSmem)
+        CK(cudaFuncGetAttributes(&fd, k_react<true, true>));
+        if (std::max({fa.sharedSizeBytes, fl.sharedSizeBytes, fd.sharedSizeBytes}) > kReactStaticSmem)
             FAIL(CWR_ECUDA, "k_react: static shared memory exceeds what its tile sizing reserves");
-        // the grid of both instantiations (k_react<true> may hold fewer CTAs per SM; its CTAs need not be co-resident)
+        // the grid of every instantiation (the factored ones may hold fewer CTAs per SM; their CTAs need not be co-resident)
         int occ = 0;
         CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_react<false>, kThreads, react_smem_bytes(K)));
         h->kin_grid_max = h->num_sms * std::max(1, occ);
@@ -1767,7 +1791,11 @@ int cwr_set_kinetics(cwr_handle* h, const double* decay, const double* theta, co
         CK(dalloc(h, &h->d_kin_srcs, (size_t)K));
         CK(dalloc(h, &h->d_kin_facs, (size_t)4 * K * K));      // at most (decay | source) x column x factor column x kind
         CK(dalloc(h, &h->d_kin_fptr, (size_t)2 * K + 1));
+        CK(dalloc(h, &h->d_kin_fptr0, (size_t)2 * K + 1));
+        CK(dalloc(h, &h->d_kin_dflag, (size_t)2 * K));
+        CK(dalloc(h, &h->d_kin_area, (size_t)h->n));
         CK(cudaMemsetAsync(h->d_kin_state, 0, sizeof(KinState), h->stream));
+        CK(cudaMemsetAsync(h->d_kin_fptr0, 0, ((size_t)2 * K + 1) * sizeof(int), h->stream));
     }
     // stream-ordered: steps queued before this call still read the previous parameters (pageable sources: the copies
     // have left the host vectors when the calls return)
@@ -1779,12 +1807,14 @@ int cwr_set_kinetics(cwr_handle* h, const double* decay, const double* theta, co
     h->kin_on = true;
     h->kin_srcs = 0;
     h->kin_facs = 0;
+    h->kin_depth = false;
     h->kin_decay_h.assign(decay, decay + K);
     h->kin_yields_h.assign((size_t)K * K, 0.0);
     if (yields) h->kin_yields_h.assign(yields, yields + (size_t)K * K);
     h->kin_step_of.assign(K, -1);
     for (size_t p = 0; p < steps.size(); ++p) h->kin_step_of[steps[p].col] = (int)p;
     h->kin_source_h.assign(K, 0.0);
+    h->kin_exchange_h.assign(K, 0.0);
     h->kin_src_of.assign(K, -1);
     return CWR_OK;
 }
@@ -1795,8 +1825,8 @@ int cwr_set_kinetics_sources(cwr_handle* h, const double* source_per_day, const 
     const int K = h->K;
     if (!h->kin_on) FAIL(CWR_EINVAL, "cwr_set_kinetics_sources: call cwr_set_kinetics first");
     if (!source_per_day && !exchange_per_day) {
-        h->kin_srcs = 0; h->kin_facs = 0;
-        h->kin_source_h.assign(K, 0.0); h->kin_src_of.assign(K, -1);
+        h->kin_srcs = 0; h->kin_facs = 0; h->kin_depth = false;
+        h->kin_source_h.assign(K, 0.0); h->kin_exchange_h.assign(K, 0.0); h->kin_src_of.assign(K, -1);
         return CWR_OK;
     }
     if (exchange_per_day && !equilibrium) FAIL(CWR_EINVAL, "cwr_set_kinetics_sources: exchange needs an equilibrium array");
@@ -1834,17 +1864,20 @@ int cwr_set_kinetics_sources(cwr_handle* h, const double* source_per_day, const 
     // at a constant temperature the coefficients take shared memory beyond the tile's 48 KB (react_src_smem_bytes); the
     // limit is the same for every handle (the attribute is the kernel's, not the handle's)
     if (h->kin_temp_k < 0 && !list.empty())
-        for (auto* fn : {k_react<false>, k_react<true>})
+        for (auto* fn : {k_react<false>, k_react<true>, k_react<true, true>})
             CK(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                     (int)(kReactSmemLimit - kReactStaticSmem + react_src_smem_bytes(kMaxK, -1))));
     if (!list.empty()) CK(cudaMemcpyAsync(h->d_kin_srcs, list.data(), list.size() * sizeof(KinSrc), cudaMemcpyHostToDevice, h->stream));
     h->kin_srcs = (int)list.size();
     h->kin_src_o2 = o2;
     h->kin_facs = 0;
+    h->kin_depth = false;
     h->kin_source_h.assign(K, 0.0);
+    h->kin_exchange_h.assign(K, 0.0);
     h->kin_src_of.assign(K, -1);
     for (size_t p = 0; p < list.size(); ++p) {
         h->kin_source_h[list[p].col] = list[p].source;
+        h->kin_exchange_h[list[p].col] = list[p].exchange;
         h->kin_src_of[list[p].col] = (int)p;
     }
     return CWR_OK;
@@ -1894,6 +1927,48 @@ int cwr_set_kinetics_limits(cwr_handle* h, int n, const int* process, const int*
     CK(cudaMemcpyAsync(h->d_kin_facs, list.data(), list.size() * sizeof(KinFac), cudaMemcpyHostToDevice, h->stream));
     CK(cudaMemcpyAsync(h->d_kin_fptr, ptr.data(), ptr.size() * sizeof(int), cudaMemcpyHostToDevice, h->stream));
     h->kin_facs = (int)list.size();
+    return CWR_OK;
+}
+
+int cwr_set_kinetics_depth(cwr_handle* h, const double* cell_area, double min_depth, const int* decay_per_depth,
+                           const int* source_per_depth, const int* exchange_per_depth) {
+    if (!h) return CWR_EINVAL;
+    const int K = h->K;
+    if (!h->kin_on) FAIL(CWR_EINVAL, "cwr_set_kinetics_depth: call cwr_set_kinetics first");
+    const int* flags[3] = {decay_per_depth, source_per_depth, exchange_per_depth};
+    bool any = false;
+    for (const int* f : flags)
+        for (int k = 0; f && k < K; ++k) {
+            if (f[k] != 0 && f[k] != 1) FAIL(CWR_EINVAL, "cwr_set_kinetics_depth: flags must be 0 or 1");
+            any |= f[k] == 1;
+        }
+    if (!any) { h->kin_depth = false; return CWR_OK; }
+    const double* rate[3] = {h->kin_decay_h.data(), h->kin_source_h.data(), h->kin_exchange_h.data()};
+    for (int w = 0; w < 3; ++w)
+        for (int k = 0; flags[w] && k < K; ++k)
+            if (flags[w][k] && rate[w][k] == 0.0)
+                FAIL(CWR_EINVAL, "cwr_set_kinetics_depth: a depth flag on a process whose rate is 0");
+    if (!cell_area) FAIL(CWR_EINVAL, "cwr_set_kinetics_depth: depth flags need the cell areas");
+    if (!std::isfinite(min_depth) || min_depth <= 0.0) FAIL(CWR_EINVAL, "cwr_set_kinetics_depth: min_depth must be finite and > 0");
+    for (int i = 0; i < h->n; ++i) {
+        const double a = cell_area[h->topo.old_of_new[i]];
+        if (!std::isfinite(a) || a <= 0.0) FAIL(CWR_EINVAL, "cwr_set_kinetics_depth: cell areas must be finite and > 0");
+    }
+    // per process, numbered as d_kin_fptr: the decay steps in their order, then the source columns in theirs
+    std::vector<int> dflag(h->kin_steps + h->kin_srcs, 0);
+    for (int k = 0; k < K; ++k) {
+        if (h->kin_step_of[k] >= 0 && decay_per_depth) dflag[h->kin_step_of[k]] = decay_per_depth[k];
+        if (h->kin_src_of[k] >= 0)
+            dflag[h->kin_steps + h->kin_src_of[k]] = (source_per_depth ? source_per_depth[k] : 0) |
+                                                     (exchange_per_depth ? exchange_per_depth[k] : 0) << 1;
+    }
+    CK(cudaSetDevice(h->device));
+    h->kin_area_h.assign(cell_area, cell_area + h->F);
+    int rc = upload_kin_area(h);
+    if (rc) return rc;
+    CK(cudaMemcpyAsync(h->d_kin_dflag, dflag.data(), dflag.size() * sizeof(int), cudaMemcpyHostToDevice, h->stream));
+    h->kin_min_depth = min_depth;
+    h->kin_depth = true;
     return CWR_OK;
 }
 

@@ -554,6 +554,13 @@ __device__ __forceinline__ void grid_totals(const double* partials, double* tot,
 // k_react<true> (launched while factors are set) has the factored code: k_react<false> keeps the registers, hence the
 // occupancy and the grid (kin_grid_max), that it has without it, and both take that grid, so the column sums of the
 // reaction mass are added in the same order with or without factors.
+// Depth-scaled processes (cwr_set_kinetics_depth) multiply a flagged rate -- the decay of step p, or the source or the
+// exchange of source column p -- by 1 / h, h = max(vol / area, min_depth) the row's depth: vol[t] from the tile (svol),
+// area read by the row's thread (coalesced).  One division per row, none per process: a division in the chain is a call
+// whose saved registers spill.  dfl[q] holds the flags of process q (numbered as fptr): bit 0 the decay or the source,
+// bit 1 the exchange.  A flagged process is evaluated per row by the factored code (at a constant temperature too); the
+// others keep their per-CTA coefficients.  Only k_react<true, true> (launched while depth flags are set, with an
+// all-empty fptr when there are no factors) has the depth code; it takes the same tile and grid as the others.
 // ---------------------------------------------------------------------------------------------
 struct KinStep { int col, y_begin, y_end, pad; double decay, log_theta; };   // a reacting constituent; its yields
 struct KinYield { int col, pad; double y; };                                 // [y_begin, y_end)
@@ -584,10 +591,12 @@ __device__ __forceinline__ void kin_src_coef(const KinSrc& s, double T, double o
     phi = r > 0.0 ? -expm1(-r * dt) / r : dt;
 }
 
-// The loss of decay step s with its nf factors a[] (the row c as it is now)
+// The loss of decay step s with its nf factors a[] (the row c as it is now); kDepth: df = 1 scales the rate by hinv = 1 / h
+template <bool kDepth = false>
 __device__ __forceinline__ double kin_decay_limited(const double* c, const KinStep& s, const KinFac* __restrict__ a, int nf,
-                                                 double T, double dt) {
-    const double r = s.decay * exp((T - 20.0) * s.log_theta) / 86400.0;
+                                                 double T, double dt, double hinv = 1.0, int df = 0) {
+    double r = s.decay * exp((T - 20.0) * s.log_theta) / 86400.0;
+    if (kDepth && df) r = r * hinv;
     double m = 1.0;
     for (int q = 0; q < nf; ++q) {
         const KinFac f = a[q];
@@ -601,13 +610,17 @@ __device__ __forceinline__ double kin_decay_limited(const double* c, const KinSt
     return loss;
 }
 
-// Source column *sp with its nf factors a[] applied to the row c (o2 = O2sat(T), read only for kind 1)
+// Source column *sp with its nf factors a[] applied to the row c (o2 = O2sat(T), read only for kind 1); kDepth: bit 0
+// of df scales the source by hinv = 1 / h, bit 1 the exchange rate
+template <bool kDepth = false>
 __device__ __forceinline__ void kin_src_limited(double* c, const KinSrc* __restrict__ sp, const KinFac* __restrict__ a, int nf,
-                                             double T, double o2, double dt) {
+                                             double T, double o2, double dt, double hinv = 1.0, int df = 0) {
     const KinSrc s = *sp;
     const double dT = T - 20.0;
-    const double r = s.exchange * exp(dT * s.log_exchange_theta) / 86400.0;
-    const double src = s.source * exp(dT * s.log_source_theta) / 86400.0;
+    double r = s.exchange * exp(dT * s.log_exchange_theta) / 86400.0;
+    double src = s.source * exp(dT * s.log_source_theta) / 86400.0;
+    if (kDepth && (df & 2)) r = r * hinv;
+    if (kDepth && (df & 1)) src = src * hinv;
     const double req = r * (s.kind ? o2 : s.equilibrium);
     double m = 1.0, self_half = 0.0;
     for (int q = 0; q < nf; ++q) {
@@ -666,12 +679,15 @@ __device__ __forceinline__ void react_pairs(const double* base, int cnt, F f) {
     }
 }
 
-template <bool kLimited>
+template <bool kLimited, bool kDepth = false>
 __global__ void __launch_bounds__(kThreads) k_react(DeviceModel M, const KinStep* __restrict__ steps, int n_steps,
                                                     const KinYield* __restrict__ yl, int temp_k, double temp_c,
                                                     const KinSrc* __restrict__ srcs, int n_src, int src_o2,
                                                     const KinFac* __restrict__ fl, const int* __restrict__ fptr,
-                                                    double* __restrict__ partials, KinState* __restrict__ ks, int accumulate) {
+                                                    double* __restrict__ partials, KinState* __restrict__ ks, int accumulate,
+                                                    const double* __restrict__ area, const int* __restrict__ dfl,
+                                                    double min_depth) {
+    static_assert(kLimited || !kDepth, "the depth code is in the factored instantiation");
     extern __shared__ double rs[];
     __shared__ KinStep st[kMaxK];
     pdl_enter();
@@ -718,14 +734,16 @@ __global__ void __launch_bounds__(kThreads) k_react(DeviceModel M, const KinStep
         if (threadIdx.x < rows) {             // one row's chain per thread
             double* c = tile + threadIdx.x * ld;
             const double T = temp_k < 0 ? temp_c : c[temp_k];
+            const double hinv = kDepth ? 1.0 / fmax(svol[threadIdx.x] / area[row0 + threadIdx.x], min_depth) : 1.0;
             for (int p = 0; p < n_steps; ++p) {
                 const KinStep& s = st[p];
                 const int fb = kLimited ? fptr[p] : 0, fe = kLimited ? fptr[p + 1] : 0;
+                const int df = kDepth ? dfl[p] : 0;
                 double loss;
-                if (fb == fe) {
+                if (fb == fe && !df) {
                     const double f = temp_k < 0 ? fac[p] : -expm1(-(s.decay * exp((T - 20.0) * s.log_theta) / 86400.0) * dt);
                     loss = c[s.col] * f;
-                } else loss = kin_decay_limited(c, s, fl + fb, fe - fb, T, dt);
+                } else loss = kin_decay_limited<kDepth>(c, s, fl + fb, fe - fb, T, dt, hinv, df);
                 c[s.col] -= loss;
                 for (int q = s.y_begin; q < s.y_end; ++q) {
                     const KinYield y = yl[q];
@@ -736,8 +754,9 @@ __global__ void __launch_bounds__(kThreads) k_react(DeviceModel M, const KinStep
                 const double o2 = src_o2 ? o2_saturation(T) : 0.0;
                 for (int p = 0; p < n_src; ++p) {
                     const int fb = fptr[n_steps + p], fe = fptr[n_steps + p + 1];
-                    if (fb != fe) {
-                        kin_src_limited(c, srcs + p, fl + fb, fe - fb, T, o2, dt);
+                    const int df = kDepth ? dfl[n_steps + p] : 0;
+                    if (fb != fe || df) {
+                        kin_src_limited<kDepth>(c, srcs + p, fl + fb, fe - fb, T, o2, dt, hinv, df);
                     } else if (temp_k < 0) {
                         const double* q = sco + 3 * p;
                         double& v = c[srcs[p].col];

@@ -34,6 +34,7 @@ class RasPlan:
     face_flow: np.ndarray       # (T,E) float32  "Face Flow"
     volume: np.ndarray          # (T,F) float32  "Cell Volume"
     boundary_data: pd.DataFrame  # columns: BC Line ID, Face Index, Name, ...
+    cell_area: Optional[np.ndarray] = None   # (F,) float64 "Cells Surface Area" (cell plan area), None when absent
 
     @property
     def nreal(self) -> int:     # reference io/hdf.py:268-269
@@ -58,6 +59,15 @@ def read_ras_plan(file_path: str | Path, datetime_range: Optional[Tuple[int, int
     geom = f[f"Geometry/2D Flow Areas/{area}"]
     fc = geom["Faces Cell Indexes"].read()
     centres = geom["Cells Center Coordinate"].read()
+    cell_area = None
+    if "Cells Surface Area" in geom:                   # the plan area of every cell (kinetics given per unit depth)
+        a = np.asarray(geom["Cells Surface Area"].read(), dtype=np.float64).reshape(-1)
+        F, n = len(centres), int(fc[:, 0].max()) + 1
+        if len(a) == n:                                # real cells only: the ghost cells' areas are never read
+            a = np.concatenate([a, np.zeros(F - n)])
+        if len(a) != F:
+            raise ValueError(f"{file_path}: 'Cells Surface Area' has {len(a)} entries for {F} cells")
+        cell_area = np.ascontiguousarray(a)
     stamps = f[f"{_TS}/Time Date Stamp"].read()
     time = pd.to_datetime(pd.Series(stamps).str.decode("utf8").str.strip(), format="%d%b%Y %H:%M:%S")
     sl = slice(None)
@@ -94,6 +104,7 @@ def read_ras_plan(file_path: str | Path, datetime_range: Optional[Tuple[int, int
         face_flow=np.ascontiguousarray(flow, dtype=np.float32),
         volume=np.ascontiguousarray(vol, dtype=np.float32),
         boundary_data=bd.reset_index(drop=True),
+        cell_area=cell_area,
     )
 
 

@@ -22,6 +22,14 @@ by their own theta^(T - 20); ceq is a constant or the oxygen saturation at T (`o
 (deg C) is a constant or another constituent's value in the cell before the step's reactions.
 A decay limited by a constituent it consumes (a negative yield) never takes more of it than the cell holds, and a sink
 limited by its own constituent is solved as a first-order sink, so such a constituent cannot be driven below zero.
+Processes that act through the water depth -- settling, fluxes through the bed such as sediment oxygen demand, transfer
+through the surface -- are given per unit depth, each in place of its volumetric key, and need the model's cell plan areas:
+
+    {"PBOD": {"settling_per_day": 0.3},                                          # v_s, length/day: r = v_s / h
+     "DO":   {"areal_source_per_day": -1.5, "source_limited_by": {"DO": 1.0},    # SOD, g/m2/day on an SI plan: s = SOD / h
+              "transfer_per_day": 2.0, "equilibrium": "oxygen_saturation"}}      # K_L, length/day: r = K_L / h
+
+with h = max(V / A, min_depth) the depth of each cell at each step, in the mesh's length unit (volume unit / area unit).
 The library checks the same conditions; checking them here names the constituents in the error.
 """
 from __future__ import annotations
@@ -33,8 +41,15 @@ from typing import Mapping, Optional, Sequence, Tuple, Union
 import numpy as np
 
 _KEYS = {"decay_per_day", "theta", "yields", "source_per_day", "source_theta", "exchange_per_day", "exchange_theta",
-         "equilibrium", "limited_by", "inhibited_by", "source_limited_by", "source_inhibited_by"}
+         "equilibrium", "limited_by", "inhibited_by", "source_limited_by", "source_inhibited_by", "settling_per_day",
+         "areal_source_per_day", "transfer_per_day"}
 OXYGEN_SATURATION = "oxygen_saturation"
+# per-depth spec key -> the volumetric key it replaces (the rate of the same process, divided by the depth)
+_DEPTH_KEYS = {"settling_per_day": "decay_per_day", "areal_source_per_day": "source_per_day",
+               "transfer_per_day": "exchange_per_day"}
+# the floor of the depth h = max(V / A, min_depth), in mesh length units (1 cm on an SI plan): keeps the rates of dry and
+# nearly dry cells finite
+DEFAULT_MIN_DEPTH = 0.01
 # spec key -> (process: 0 decay, 1 source; kind: 0 limitation, 1 inhibition), in the order a block's factors compile
 _FACTOR_KEYS = {"limited_by": (0, 0), "source_limited_by": (1, 0), "inhibited_by": (0, 1), "source_inhibited_by": (1, 1)}
 
@@ -68,6 +83,13 @@ class Kinetics:
     limit_factor_column: Optional[np.ndarray] = None
     limit_kind: Optional[np.ndarray] = None
     limit_half_saturation: Optional[np.ndarray] = None
+    # depth-scaled processes, (K,) int32 0/1 each or None: 1 divides the decay / source / exchange rate of column k by the
+    # cell's depth h = max(V[t] / cell_area, min_depth); cell_area (F,) the plan areas, min_depth in mesh length units
+    decay_per_depth: Optional[np.ndarray] = None
+    source_per_depth: Optional[np.ndarray] = None
+    exchange_per_depth: Optional[np.ndarray] = None
+    cell_area: Optional[np.ndarray] = None
+    min_depth: float = DEFAULT_MIN_DEPTH
 
     @property
     def has_sources(self) -> bool:
@@ -88,6 +110,17 @@ class Kinetics:
         """The arguments of TransportBackend.set_kinetics_limits."""
         return dict(process=self.limit_process, column=self.limit_column, factor_column=self.limit_factor_column,
                     factor_kind=self.limit_kind, half_saturation=self.limit_half_saturation)
+
+    @property
+    def has_depth(self) -> bool:
+        """Whether any process is given per unit depth (otherwise cwr_set_kinetics_depth is not needed)."""
+        return any(a is not None and (np.asarray(a) != 0).any()
+                   for a in (self.decay_per_depth, self.source_per_depth, self.exchange_per_depth))
+
+    def depth_arguments(self) -> dict:
+        """The arguments of TransportBackend.set_kinetics_depth."""
+        return dict(cell_area=self.cell_area, min_depth=self.min_depth, decay_per_depth=self.decay_per_depth,
+                    source_per_depth=self.source_per_depth, exchange_per_depth=self.exchange_per_depth)
 
 
 def topological_order(yields: np.ndarray) -> Tuple[int, ...]:
@@ -112,10 +145,12 @@ def topological_order(yields: np.ndarray) -> Tuple[int, ...]:
 def validate(decay_per_day, theta, yields, temperature_k: int, temperature_c: float, names: Sequence[str] = (), *,
              source_per_day=None, source_theta=None, exchange_per_day=None, exchange_theta=None, equilibrium=None,
              equilibrium_kind=None, limit_process=None, limit_column=None, limit_factor_column=None, limit_kind=None,
-             limit_half_saturation=None) -> None:
-    """The conditions cwr_set_kinetics, cwr_set_kinetics_sources and cwr_set_kinetics_limits reject with CWR_EINVAL, as
-    ValueError.  The source arrays follow the ABI: None = none / all 1 / all 0 as there; the limit arrays are (n,) or
-    None = no limits."""
+             limit_half_saturation=None, decay_per_depth=None, source_per_depth=None, exchange_per_depth=None,
+             cell_area=None, min_depth: float = DEFAULT_MIN_DEPTH) -> None:
+    """The conditions cwr_set_kinetics, cwr_set_kinetics_sources, cwr_set_kinetics_limits and cwr_set_kinetics_depth
+    reject with CWR_EINVAL, as ValueError.  The source arrays follow the ABI: None = none / all 1 / all 0 as there; the
+    limit arrays are (n,) or None = no limits; the depth flags (K,) or None = none; cell_area: the plan areas of the real
+    cells (the ones the library reads), or None."""
     d, th, y = np.asarray(decay_per_day, np.float64), np.asarray(theta, np.float64), np.asarray(yields, np.float64)
     K = d.shape[0]
     nm = (lambda k: repr(names[k])) if len(names) == K else (lambda k: f"#{k}")
@@ -141,6 +176,8 @@ def validate(decay_per_day, theta, yields, temperature_k: int, temperature_c: fl
     topological_order(y)
     _validate_limits(d, y, source_per_day, nm, limit_process, limit_column, limit_factor_column, limit_kind,
                      limit_half_saturation)
+    _validate_depth(d, source_per_day, exchange_per_day, nm, decay_per_depth, source_per_depth, exchange_per_depth,
+                    cell_area, min_depth)
     if source_per_day is None and exchange_per_day is None:
         return
     if exchange_per_day is not None and equilibrium is None:
@@ -201,13 +238,53 @@ def _validate_limits(d, y, source_per_day, nm, process, column, factor_column, k
         seen.add((pr, k, j, kd))
 
 
+def _validate_depth(d, source_per_day, exchange_per_day, nm, decay_per_depth, source_per_depth, exchange_per_depth,
+                    cell_area, min_depth) -> None:
+    K = d.shape[0]
+    rates = {"decay": d, "source": source_per_day, "exchange": exchange_per_day}
+    per_depth = {"decay": decay_per_depth, "source": source_per_depth, "exchange": exchange_per_depth}
+    flagged = []
+    for what, flags in per_depth.items():
+        if flags is None:
+            continue
+        f = np.asarray(flags).reshape(-1)
+        if f.shape[0] != K:
+            raise ValueError(f"{what}_per_depth: expected {K} flags, got {f.shape[0]}")
+        for k in range(K):
+            if f[k] not in (0, 1):
+                raise ValueError(f"{what}_per_depth of {nm(k)} must be 0 or 1, got {f[k]}")
+            if f[k] == 1:
+                flagged.append((what, k))
+    if not flagged:
+        return
+    for what, k in flagged:
+        r = rates[what]
+        if r is None or np.asarray(r, np.float64)[k] == 0:
+            raise ValueError(f"the {what} of {nm(k)} is given per depth, but its rate is 0")
+    if cell_area is None:
+        what, k = flagged[0]
+        raise ValueError(f"the {what} of {nm(k)} is given per depth, which needs the cell plan areas (cell_area)")
+    if not (math.isfinite(min_depth) and min_depth > 0):
+        raise ValueError(f"min_depth must be finite and > 0, got {min_depth}")
+    a = np.asarray(cell_area, np.float64)
+    bad = ~(np.isfinite(a) & (a > 0))
+    if bad.any():
+        i = int(np.argmax(bad))
+        raise ValueError(f"cell areas must be finite and > 0 (processes of {nm(flagged[0][1])} are per depth); "
+                         f"cell {i} has {a[i]}")
+
+
 def compile_kinetics(spec: Mapping[str, Mapping], constituents: Sequence[str],
-                     temperature: Union[str, float] = 20.0) -> Kinetics:
+                     temperature: Union[str, float] = 20.0, *, cell_area=None, min_depth: float = DEFAULT_MIN_DEPTH,
+                     n_real: Optional[int] = None) -> Kinetics:
     """spec: {constituent: {"decay_per_day": float, "theta": float (default 1), "yields": {constituent: float},
     "source_per_day": float, "source_theta": float (default 1), "exchange_per_day": float, "exchange_theta": float
     (default 1), "equilibrium": float or "oxygen_saturation" (required when exchange_per_day > 0), "limited_by",
-    "inhibited_by", "source_limited_by", "source_inhibited_by": {constituent: half_saturation}}};
-    temperature: a constituent name, or a constant in deg C.  The factors compile per block in spec order of the blocks:
+    "inhibited_by", "source_limited_by", "source_inhibited_by": {constituent: half_saturation}, "settling_per_day",
+    "areal_source_per_day", "transfer_per_day": the per-depth forms of decay_per_day, source_per_day and
+    exchange_per_day, each in place of its counterpart}};
+    temperature: a constituent name, or a constant in deg C; cell_area (F,) the plan areas, needed by the per-depth keys,
+    of which the first n_real (default all) are the real cells; min_depth the floor of the depth.  The factors compile per block in spec order of the blocks:
     the limitations (decay, then source) first, then the inhibitions (decay, then source), each mapping in its order."""
     names = list(constituents)
     index = {n: k for k, n in enumerate(names)}
@@ -216,6 +293,7 @@ def compile_kinetics(spec: Mapping[str, Mapping], constituents: Sequence[str],
     source, source_theta, exchange, exchange_theta = np.zeros(K), np.ones(K), np.zeros(K), np.ones(K)
     equilibrium, kind = np.zeros(K), np.zeros(K, np.int32)
     factors = []                     # (process, column, factor column, kind, half-saturation)
+    per_depth = {key: np.zeros(K, np.int32) for key in _DEPTH_KEYS}
     for name, block in spec.items():
         if name not in index:
             raise ValueError(f"kinetics given for {name!r}, which is not a constituent of the model")
@@ -225,6 +303,13 @@ def compile_kinetics(spec: Mapping[str, Mapping], constituents: Sequence[str],
         if unknown:
             raise ValueError(f"kinetics of {name!r}: unknown keys {sorted(unknown)} (expected {sorted(_KEYS)})")
         k = index[name]
+        block = dict(block)
+        for key, volumetric in _DEPTH_KEYS.items():
+            if key in block:
+                if volumetric in block:
+                    raise ValueError(f"kinetics of {name!r}: {key} replaces {volumetric}; give one of them")
+                block[volumetric] = block[key]
+                per_depth[key][k] = float(block[key]) != 0.0
         decay[k] = float(block.get("decay_per_day", 0.0))
         theta[k] = float(block.get("theta", 1.0))
         for target, y in (block.get("yields") or {}).items():
@@ -243,7 +328,8 @@ def compile_kinetics(spec: Mapping[str, Mapping], constituents: Sequence[str],
         elif eq is not None:
             equilibrium[k] = float(eq)
         elif exchange[k] > 0:
-            raise ValueError(f"kinetics of {name!r}: exchange_per_day > 0 needs an equilibrium")
+            key = "transfer_per_day" if per_depth["transfer_per_day"][k] else "exchange_per_day"
+            raise ValueError(f"kinetics of {name!r}: {key} > 0 needs an equilibrium")
         for key, (process, fkind) in _FACTOR_KEYS.items():
             entries = block.get(key) or {}
             if not isinstance(entries, Mapping):
@@ -262,9 +348,14 @@ def compile_kinetics(spec: Mapping[str, Mapping], constituents: Sequence[str],
     if factors:
         cols = list(zip(*factors))
         lim = [np.array(cols[i], np.int32) for i in range(4)] + [np.array(cols[4], np.float64)]
+    depth = [per_depth[key] if per_depth[key].any() else None for key in _DEPTH_KEYS]
+    area = None
+    if cell_area is not None and any(f is not None for f in depth):
+        area = np.ascontiguousarray(cell_area, np.float64)
     validate(decay, theta, yields, temperature_k, temperature_c, names, source_per_day=source, source_theta=source_theta,
              exchange_per_day=exchange, exchange_theta=exchange_theta, equilibrium=equilibrium, equilibrium_kind=kind,
              limit_process=lim[0], limit_column=lim[1], limit_factor_column=lim[2], limit_kind=lim[3],
-             limit_half_saturation=lim[4])
+             limit_half_saturation=lim[4], decay_per_depth=depth[0], source_per_depth=depth[1],
+             exchange_per_depth=depth[2], cell_area=None if area is None else area[:n_real], min_depth=float(min_depth))
     return Kinetics(decay, theta, yields, temperature_k, temperature_c, topological_order(yields), source, source_theta,
-                    exchange, exchange_theta, equilibrium, kind, *lim)
+                    exchange, exchange_theta, equilibrium, kind, *lim, *depth, area, float(min_depth))

@@ -45,6 +45,7 @@ class SyntheticPlan:
     n_real: int                 # n  (number of real cells = matrix order)
     boundary_faces: Dict[str, np.ndarray]   # BC line name -> ghost-edge ids
     dry_cells: np.ndarray
+    cell_area: Optional[np.ndarray] = None  # (F,) float64 plan areas (ghost cells: the full quad's)
 
     @property
     def n_face(self) -> int:
@@ -241,6 +242,8 @@ def make_plan(nx: int, ny: int, n_time: int, *, dt: float = 30.0, dx: float = 10
     volume = np.zeros((n_time, F), dtype=np.float32)
     volume[:, :n] = vol[:, inv].astype(np.float32)
     volume[:, n:] = np.float32(dx * dy * depth)                # ghost-cell volumes are never read by the step
+    cell_area = np.full(F, dx * dy)
+    cell_area[:n] = area[inv]
 
     # boundary lines: which original side each ghost edge came from
     side = np.full(E, -1)
@@ -256,7 +259,7 @@ def make_plan(nx: int, ny: int, n_time: int, *, dt: float = 30.0, dx: float = 10
     return SyntheticPlan(
         f1=f1.astype(np.int32), f2=f2.astype(np.int32), face_x=face_x, face_y=face_y, time_seconds=t,
         face_flow=flow, edge_velocity=vel, volume=volume, n_real=n, boundary_faces=bfaces,
-        dry_cells=np.sort(perm[dry_cells]))
+        dry_cells=np.sort(perm[dry_cells]), cell_area=cell_area)
 
 
 def make_inputs(plan: SyntheticPlan, n_constituents: int, *, seed: int = 0, ic_range=(0.0, 100.0),
@@ -385,3 +388,30 @@ def make_kinetics_limits(kin: dict, src: Optional[dict] = None, *, seed: int = 0
     return dict(process=np.array(cols[0], np.int32), column=np.array(cols[1], np.int32),
                 factor_column=np.array(cols[2], np.int32), factor_kind=np.array(cols[3], np.int32),
                 half_saturation=np.array(cols[4], np.float64))
+
+
+def make_kinetics_depth(kin: dict, src: Optional[dict] = None, *, seed: int = 0, depth: float = 2.0):
+    """Seeded depth-scaled processes for a network of make_kinetics (kin) and make_kinetics_sources (src, or None), in the
+    manner of a BOD-DO model: the decay of every reacting k = 0 mod 3 becomes a settling velocity, the source of every
+    k = 1 mod 2 an areal flux (sediment-oxygen-demand-like sinks) and about half of the exchange rates transfer
+    velocities, chosen with the seed.  Each flagged rate is multiplied by `depth` (mesh length units; make_plan's default
+    depth), so that at that depth it is the rate it replaces.
+    Returns (kin', src', dict of the flags of TransportBackend.set_kinetics_depth)."""
+    rng = np.random.default_rng(seed + 179424673)
+    decay = np.array(kin["decay_per_day"], np.float64, copy=True)
+    K = len(decay)
+    zero = np.zeros(K)
+    source = np.array(zero if src is None or src.get("source_per_day") is None else src["source_per_day"], np.float64)
+    exchange = np.array(zero if src is None or src.get("exchange_per_day") is None else src["exchange_per_day"], np.float64)
+    k = np.arange(K)
+    coin = rng.random(K) < 0.5
+    flags = dict(decay_per_depth=((k % 3 == 0) & (decay != 0)).astype(np.int32),
+                 source_per_depth=((k % 2 == 1) & (source != 0)).astype(np.int32),
+                 exchange_per_depth=(coin & (exchange != 0)).astype(np.int32))
+    decay[flags["decay_per_depth"] == 1] *= depth
+    source[flags["source_per_depth"] == 1] *= depth
+    exchange[flags["exchange_per_depth"] == 1] *= depth
+    kin = dict(kin, decay_per_day=decay)
+    if src is not None:
+        src = dict(src, source_per_day=source, exchange_per_day=exchange)
+    return kin, src, flags

@@ -93,6 +93,8 @@ class ClearwaterRiverine:
         mesh_file_path: Optional[str | Path] = None,
         kinetics: Optional[Dict[str, Dict[str, Any]]] = None,
         temperature: Optional[str | float] = None,
+        cell_area: Optional[np.ndarray] = None,
+        min_depth: Optional[float] = None,
         **backend_options,
     ) -> None:
         from .io import ras
@@ -115,6 +117,8 @@ class ClearwaterRiverine:
                             if isinstance(c, dict) and c.get("kinetics") is not None} or None
             if temperature is None:
                 temperature = cfg.get("temperature")
+            if min_depth is None:
+                min_depth = cfg.get("min_depth")
         if not flow_field_file_path or not isinstance(constituent_dict, dict):
             raise TypeError("Missing a `config_filepath` or a `constituent_dict` and `flow_field_file_path` to run the model.")
         plan = ras.read_ras_plan(flow_field_file_path, datetime_range)
@@ -127,7 +131,8 @@ class ClearwaterRiverine:
             units[name] = cfg_c.get("units", "Unknown")
         self._setup(plan.f1, plan.f2, plan.face_x, plan.face_y, plan.time_seconds, plan.face_flow, plan.edge_velocity,
                     plan.volume, float(diffusion_coefficient_input), inputs, units, time=plan.time,
-                    backend_options=backend_options, kinetics=kinetics, temperature=temperature)
+                    backend_options=backend_options, kinetics=kinetics, temperature=temperature,
+                    cell_area=plan.cell_area if cell_area is None else cell_area, min_depth=min_depth)
         self.boundary_data = plan.boundary_data
         self.mesh.attrs["boundary_data"] = plan.boundary_data
 
@@ -135,16 +140,20 @@ class ClearwaterRiverine:
     def from_arrays(cls, f1, f2, face_x, face_y, time_seconds, face_flow, edge_velocity, volume,
                     diffusion_coefficient: float, inputs: Dict[str, np.ndarray], units: Optional[Dict[str, str]] = None,
                     kinetics: Optional[Dict[str, Dict[str, Any]]] = None, temperature: Optional[str | float] = None,
+                    cell_area: Optional[np.ndarray] = None, min_depth: Optional[float] = None,
                     **backend_options) -> "ClearwaterRiverine":
+        """cell_area (F,): the plan area of every cell, which kinetics given per unit depth need; min_depth: the floor of
+        the depth V / cell_area (default kinetics.DEFAULT_MIN_DEPTH), both in the mesh's length unit."""
         self = cls.__new__(cls)
         self._setup(f1, f2, face_x, face_y, time_seconds, face_flow, edge_velocity, volume, float(diffusion_coefficient),
-                    inputs, units or {}, time=None, backend_options=backend_options, kinetics=kinetics, temperature=temperature)
+                    inputs, units or {}, time=None, backend_options=backend_options, kinetics=kinetics, temperature=temperature,
+                    cell_area=cell_area, min_depth=min_depth)
         self.boundary_data = None
         return self
 
     # ------------------------------------------------------------------------------------------
     def _setup(self, f1, f2, face_x, face_y, time_seconds, face_flow, edge_velocity, volume, D, inputs, units, time,
-               backend_options, kinetics=None, temperature=None):
+               backend_options, kinetics=None, temperature=None, cell_area=None, min_depth=None):
         store_mass_flux = backend_options.pop("store_mass_flux", True)
         # 'eager': update() returns with the results in the host arrays; 'pipelined': the copies overlap the next
         # update() (sync() before reading); 'none': results stay on the device (read them through self.backend)
@@ -192,6 +201,9 @@ class ClearwaterRiverine:
         for k, name in enumerate(self.constituents):
             self.backend.set_inputs(k, self.constituent_dict[name].input_array)
         self._index = {name: k for k, name in enumerate(self.constituents)}
+        from .kinetics import DEFAULT_MIN_DEPTH
+        self.cell_area = None if cell_area is None else np.array(cell_area, np.float64).reshape(F)
+        self.min_depth = DEFAULT_MIN_DEPTH if min_depth is None else float(min_depth)
         self.kinetics = None
         if kinetics is not None:
             self.set_kinetics(kinetics, 20.0 if temperature is None else temperature)
@@ -281,19 +293,24 @@ class ClearwaterRiverine:
         """Kinetics applied on the device in every later step, after the update_concentration override and before
         transport: first-order decay and yields, then zero-order sources and relaxation toward an equilibrium such as
         reaeration toward oxygen saturation, each optionally scaled by Monod limitation and inhibition factors such as
-        oxygen limitation of BOD oxidation (kinetics.py: spec format; temperature is a constituent name or a constant
-        in deg C).  None switches kinetics off.  History rows are not rewritten: the reaction of step t shows in row t + 1."""
+        oxygen limitation of BOD oxidation, and processes given per unit depth such as settling, areal sediment oxygen
+        demand or a surface transfer velocity, which act through each cell's depth V / cell_area (kinetics.py: spec format;
+        temperature is a constituent name or a constant in deg C).  None switches kinetics off.  History rows are not
+        rewritten: the reaction of step t shows in row t + 1."""
         from .kinetics import compile_kinetics
         if spec is None:
             self.backend.set_kinetics(None)
             self.kinetics = None
             return
-        kin = compile_kinetics(spec, self.constituents, temperature)
+        kin = compile_kinetics(spec, self.constituents, temperature, cell_area=self.cell_area, min_depth=self.min_depth,
+                               n_real=self.mesh.attrs[NUMBER_OF_REAL_CELLS] + 1)
         self.backend.set_kinetics(kin.decay_per_day, kin.theta, kin.yields, kin.temperature_k, kin.temperature_c)
         if kin.has_sources:
             self.backend.set_kinetics_sources(**kin.sources_arguments())
         if kin.has_limits:
             self.backend.set_kinetics_limits(**kin.limits_arguments())
+        if kin.has_depth:
+            self.backend.set_kinetics_depth(**kin.depth_arguments())
         self.kinetics = kin
 
     def sync(self):

@@ -234,13 +234,26 @@ int cwr_get_volume_sums(cwr_handle* h, double* total_sum, double* in_sum, double
  *     it, its own sink is self-limited and its equilibrium is >= 0.  The cap holds exactly in floating point for any
  *     yield: the rounded-down quotient keeps -yields[j, k] * loss <= c+_j.  This covers the reaction; transport adds
  *     only solver-tolerance noise.  Processes without factors are computed exactly as without cwr_set_kinetics_limits.
+ * With cwr_set_kinetics_depth, a process may be given per unit depth -- a settling velocity, an areal source such as
+ * sediment oxygen demand, a surface transfer velocity -- and acts through the depth of cell i at step t:
+ *         h_i = max(V_i[t] / A_i, min_depth)      (V[t]: the f32 volume of the load term and the reaction mass, in f64)
+ *     with A_i the cell's plan area.  A flagged rate, its theta^(T_i - 20) included, is divided by h_i before use, as a
+ *     product with the rounded reciprocal g_i = 1 / h_i (one division per cell):
+ *         decay:    r = decay_k * theta_k^(T_i - 20) / 86400 * g_i          (decay_k: a velocity, length / day)
+ *         source:   s = source_k * source_theta_k^(T_i - 20) / 86400 * g_i  (source_k: concentration x length / day)
+ *         exchange: r = exchange_k * exchange_theta_k^(T_i - 20) / 86400 * g_i   (exchange_k: length / day)
+ *     Everything else -- the yields, the Monod factors and the cap, the self-limited sink a = -s M' / (K + c+_k) with this
+ *     s, the order of the chain, the exact per-step solutions -- is unchanged, so the non-negativity guarantee above holds
+ *     at any depth, min_depth included.  Lengths are in the mesh's unit, volume unit / area unit: m for SI plans, ft for
+ *     US-customary ones.  An areal flux in g/m2/day on a plan in ft is given as flux / 0.3048 (mg/L ft/day); a velocity in
+ *     m/day as v / 0.3048.  A dry cell (V = 0) takes h = min_depth: its rates stay finite and its load term is 0.
  * O2sat is the APHA / Benson-Krause freshwater saturation at 1 atm, Ta = T + 273.15 K:
  *     ln O2sat = -139.34411 + 1.575701e5/Ta - 6.642308e7/Ta^2 + 1.243800e10/Ta^3 - 8.621949e11/Ta^4
  *
  * decay_per_day (K) or NULL = kinetics off; theta (K) or NULL = all 1; yields (K,K) row-major,
  * yields[j*K + k] = mass of j formed per mass of k decayed, or NULL = none; temperature_k = index of the
  * temperature constituent or -1 for the constant temperature_c.  Takes effect for steps queued after the call
- * (stream-ordered upload) and clears the sources and the limits.  CWR_EINVAL for a negative or non-finite decay, theta <= 0 or
+ * (stream-ordered upload) and clears the sources, the limits and the depth flags.  CWR_EINVAL for a negative or non-finite decay, theta <= 0 or
  * non-finite, a non-finite yield or yields[k*K + k] != 0, a cycle in the yield graph, a temperature constituent that
  * decays or receives a yield, an index out of range.  Domain decomposition: every rank makes the same call. */
 int cwr_set_kinetics(cwr_handle* h, const double* decay_per_day, const double* theta, const double* yields,
@@ -249,7 +262,7 @@ int cwr_set_kinetics(cwr_handle* h, const double* decay_per_day, const double* t
  * first-order chain of the kinetics set last (see above); all arrays (K).  source_per_day (concentration units per day)
  * or NULL = none; exchange_per_day (1/day) or NULL = none; both NULL = sources off; a theta NULL = all 1; equilibrium
  * (the constant target of kind 0); equilibrium_kind 0 = constant, 1 = O2sat(T), or NULL = all 0.  Acts only while
- * kinetics is set (all-zero decay rates are allowed); cwr_set_kinetics clears it; it clears the limits.  Stream-ordered
+ * kinetics is set (all-zero decay rates are allowed); cwr_set_kinetics clears it; it clears the limits and the depth flags.  Stream-ordered
  * upload.  CWR_EINVAL
  * when kinetics is not set, for a non-finite source, a theta <= 0 or non-finite, a negative or non-finite exchange, a kind
  * other than 0 or 1, exchange without equilibrium, a non-finite equilibrium of a kind-0 column with exchange > 0, or kind 1
@@ -269,6 +282,17 @@ int cwr_set_kinetics_sources(cwr_handle* h, const double* source_per_day, const 
  * decomposition: every rank makes the same call. */
 int cwr_set_kinetics_limits(cwr_handle* h, int n, const int* process, const int* column, const int* factor_column,
                             const int* factor_kind, const double* half_saturation);
+/* Depth-scaled processes of the kinetics and sources set last (see above).  cell_area (F) in reference numbering, the plan
+ * area of every cell (only the real cells are read); min_depth > 0 the floor of h; decay_per_depth, source_per_depth,
+ * exchange_per_depth (K) each 0 / 1 or NULL = none: 1 divides that process's rate of column k by h.  All flags NULL or 0 =
+ * depth off (cell_area may then be NULL).  Acts only while kinetics is set; cwr_set_kinetics and cwr_set_kinetics_sources
+ * clear it; it and cwr_set_kinetics_limits do not clear each other, so the order is kinetics, sources, then limits and
+ * depth in either order.  Stream-ordered upload, the areas permuted to the device order like the volumes.  CWR_EINVAL
+ * when kinetics is not set, for a flag other than 0 or 1, a flag on a process whose rate is 0, a flag with cell_area NULL,
+ * a real cell's area not finite and > 0, or min_depth not finite and > 0.  Domain decomposition: every rank makes the
+ * same call. */
+int cwr_set_kinetics_depth(cwr_handle* h, const double* cell_area, double min_depth, const int* decay_per_depth,
+                           const int* source_per_depth, const int* exchange_per_depth);
 /* Reaction mass of constituent k, sum over the steps taken of sum_i V[t]_i (c~'_ik - c~_ik), reduced on the device in a fixed
  * order (the same bits every run): a running sum since cwr_create, 0 while kinetics was never set.  Domain decomposition:
  * the partial sum over the rows the rank owns (as cwr_mass_totals_at). */

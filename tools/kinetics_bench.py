@@ -17,9 +17,12 @@ equilibrium temperature), with the temperature constituent and at a constant tem
 without its sources, alternately on the same handle: the step time and k_react's time (the CWR_FAM_RHS delta).
 With Monod factors (cwr_set_kinetics_limits), 1M x 16: the network with its sources and the factors of
 synthetic.make_kinetics_limits against the same network without the factors, alternately on the same handle, with the
-temperature constituent and at a constant temperature (--limits-only: this leg alone).  --parent-root DIR: the
-kinetics-only and the sources-only network timed in this tree's build and in DIR's (another checkout with its library
-built), one process per measurement, alternating, --parent-rounds times each; every process also reports the spread of
+temperature constituent and at a constant temperature (--limits-only: this leg alone).
+With depth-scaled processes (cwr_set_kinetics_depth), 1M x 16: the network with its sources and the flags of
+synthetic.make_kinetics_depth over the plan areas against the same network without the flags, alternately on the same
+handle, with the temperature constituent and at a constant temperature (--depth-only: this leg alone).
+--parent-root DIR: the kinetics-only, the sources-only and the sources-with-factors network timed in this tree's build
+and in DIR's (another checkout with its library built), one process per measurement, alternating, --parent-rounds times each; every process also reports the spread of
 its own repetitions.
 Prints one JSON object and writes it to --out.
 """
@@ -165,9 +168,61 @@ def limits_leg(torch, res, reps, scale):
     be.close()
 
 
+def alternate_depth(torch, be, kin, src, flags, dep, step, reps):
+    """The network with its sources, without and with its depth flags (kin, src: the unflagged rates; flags: the flagged
+    ones and the set_kinetics_depth arguments), alternately, reps times each: medians of the step time (ms, CUDA events)
+    and of the CWR_FAM_RHS family time (ms per step, in separate profiled steps)."""
+    out = {"step_ms": ([], []), "rhs_family_ms": ([], [])}
+    for _ in range(reps):
+        for i, with_depth in enumerate((False, True)):
+            k, s = (flags[0], flags[1]) if with_depth else (kin, src)
+            be.set_kinetics(**k)
+            be.set_kinetics_sources(**s)
+            if with_depth:
+                be.set_kinetics_depth(**dep)
+            step()
+            out["step_ms"][i].append(timed(torch, be, step, 5))
+            be.profile(1)
+            for _ in range(5):
+                step()
+            out["rhs_family_ms"][i].append(be.profile(-1)["rhs"][0] / 5)
+            be.profile(0)
+    return {f"{key}_{name}": float(np.median(v[i])) for key, v in out.items() for i, name in enumerate(("without", "with"))}
+
+
+def depth_leg(torch, res, reps, scale):
+    """1M x 16 with sources: without and with depth flags, with the temperature constituent and at a constant one."""
+    import bench
+    from clearwater_riverine_b200 import synthetic
+    plan, K = bench.workload_plan("1m16", 14, seed=0, scale=scale)
+    inputs, kin = synthetic.make_kinetics(synthetic.make_inputs(plan, K, seed=0), seed=0, decay_range=(0.05, 2.0))
+    src = synthetic.make_kinetics_sources(kin, seed=0, rate_range=(0.05, 2.0))
+    kin_d, src_d, flags = synthetic.make_kinetics_depth(kin, src, seed=0)
+    dep = dict(cell_area=plan.cell_area, min_depth=0.01, **flags)
+    be = build(plan, inputs, torch)
+    for t in range(3):
+        be.step(t)
+    step = lambda: be.step(3)
+    be.profile(1)
+    for _ in range(10):
+        step()
+    fam_off = be.profile(-1)["rhs"][0] / 10
+    be.profile(0)
+    for key, const in (("1m16_depth", False), ("1m16_depth_constant_temperature", True)):
+        c = (lambda k: dict(k, temperature_k=-1, temperature_c=24.0)) if const else (lambda k: k)
+        r = alternate_depth(torch, be, c(kin), src, (c(kin_d), src_d), dep, step, reps)
+        r["k_react_ms_without_depth"] = r["rhs_family_ms_without"] - fam_off
+        r["k_react_ms_with_depth"] = r["rhs_family_ms_with"] - fam_off
+        r["k_react_added_ms"] = r["rhs_family_ms_with"] - r["rhs_family_ms_without"]
+        r["step_added_ms"] = r["step_ms_with"] - r["step_ms_without"]
+        r["flagged_processes"] = {k: int(np.sum(v)) for k, v in flags.items()}
+        res[key] = r
+    be.close()
+
+
 def regression_child(reps, scale):
-    """One process of --parent-root: kinetics off, the kinetics-only and the sources-only 1M x 16 network (temperature
-    constituent) on one handle; medians and spreads (min, max) of the step time and of k_react's time (CWR_FAM_RHS
+    """One process of --parent-root: kinetics off, the kinetics-only, the sources-only and the sources-with-factors 1M x 16
+    network (temperature constituent) on one handle; medians and spreads (min, max) of the step time and of k_react's time (CWR_FAM_RHS
     delta).  Uses only calls both builds have."""
     import os
     import torch
@@ -177,11 +232,12 @@ def regression_child(reps, scale):
     plan, K = bench.workload_plan("1m16", 14, seed=0, scale=scale)
     inputs, kin = synthetic.make_kinetics(synthetic.make_inputs(plan, K, seed=0), seed=0, decay_range=(0.05, 2.0))
     src = synthetic.make_kinetics_sources(kin, seed=0, rate_range=(0.05, 2.0))
+    lim = synthetic.make_kinetics_limits(kin, src, seed=0)
     be = build(plan, inputs, torch)
     for t in range(3):
         be.step(t)
     step = lambda: be.step(3)
-    modes = {"off": None, "kinetics": (kin, None), "sources": (kin, src)}
+    modes = {"off": None, "kinetics": (kin, None, None), "sources": (kin, src, None), "limits": (kin, src, lim)}
     samples = {m: {"step_ms": [], "rhs_family_ms": []} for m in modes}
     for _ in range(reps):
         for m, v in modes.items():
@@ -191,6 +247,8 @@ def regression_child(reps, scale):
                 be.set_kinetics(**v[0])
                 if v[1] is not None:
                     be.set_kinetics_sources(**v[1])
+                if v[2] is not None:
+                    be.set_kinetics_limits(**v[2])
             step()
             samples[m]["step_ms"].append(timed(torch, be, step, 5))
             be.profile(1)
@@ -202,7 +260,7 @@ def regression_child(reps, scale):
     lib = Path(os.environ.get("CWR_B200_LIB", library_path())).resolve()   # what load_library actually loaded
     out = {"library": str(lib.relative_to(Path.cwd().resolve())) if lib.is_relative_to(Path.cwd().resolve()) else str(lib)}
     off = np.array(samples["off"]["rhs_family_ms"])
-    for m in ("kinetics", "sources"):
+    for m in ("kinetics", "sources", "limits"):
         st, fam = np.array(samples[m]["step_ms"]), np.array(samples[m]["rhs_family_ms"])
         react = fam - np.median(off)
         out[m] = {"step_ms": float(np.median(st)), "step_ms_min": float(st.min()), "step_ms_max": float(st.max()),
@@ -225,7 +283,7 @@ def parent_comparison(parent_root: str, rounds: int, reps: int, scale: float) ->
                 raise SystemExit(f"regression child failed ({name}):\n{out.stderr[-3000:]}")
             runs[name].append(json.loads(out.stdout.strip().splitlines()[-1]))
     res = {"rounds": rounds, "reps_per_round": reps, "runs": runs}
-    for m in ("kinetics", "sources"):
+    for m in ("kinetics", "sources", "limits"):
         for key in ("step_ms", "k_react_ms"):
             a = [r[m][key] for r in runs["this"]]
             b = [r[m][key] for r in runs["parent"]]
@@ -263,6 +321,7 @@ def main():
     ap.add_argument("--scale", type=float, default=1.0, help="1m16 mesh side scale (1.0 = 1M cells)")
     ap.add_argument("--out", default=None)
     ap.add_argument("--limits-only", action="store_true", help="only the Monod-factor leg (and --parent-root)")
+    ap.add_argument("--depth-only", action="store_true", help="only the depth leg (and --parent-root)")
     ap.add_argument("--parent-root", default=None,
                     help="another checkout with its library built: the no-factor networks timed in both builds, alternately")
     ap.add_argument("--parent-rounds", type=int, default=3)
@@ -278,8 +337,8 @@ def main():
     if not torch.cuda.is_available():
         raise SystemExit("kinetics_bench needs a CUDA device")
     res = {"gpu": gpu_name_and_power()}
-    if args.limits_only:
-        limits_leg(torch, res, args.reps, args.scale)
+    if args.limits_only or args.depth_only:
+        (limits_leg if args.limits_only else depth_leg)(torch, res, args.reps, args.scale)
         if args.parent_root:
             res["no_factor_paths_vs_parent"] = parent_comparison(args.parent_root, args.parent_rounds, max(3, args.reps // 3),
                                                                  args.scale)
@@ -355,6 +414,7 @@ def main():
         res[key]["coupled_device_ms_per_step"] = 1e3 * device_loop(torch, be, kin, 0, 100)
         be.close()
     limits_leg(torch, res, args.reps, args.scale)
+    depth_leg(torch, res, args.reps, args.scale)
     if args.parent_root:
         res["no_factor_paths_vs_parent"] = parent_comparison(args.parent_root, args.parent_rounds, max(3, args.reps // 3),
                                                              args.scale)
