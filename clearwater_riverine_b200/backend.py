@@ -108,6 +108,7 @@ def load_library():
         "cwr_set_kinetics_sources": ([H, dp, dp, dp, dp, dp, ip], C.c_int),
         "cwr_set_kinetics_limits": ([H, C.c_int, ip, ip, ip, ip, dp], C.c_int),
         "cwr_set_kinetics_depth": ([H, dp, C.c_double, ip, ip, ip], C.c_int),
+        "cwr_set_kinetics_forcing": ([H, C.c_int, C.c_int, ip, ip, dp], C.c_int),
         "cwr_get_reaction_mass": ([H, C.c_int, dp], C.c_int),
         "cwr_get_lhs": ([H, C.POINTER(C.c_int64), ip, ip, dp], C.c_int),
         "cwr_get_rhs": ([H, C.c_int, dp], C.c_int),
@@ -482,6 +483,27 @@ class TransportBackend:
         area = None if cell_area is None else _arr(cell_area, np.float64, (self.n_face,), "cell_area")
         rc = self._lib.cwr_set_kinetics_depth(self._h, _ptr(area, C.c_double), float(min_depth),
                                               *[_ptr(a, C.c_int32) for a in flags])
+        if rc == CWR_EINVAL:
+            raise ValueError(self._lib.cwr_last_error(self._h).decode())
+        self._check(rc)
+
+    def set_kinetics_forcing(self, target=None, column=None, values=None):
+        """Time-varying forcing of the kinetics and sources set last (cwr_set_kinetics_forcing): (n,) target (0 the
+        temperature, column -1; 1 the equilibrium of column k; 2, 3, 4 scales of its decay, source and exchange rate) and
+        column, values (n, n_time): step t uses values[:, t].  target None or n == 0 = forcing off.  set_kinetics and
+        set_kinetics_sources clear it; set_kinetics_limits and set_kinetics_depth do not.  An invalid set raises
+        ValueError.  kinetics.compile_kinetics builds the arrays from series given by constituent name."""
+        if target is None or len(target) == 0:
+            self._check(self._lib.cwr_set_kinetics_forcing(self._h, 0, self.n_time, None, None, None))
+            return
+        tg = _arr(target, np.int32).reshape(-1)
+        n = tg.shape[0]
+        col = _arr(column, np.int32, (n,), "column")
+        v = np.ascontiguousarray(values, np.float64)
+        if v.ndim != 2 or v.shape[0] != n:
+            raise ValueError(f"values: expected shape ({n}, n_time), got {v.shape}")
+        rc = self._lib.cwr_set_kinetics_forcing(self._h, n, v.shape[1], _ptr(tg, C.c_int32), _ptr(col, C.c_int32),
+                                                _ptr(v, C.c_double))
         if rc == CWR_EINVAL:
             raise ValueError(self._lib.cwr_last_error(self._h).decode())
         self._check(rc)

@@ -134,6 +134,12 @@ struct cwr_handle {
     double kin_min_depth = 0.0;
     std::vector<double> kin_area_h;
     double* d_kin_area = nullptr; int* d_kin_dflag = nullptr; int* d_kin_fptr0 = nullptr;
+    // time-varying forcing (cwr_set_kinetics_forcing): the (n, T) series (d_kin_force, room for 1 + 4K of them, allocated
+    // by the first call) and the series row of every forced parameter (d_kin_fmap, 1 + n_steps + 3 n_src, see k_react);
+    // the kForced instantiations of k_react run while kin_forced.  kin_kind_h: the equilibrium kind of every column
+    bool kin_forced = false;
+    double* d_kin_force = nullptr; int* d_kin_fmap = nullptr;
+    std::vector<int> kin_kind_h;
     // optional per-kernel-family timing with CUDA events on the handle's stream (bench.py roofline)
     bool profiling = false;
     std::vector<cudaEvent_t> ev_pool;
@@ -1367,9 +1373,12 @@ static int build_rhs(cwr_handle* h, int t, int accumulate) {
         // after cwr_set_kinetics), at most the resident grid; the same rows give the same grid, hence the same sums
         const int R = react_tile_rows(h->K);
         const int grid = grid_for((M.row_hi - M.row_lo + R - 1) / R, 1, h->kin_grid_max);
-        auto* fn = h->kin_depth ? k_react<true, true> : h->kin_facs ? k_react<true> : k_react<false>;
+        auto* fn = h->kin_forced ? (h->kin_depth ? k_react<true, true, true> : h->kin_facs ? k_react<true, false, true> : k_react<false, false, true>)
+                                 : (h->kin_depth ? k_react<true, true> : h->kin_facs ? k_react<true> : k_react<false>);
         const int* fptr = h->kin_depth && !h->kin_facs ? h->d_kin_fptr0 : h->d_kin_fptr;
-        CK(launch_chain(h, fn, grid, kThreads, react_smem_bytes(h->K) + react_src_smem_bytes(h->kin_srcs, h->kin_temp_k), M,
+        const size_t smem = react_smem_bytes(h->K) + react_src_smem_bytes(h->kin_srcs, h->kin_temp_k) +
+                            (h->kin_forced ? react_force_smem_bytes(h->kin_srcs) : 0);
+        CK(launch_chain(h, fn, grid, kThreads, smem, M,
                         (const KinStep*)h->d_kin_steps, h->kin_steps, (const KinYield*)h->d_kin_yields, h->kin_temp_k, h->kin_temp_c,
                         (const KinSrc*)h->d_kin_srcs, h->kin_srcs, h->kin_src_o2, (const KinFac*)h->d_kin_facs,
                         fptr, h->d_kin_partials, h->d_kin_state, accumulate, (const double*)h->d_kin_area,
@@ -1725,7 +1734,7 @@ int cwr_set_kinetics(cwr_handle* h, const double* decay, const double* theta, co
                      double temperature_c) {
     if (!h) return CWR_EINVAL;
     const int K = h->K;
-    if (!decay) { h->kin_on = false; h->kin_srcs = 0; h->kin_facs = 0; h->kin_depth = false; return CWR_OK; }
+    if (!decay) { h->kin_on = false; h->kin_srcs = 0; h->kin_facs = 0; h->kin_depth = false; h->kin_forced = false; return CWR_OK; }
     for (int k = 0; k < K; ++k) {
         if (!std::isfinite(decay[k]) || decay[k] < 0.0) FAIL(CWR_EINVAL, "cwr_set_kinetics: decay rates must be finite and >= 0");
         if (theta && (!std::isfinite(theta[k]) || theta[k] <= 0.0)) FAIL(CWR_EINVAL, "cwr_set_kinetics: theta must be finite and > 0");
@@ -1774,12 +1783,13 @@ int cwr_set_kinetics(cwr_handle* h, const double* decay, const double* theta, co
     }
     CK(cudaSetDevice(h->device));
     if (!h->d_kin_state) {
-        cudaFuncAttributes fa{}, fl{}, fd{};
-        CK(cudaFuncGetAttributes(&fa, k_react<false>));
-        CK(cudaFuncGetAttributes(&fl, k_react<true>));
-        CK(cudaFuncGetAttributes(&fd, k_react<true, true>));
-        if (std::max({fa.sharedSizeBytes, fl.sharedSizeBytes, fd.sharedSizeBytes}) > kReactStaticSmem)
-            FAIL(CWR_ECUDA, "k_react: static shared memory exceeds what its tile sizing reserves");
+        for (auto* fn : {k_react<false>, k_react<true>, k_react<true, true>, k_react<false, false, true>,
+                         k_react<true, false, true>, k_react<true, true, true>}) {
+            cudaFuncAttributes fa{};
+            CK(cudaFuncGetAttributes(&fa, fn));
+            if (fa.sharedSizeBytes > kReactStaticSmem)
+                FAIL(CWR_ECUDA, "k_react: static shared memory exceeds what its tile sizing reserves");
+        }
         // the grid of every instantiation (the factored ones may hold fewer CTAs per SM; their CTAs need not be co-resident)
         int occ = 0;
         CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_react<false>, kThreads, react_smem_bytes(K)));
@@ -1808,6 +1818,7 @@ int cwr_set_kinetics(cwr_handle* h, const double* decay, const double* theta, co
     h->kin_srcs = 0;
     h->kin_facs = 0;
     h->kin_depth = false;
+    h->kin_forced = false;
     h->kin_decay_h.assign(decay, decay + K);
     h->kin_yields_h.assign((size_t)K * K, 0.0);
     if (yields) h->kin_yields_h.assign(yields, yields + (size_t)K * K);
@@ -1816,6 +1827,7 @@ int cwr_set_kinetics(cwr_handle* h, const double* decay, const double* theta, co
     h->kin_source_h.assign(K, 0.0);
     h->kin_exchange_h.assign(K, 0.0);
     h->kin_src_of.assign(K, -1);
+    h->kin_kind_h.assign(K, 0);
     return CWR_OK;
 }
 
@@ -1825,8 +1837,8 @@ int cwr_set_kinetics_sources(cwr_handle* h, const double* source_per_day, const 
     const int K = h->K;
     if (!h->kin_on) FAIL(CWR_EINVAL, "cwr_set_kinetics_sources: call cwr_set_kinetics first");
     if (!source_per_day && !exchange_per_day) {
-        h->kin_srcs = 0; h->kin_facs = 0; h->kin_depth = false;
-        h->kin_source_h.assign(K, 0.0); h->kin_exchange_h.assign(K, 0.0); h->kin_src_of.assign(K, -1);
+        h->kin_srcs = 0; h->kin_facs = 0; h->kin_depth = false; h->kin_forced = false;
+        h->kin_source_h.assign(K, 0.0); h->kin_exchange_h.assign(K, 0.0); h->kin_src_of.assign(K, -1); h->kin_kind_h.assign(K, 0);
         return CWR_OK;
     }
     if (exchange_per_day && !equilibrium) FAIL(CWR_EINVAL, "cwr_set_kinetics_sources: exchange needs an equilibrium array");
@@ -1872,13 +1884,16 @@ int cwr_set_kinetics_sources(cwr_handle* h, const double* source_per_day, const 
     h->kin_src_o2 = o2;
     h->kin_facs = 0;
     h->kin_depth = false;
+    h->kin_forced = false;
     h->kin_source_h.assign(K, 0.0);
     h->kin_exchange_h.assign(K, 0.0);
     h->kin_src_of.assign(K, -1);
+    h->kin_kind_h.assign(K, 0);
     for (size_t p = 0; p < list.size(); ++p) {
         h->kin_source_h[list[p].col] = list[p].source;
         h->kin_exchange_h[list[p].col] = list[p].exchange;
         h->kin_src_of[list[p].col] = (int)p;
+        h->kin_kind_h[list[p].col] = list[p].kind;
     }
     return CWR_OK;
 }
@@ -1969,6 +1984,67 @@ int cwr_set_kinetics_depth(cwr_handle* h, const double* cell_area, double min_de
     CK(cudaMemcpyAsync(h->d_kin_dflag, dflag.data(), dflag.size() * sizeof(int), cudaMemcpyHostToDevice, h->stream));
     h->kin_min_depth = min_depth;
     h->kin_depth = true;
+    return CWR_OK;
+}
+
+int cwr_set_kinetics_forcing(cwr_handle* h, int n, int n_time, const int* target, const int* column, const double* values) {
+    if (!h) return CWR_EINVAL;
+    const int K = h->K, T = h->T;
+    if (!h->kin_on) FAIL(CWR_EINVAL, "cwr_set_kinetics_forcing: call cwr_set_kinetics first");
+    if (n < 0) FAIL(CWR_EINVAL, "cwr_set_kinetics_forcing: n must be >= 0");
+    if (n == 0) { h->kin_forced = false; return CWR_OK; }
+    if (n_time != T) FAIL(CWR_EINVAL, "cwr_set_kinetics_forcing: n_time must be the handle's n_time");
+    if (!target || !column || !values) FAIL(CWR_EINVAL, "cwr_set_kinetics_forcing: NULL array with n > 0");
+    const double* rate[5] = {nullptr, nullptr, h->kin_decay_h.data(), h->kin_source_h.data(), h->kin_exchange_h.data()};
+    std::vector<int> seen;
+    for (int i = 0; i < n; ++i) {
+        const int g = target[i], k = column[i];
+        if (g < CWR_FORCE_TEMPERATURE || g > CWR_FORCE_EXCHANGE_SCALE) FAIL(CWR_EINVAL, "cwr_set_kinetics_forcing: unknown target");
+        if (g == CWR_FORCE_TEMPERATURE) {
+            if (k != -1) FAIL(CWR_EINVAL, "cwr_set_kinetics_forcing: the temperature series takes column -1");
+            if (h->kin_temp_k >= 0)
+                FAIL(CWR_EINVAL, "cwr_set_kinetics_forcing: a temperature series while a temperature constituent is set");
+        } else if (k < 0 || k >= K) FAIL(CWR_EINVAL, "cwr_set_kinetics_forcing: column index out of range");
+        seen.push_back(g * (K + 1) + k + 1);
+        const double* v = values + (size_t)i * T;
+        for (int t = 0; t < T; ++t) {
+            if (!std::isfinite(v[t])) FAIL(CWR_EINVAL, "cwr_set_kinetics_forcing: a series value is not finite");
+            if (g >= CWR_FORCE_DECAY_SCALE && v[t] < 0.0) FAIL(CWR_EINVAL, "cwr_set_kinetics_forcing: a scale is negative");
+        }
+        if (g >= CWR_FORCE_DECAY_SCALE && rate[g][k] == 0.0)
+            FAIL(CWR_EINVAL, "cwr_set_kinetics_forcing: a scale on a process whose rate is 0");
+        if (g == CWR_FORCE_EQUILIBRIUM && h->kin_exchange_h[k] == 0.0)
+            FAIL(CWR_EINVAL, "cwr_set_kinetics_forcing: an equilibrium series on a column without exchange");
+        if (g == CWR_FORCE_EQUILIBRIUM && h->kin_kind_h[k] != 0)
+            FAIL(CWR_EINVAL, "cwr_set_kinetics_forcing: an equilibrium series on a column that relaxes toward oxygen saturation");
+    }
+    std::sort(seen.begin(), seen.end());
+    if (std::adjacent_find(seen.begin(), seen.end()) != seen.end())
+        FAIL(CWR_EINVAL, "cwr_set_kinetics_forcing: the same (target, column) given twice");
+    // the series row of every forced parameter, numbered as k_react reads them (-1: not forced)
+    std::vector<int> fmap(1 + h->kin_steps + 3 * h->kin_srcs, -1);
+    for (int i = 0; i < n; ++i) {
+        const int g = target[i], k = column[i];
+        if (g == CWR_FORCE_TEMPERATURE) fmap[0] = i;
+        else if (g == CWR_FORCE_DECAY_SCALE) fmap[1 + h->kin_step_of[k]] = i;
+        else fmap[1 + h->kin_steps + 3 * h->kin_src_of[k] + (g == CWR_FORCE_SOURCE_SCALE ? 0 : g == CWR_FORCE_EXCHANGE_SCALE ? 1 : 2)] = i;
+    }
+    CK(cudaSetDevice(h->device));
+    if (!h->d_kin_force) {
+        CK(dalloc(h, &h->d_kin_force, (size_t)(1 + 4 * K) * T));
+        CK(dalloc(h, &h->d_kin_fmap, (size_t)1 + 4 * K));
+        h->M.kin_force = h->d_kin_force; h->M.kin_fmap = h->d_kin_fmap; h->M.n_time = T;
+        // the forced source columns take shared memory beyond the coefficients (react_force_smem_bytes)
+        for (auto* fn : {k_react<false, false, true>, k_react<true, false, true>, k_react<true, true, true>})
+            CK(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                    (int)(kReactSmemLimit - kReactStaticSmem + react_src_smem_bytes(kMaxK, -1) +
+                                          react_force_smem_bytes(kMaxK))));
+    }
+    // stream-ordered, from host copies: steps queued before this call still read the previous series
+    std::vector<double> table(values, values + (size_t)n * T);
+    CK(cudaMemcpyAsync(h->d_kin_force, table.data(), table.size() * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(h->d_kin_fmap, fmap.data(), fmap.size() * sizeof(int), cudaMemcpyHostToDevice, h->stream));
+    h->kin_forced = true;
     return CWR_OK;
 }
 

@@ -135,6 +135,11 @@ struct DeviceModel {
     double diffusion_coefficient;
     int max_iter;
     int want_flux;
+    // time-varying kinetics forcing (cwr_set_kinetics_forcing; read only by k_react's kForced instantiations): the
+    // (n, n_time) series and the series row of every forced parameter
+    const double* kin_force;
+    const int* kin_fmap;
+    int n_time;
 };
 
 // Programmatic dependent launch (small-mesh path: a step is a chain of 6 - 8 launches of a few microseconds each, so the
@@ -561,6 +566,13 @@ __device__ __forceinline__ void grid_totals(const double* partials, double* tot,
 // bit 1 the exchange.  A flagged process is evaluated per row by the factored code (at a constant temperature too); the
 // others keep their per-CTA coefficients.  Only k_react<true, true> (launched while depth flags are set, with an
 // all-empty fptr when there are no factors) has the depth code; it takes the same tile and grid as the others.
+// Time-varying forcing (cwr_set_kinetics_forcing) replaces or scales a per-launch parameter with entry sp.t of a series,
+// fv[row * n_time + sp.t] (fv = M.kin_force, fmap = M.kin_fmap); fmap names the row of each parameter (-1: not forced): fmap[0] the constant temperature,
+// fmap[1 + p] the decay of step p, fmap[1 + n_steps + 3 p + {0, 1, 2}] the source, the exchange rate and the constant
+// equilibrium of source column p.  A scale multiplies the per-day rate before anything else touches it, so the CTA
+// prologue writes decay f into st[] and the forced KinSrc of every source column into dynamic shared memory
+// (react_force_smem_bytes), and the row loop runs the code above on them.  Only the kForced instantiations (launched while
+// forcing is set) read fv; each takes the same tile and grid as its unforced twin.
 // ---------------------------------------------------------------------------------------------
 struct KinStep { int col, y_begin, y_end, pad; double decay, log_theta; };   // a reacting constituent; its yields
 struct KinYield { int col, pad; double y; };                                 // [y_begin, y_end)
@@ -664,6 +676,10 @@ static_assert(react_smem_fits_every_k(), "k_react's shared memory must fit in 48
 __host__ __device__ constexpr size_t react_src_smem_bytes(int n_src, int temp_k) {
     return temp_k < 0 ? (size_t)3 * n_src * sizeof(double) : 0;
 }
+// [n_src] the forced KinSrc of every source column, after the coefficients; only while forcing is set
+__host__ __device__ constexpr size_t react_force_smem_bytes(int n_src) {
+    return (size_t)n_src * sizeof(KinSrc);
+}
 
 // f(e) for the elements [0, cnt) of a tile of the interleaved state that starts at `base`: each thread takes pairs that
 // are 16-byte aligned there, the unpaired element at either end is taken by one thread.  (A state slot starts at an odd
@@ -679,7 +695,7 @@ __device__ __forceinline__ void react_pairs(const double* base, int cnt, F f) {
     }
 }
 
-template <bool kLimited, bool kDepth = false>
+template <bool kLimited, bool kDepth = false, bool kForced = false>
 __global__ void __launch_bounds__(kThreads) k_react(DeviceModel M, const KinStep* __restrict__ steps, int n_steps,
                                                     const KinYield* __restrict__ yl, int temp_k, double temp_c,
                                                     const KinSrc* __restrict__ srcs, int n_src, int src_o2,
@@ -700,15 +716,35 @@ __global__ void __launch_bounds__(kThreads) k_react(DeviceModel M, const KinStep
     double* red = fac + kMaxK;                // [kThreads] column sums
     double* sco = red + kThreads;             // [3 n_src] constant temperature: s + r ceq, r, phi (react_src_smem_bytes)
     const double dt = sp.dt;
+    const KinSrc* sv = srcs;                  // the source columns the row loop reads (forced: their shared copies)
+    double tc = temp_c;                       // the constant temperature of the step (the prologue's)
+    const double* __restrict__ fv = M.kin_force;
+    const int* __restrict__ fmap = M.kin_fmap;
+    const int n_time = M.n_time;
+    if constexpr (kForced) {                  // entry sp.t of every series: a few loads per CTA
+        const double* f = fv + sp.t;
+        const int* fs = fmap + 1 + n_steps;
+        KinSrc* ss = reinterpret_cast<KinSrc*>(sco + (temp_k < 0 ? 3 * n_src : 0));   // react_force_smem_bytes
+        if (fmap[0] >= 0) tc = f[(size_t)fmap[0] * n_time];
+        if (threadIdx.x == 0) red[0] = tc;    // the rows read it from there (red is free until the column sums)
+        for (int p = threadIdx.x; p < n_src; p += blockDim.x) {
+            ss[p] = srcs[p];
+            if (fs[3 * p] >= 0) ss[p].source = ss[p].source * f[(size_t)fs[3 * p] * n_time];
+            if (fs[3 * p + 1] >= 0) ss[p].exchange = ss[p].exchange * f[(size_t)fs[3 * p + 1] * n_time];
+            if (fs[3 * p + 2] >= 0) ss[p].equilibrium = f[(size_t)fs[3 * p + 2] * n_time];
+        }
+        sv = ss;
+    }
     for (int p = threadIdx.x; p < n_steps; p += blockDim.x) {
-        const KinStep s = steps[p];
+        KinStep s = steps[p];
+        if (kForced && fmap[1 + p] >= 0) s.decay = s.decay * fv[(size_t)fmap[1 + p] * n_time + sp.t];
         st[p] = s;
-        if (temp_k < 0) fac[p] = -expm1(-(s.decay * exp((temp_c - 20.0) * s.log_theta) / 86400.0) * dt);
+        if (temp_k < 0) fac[p] = -expm1(-(s.decay * exp((tc - 20.0) * s.log_theta) / 86400.0) * dt);
     }
     if (temp_k < 0)
-        for (int p = threadIdx.x; p < n_src; p += blockDim.x) {
-            const KinSrc s = srcs[p];
-            kin_src_coef(s, temp_c, s.kind ? o2_saturation(temp_c) : 0.0, dt, sco[3 * p], sco[3 * p + 1], sco[3 * p + 2]);
+        for (int p = threadIdx.x; p < n_src; p += blockDim.x) {    // (forced: sv[p] was written by this thread)
+            const KinSrc s = sv[p];
+            kin_src_coef(s, tc, s.kind ? o2_saturation(tc) : 0.0, dt, sco[3 * p], sco[3 * p + 1], sco[3 * p + 2]);
         }
     __syncthreads();
     // column sums: thread (g, k) adds rows g, g + G, ... of every tile the CTA takes, in that order
@@ -733,7 +769,7 @@ __global__ void __launch_bounds__(kThreads) k_react(DeviceModel M, const KinStep
         __syncthreads();
         if (threadIdx.x < rows) {             // one row's chain per thread
             double* c = tile + threadIdx.x * ld;
-            const double T = temp_k < 0 ? temp_c : c[temp_k];
+            const double T = temp_k < 0 ? (kForced ? red[0] : temp_c) : c[temp_k];
             const double hinv = kDepth ? 1.0 / fmax(svol[threadIdx.x] / area[row0 + threadIdx.x], min_depth) : 1.0;
             for (int p = 0; p < n_steps; ++p) {
                 const KinStep& s = st[p];
@@ -756,28 +792,28 @@ __global__ void __launch_bounds__(kThreads) k_react(DeviceModel M, const KinStep
                     const int fb = fptr[n_steps + p], fe = fptr[n_steps + p + 1];
                     const int df = kDepth ? dfl[n_steps + p] : 0;
                     if (fb != fe || df) {
-                        kin_src_limited<kDepth>(c, srcs + p, fl + fb, fe - fb, T, o2, dt, hinv, df);
+                        kin_src_limited<kDepth>(c, sv + p, fl + fb, fe - fb, T, o2, dt, hinv, df);
                     } else if (temp_k < 0) {
                         const double* q = sco + 3 * p;
-                        double& v = c[srcs[p].col];
+                        double& v = c[sv[p].col];
                         v += (q[0] - q[1] * v) * q[2];
                     } else {
                         double sr, r, phi;
-                        kin_src_coef(srcs[p], T, o2, dt, sr, r, phi);
-                        double& v = c[srcs[p].col];
+                        kin_src_coef(sv[p], T, o2, dt, sr, r, phi);
+                        double& v = c[sv[p].col];
                         v += (sr - r * v) * phi;
                     }
                 }
             } else if (temp_k < 0) {
                 for (int p = 0; p < n_src; ++p) {
                     const double* q = sco + 3 * p;
-                    double& v = c[srcs[p].col];
+                    double& v = c[sv[p].col];
                     v += (q[0] - q[1] * v) * q[2];
                 }
             } else if (n_src > 0) {
                 const double o2 = src_o2 ? o2_saturation(T) : 0.0;
                 for (int p = 0; p < n_src; ++p) {
-                    const KinSrc s = srcs[p];
+                    const KinSrc s = sv[p];
                     double sr, r, phi;
                     kin_src_coef(s, T, o2, dt, sr, r, phi);
                     double& v = c[s.col];

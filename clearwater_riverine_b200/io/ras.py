@@ -129,12 +129,29 @@ def build_input_array(
     inp[0, ic["Cell_Index"].astype(int).to_numpy()] = ic["Concentration"].to_numpy()
     bc = boundary_conditions if isinstance(boundary_conditions, pd.DataFrame) \
         else pd.read_csv(boundary_conditions, parse_dates=["Datetime"])
-    model = pd.DataFrame({"Datetime": pd.DatetimeIndex(time), "Time Index": np.arange(n_time)})
     f2 = np.asarray(f2)
     for name, group in bc.groupby("RAS2D_TS_Name"):
-        merged = pd.merge_asof(model, group.sort_values("Datetime"), on="Datetime")
-        conc = merged["Concentration"].interpolate(method="linear").to_numpy()
+        conc = series_on_model_times(time, group["Datetime"], group["Concentration"])
         faces = boundary_data.loc[boundary_data["Name"] == name, "Face Index"].to_numpy(dtype=np.int64)
         if len(faces):
             inp[:, f2[faces]] = conc[:, None]
     return inp
+
+
+def series_on_model_times(time: np.ndarray, datetime, values) -> np.ndarray:
+    """(T,) float64: a time series (datetime, values) put onto the model times `time` as the boundary conditions are
+    (reference constituents.py:100-164): a backward `merge_asof` (the last sample at or before each model time), then
+    linear interpolation over the model times that have none.  Model times before the first sample stay NaN."""
+    model = pd.DataFrame({"Datetime": pd.DatetimeIndex(time), "Time Index": np.arange(len(time))})
+    src = pd.DataFrame({"Datetime": pd.DatetimeIndex(datetime), "Value": np.asarray(values, np.float64)})
+    merged = pd.merge_asof(model, src.sort_values("Datetime"), on="Datetime")
+    return merged["Value"].interpolate(method="linear").to_numpy()
+
+
+def read_series_csv(path: str | Path, time: np.ndarray) -> np.ndarray:
+    """(T,) float64: the `Datetime`, `Value` columns of a CSV file put onto the model times (series_on_model_times)."""
+    df = pd.read_csv(path, parse_dates=["Datetime"])
+    for col in ("Datetime", "Value"):
+        if col not in df:
+            raise ValueError(f"{path}: a series CSV needs the columns Datetime and Value; {col} is missing")
+    return series_on_model_times(time, df["Datetime"], df["Value"])

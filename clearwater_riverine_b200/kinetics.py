@@ -30,6 +30,14 @@ through the surface -- are given per unit depth, each in place of its volumetric
               "transfer_per_day": 2.0, "equilibrium": "oxygen_saturation"}}      # K_L, length/day: r = K_L / h
 
 with h = max(V / A, min_depth) the depth of each cell at each step, in the mesh's length unit (volume unit / area unit).
+Quantities that change with time are series of n_time values, one per model time index (step t uses entry t): a scale
+of a rate (`decay_scale`, `source_scale`, `exchange_scale`, >= 0, multiplying the per-day rate before anything else acts
+on it), an equilibrium that moves (`equilibrium` as a series), and the temperature (`temperature=` as a series):
+
+    {"DO": {"source_per_day": 8.0, "source_scale": light / light.max(),          # photosynthesis Pmax I(t) / Imax
+            "exchange_per_day": 2.0, "exchange_scale": wind_factor, "equilibrium": "oxygen_saturation"},
+     "T":  {"exchange_per_day": 0.5, "equilibrium": Te}}                           # Te(t) from meteorology
+
 The library checks the same conditions; checking them here names the constituents in the error.
 """
 from __future__ import annotations
@@ -42,7 +50,7 @@ import numpy as np
 
 _KEYS = {"decay_per_day", "theta", "yields", "source_per_day", "source_theta", "exchange_per_day", "exchange_theta",
          "equilibrium", "limited_by", "inhibited_by", "source_limited_by", "source_inhibited_by", "settling_per_day",
-         "areal_source_per_day", "transfer_per_day"}
+         "areal_source_per_day", "transfer_per_day", "decay_scale", "source_scale", "exchange_scale"}
 OXYGEN_SATURATION = "oxygen_saturation"
 # per-depth spec key -> the volumetric key it replaces (the rate of the same process, divided by the depth)
 _DEPTH_KEYS = {"settling_per_day": "decay_per_day", "areal_source_per_day": "source_per_day",
@@ -52,6 +60,13 @@ _DEPTH_KEYS = {"settling_per_day": "decay_per_day", "areal_source_per_day": "sou
 DEFAULT_MIN_DEPTH = 0.01
 # spec key -> (process: 0 decay, 1 source; kind: 0 limitation, 1 inhibition), in the order a block's factors compile
 _FACTOR_KEYS = {"limited_by": (0, 0), "source_limited_by": (1, 0), "inhibited_by": (0, 1), "source_inhibited_by": (1, 1)}
+# the targets of cwr_set_kinetics_forcing: what series i replaces (temperature, equilibrium) or scales (the rest)
+FORCE_TEMPERATURE, FORCE_EQUILIBRIUM, FORCE_DECAY_SCALE, FORCE_SOURCE_SCALE, FORCE_EXCHANGE_SCALE = range(5)
+_FORCE_NAMES = ("temperature", "equilibrium", "decay_scale", "source_scale", "exchange_scale")
+# spec key of a scale series -> its target
+_SCALE_KEYS = {"decay_scale": FORCE_DECAY_SCALE, "source_scale": FORCE_SOURCE_SCALE, "exchange_scale": FORCE_EXCHANGE_SCALE}
+# the spec keys that may be given as a series (and so as {csv: path} in a config file)
+SERIES_KEYS = ("equilibrium",) + tuple(_SCALE_KEYS)
 
 
 def oxygen_saturation(T):
@@ -90,6 +105,11 @@ class Kinetics:
     exchange_per_depth: Optional[np.ndarray] = None
     cell_area: Optional[np.ndarray] = None
     min_depth: float = DEFAULT_MIN_DEPTH
+    # time-varying forcing: series i, values (n, n_time), has target forcing_target[i] (int32, FORCE_*) on column
+    # forcing_column[i] (int32, -1 for the temperature); step t uses forcing_values[:, t]
+    forcing_target: Optional[np.ndarray] = None
+    forcing_column: Optional[np.ndarray] = None
+    forcing_values: Optional[np.ndarray] = None
 
     @property
     def has_sources(self) -> bool:
@@ -122,6 +142,15 @@ class Kinetics:
         return dict(cell_area=self.cell_area, min_depth=self.min_depth, decay_per_depth=self.decay_per_depth,
                     source_per_depth=self.source_per_depth, exchange_per_depth=self.exchange_per_depth)
 
+    @property
+    def has_forcing(self) -> bool:
+        """Whether any parameter follows a series (otherwise cwr_set_kinetics_forcing is not needed)."""
+        return self.forcing_target is not None and len(self.forcing_target) > 0
+
+    def forcing_arguments(self) -> dict:
+        """The arguments of TransportBackend.set_kinetics_forcing."""
+        return dict(target=self.forcing_target, column=self.forcing_column, values=self.forcing_values)
+
 
 def topological_order(yields: np.ndarray) -> Tuple[int, ...]:
     """Order of the constituents in which every one comes after all those it receives a yield from (edges k -> j where
@@ -146,11 +175,13 @@ def validate(decay_per_day, theta, yields, temperature_k: int, temperature_c: fl
              source_per_day=None, source_theta=None, exchange_per_day=None, exchange_theta=None, equilibrium=None,
              equilibrium_kind=None, limit_process=None, limit_column=None, limit_factor_column=None, limit_kind=None,
              limit_half_saturation=None, decay_per_depth=None, source_per_depth=None, exchange_per_depth=None,
-             cell_area=None, min_depth: float = DEFAULT_MIN_DEPTH) -> None:
-    """The conditions cwr_set_kinetics, cwr_set_kinetics_sources, cwr_set_kinetics_limits and cwr_set_kinetics_depth
-    reject with CWR_EINVAL, as ValueError.  The source arrays follow the ABI: None = none / all 1 / all 0 as there; the
-    limit arrays are (n,) or None = no limits; the depth flags (K,) or None = none; cell_area: the plan areas of the real
-    cells (the ones the library reads), or None."""
+             cell_area=None, min_depth: float = DEFAULT_MIN_DEPTH, forcing_target=None, forcing_column=None,
+             forcing_values=None, n_time: Optional[int] = None) -> None:
+    """The conditions cwr_set_kinetics, cwr_set_kinetics_sources, cwr_set_kinetics_limits, cwr_set_kinetics_depth and
+    cwr_set_kinetics_forcing reject with CWR_EINVAL, as ValueError.  The source arrays follow the ABI: None = none / all 1
+    / all 0 as there; the limit arrays are (n,) or None = no limits; the depth flags (K,) or None = none; cell_area: the
+    plan areas of the real cells (the ones the library reads), or None; the forcing arrays (n,), (n,), (n, n_time) or
+    None = no forcing, n_time the model's number of time indices (None: the series' own length)."""
     d, th, y = np.asarray(decay_per_day, np.float64), np.asarray(theta, np.float64), np.asarray(yields, np.float64)
     K = d.shape[0]
     nm = (lambda k: repr(names[k])) if len(names) == K else (lambda k: f"#{k}")
@@ -178,6 +209,8 @@ def validate(decay_per_day, theta, yields, temperature_k: int, temperature_c: fl
                      limit_half_saturation)
     _validate_depth(d, source_per_day, exchange_per_day, nm, decay_per_depth, source_per_depth, exchange_per_depth,
                     cell_area, min_depth)
+    _validate_forcing(d, source_per_day, exchange_per_day, equilibrium_kind, temperature_k, nm, forcing_target,
+                      forcing_column, forcing_values, n_time)
     if source_per_day is None and exchange_per_day is None:
         return
     if exchange_per_day is not None and equilibrium is None:
@@ -274,18 +307,93 @@ def _validate_depth(d, source_per_day, exchange_per_day, nm, decay_per_depth, so
                          f"cell {i} has {a[i]}")
 
 
+def _validate_forcing(d, source_per_day, exchange_per_day, equilibrium_kind, temperature_k, nm, target, column, values,
+                      n_time) -> None:
+    if target is None:
+        return
+    tg, col = np.asarray(target).reshape(-1), np.asarray(column).reshape(-1)
+    v = np.asarray(values, np.float64)
+    n, K = len(tg), d.shape[0]
+    if len(col) != n or v.ndim != 2 or v.shape[0] != n:
+        raise ValueError(f"forcing: {n} targets need {n} columns and ({n}, n_time) values, got {len(col)} and {v.shape}")
+    if n_time is not None and n > 0 and v.shape[1] != n_time:
+        raise ValueError(f"forcing: a series has {v.shape[1]} values, the model {n_time} time indices")
+    zero = np.zeros(K)
+    rates = {FORCE_DECAY_SCALE: ("decay", d),
+             FORCE_SOURCE_SCALE: ("source", zero if source_per_day is None else np.asarray(source_per_day, np.float64)),
+             FORCE_EXCHANGE_SCALE: ("exchange", zero if exchange_per_day is None else np.asarray(exchange_per_day, np.float64))}
+    kind = np.zeros(K, np.int64) if equilibrium_kind is None else np.asarray(equilibrium_kind)
+    seen = set()
+    for i in range(n):
+        g, k = int(tg[i]), int(col[i])
+        if not 0 <= g < len(_FORCE_NAMES):
+            raise ValueError(f"forcing: unknown target {g} (expected 0..{len(_FORCE_NAMES) - 1})")
+        if g == FORCE_TEMPERATURE:
+            if k != -1:
+                raise ValueError(f"forcing: the temperature series takes column -1, got {k}")
+            if temperature_k >= 0:
+                raise ValueError(f"the temperature series replaces a constant temperature, but {nm(temperature_k)} is "
+                                 "the temperature constituent")
+            what = "the temperature series"
+        elif not 0 <= k < K:
+            raise ValueError(f"forcing: {_FORCE_NAMES[g]} column index {k} out of range")
+        else:
+            what = f"{_FORCE_NAMES[g]} of {nm(k)}"
+        if (g, k) in seen:
+            raise ValueError(f"{what} given twice")
+        seen.add((g, k))
+        bad = ~np.isfinite(v[i])
+        if bad.any():
+            t = int(np.argmax(bad))
+            raise ValueError(f"{what} must be finite; time index {t} has {v[i, t]}")
+        if g in rates:
+            neg = v[i] < 0
+            if neg.any():
+                t = int(np.argmax(neg))
+                raise ValueError(f"{what} must be >= 0; time index {t} has {v[i, t]}")
+            process, r = rates[g]
+            if r[k] == 0:
+                raise ValueError(f"{what}: its {process} rate is 0")
+        if g == FORCE_EQUILIBRIUM:
+            if rates[FORCE_EXCHANGE_SCALE][1][k] == 0:
+                raise ValueError(f"{what}: {nm(k)} has no exchange")
+            if kind[k] != 0:
+                raise ValueError(f"{what}: {nm(k)} relaxes toward {OXYGEN_SATURATION}")
+
+
+def _series(value, what: str, n_time: Optional[int]) -> np.ndarray:
+    if isinstance(value, Mapping):
+        raise ValueError(f"{what}: a series given as {dict(value)!r} needs the model's datetimes; a config file reads "
+                         "{csv: path} series, elsewhere give an array")
+    a = np.asarray(value, np.float64)
+    if a.ndim != 1 or (n_time is not None and a.shape[0] != n_time):
+        raise ValueError(f"{what}: expected a series of {n_time if n_time is not None else 'n_time'} values (one per "
+                         f"model time index), got shape {a.shape}")
+    return a
+
+
+def _is_series(value) -> bool:
+    return isinstance(value, Mapping) or np.ndim(value) > 0
+
+
 def compile_kinetics(spec: Mapping[str, Mapping], constituents: Sequence[str],
-                     temperature: Union[str, float] = 20.0, *, cell_area=None, min_depth: float = DEFAULT_MIN_DEPTH,
-                     n_real: Optional[int] = None) -> Kinetics:
+                     temperature: Union[str, float, Sequence[float]] = 20.0, *, cell_area=None,
+                     min_depth: float = DEFAULT_MIN_DEPTH, n_real: Optional[int] = None,
+                     n_time: Optional[int] = None) -> Kinetics:
     """spec: {constituent: {"decay_per_day": float, "theta": float (default 1), "yields": {constituent: float},
     "source_per_day": float, "source_theta": float (default 1), "exchange_per_day": float, "exchange_theta": float
     (default 1), "equilibrium": float or "oxygen_saturation" (required when exchange_per_day > 0), "limited_by",
     "inhibited_by", "source_limited_by", "source_inhibited_by": {constituent: half_saturation}, "settling_per_day",
     "areal_source_per_day", "transfer_per_day": the per-depth forms of decay_per_day, source_per_day and
     exchange_per_day, each in place of its counterpart}};
-    temperature: a constituent name, or a constant in deg C; cell_area (F,) the plan areas, needed by the per-depth keys,
-    of which the first n_real (default all) are the real cells; min_depth the floor of the depth.  The factors compile per block in spec order of the blocks:
-    the limitations (decay, then source) first, then the inhibitions (decay, then source), each mapping in its order."""
+    "decay_scale", "source_scale", "exchange_scale": series of n_time scales >= 0 of those rates, and "equilibrium" also
+    as a series of n_time values}};
+    temperature: a constituent name, a constant in deg C or a series of n_time of them; cell_area (F,) the plan areas,
+    needed by the per-depth keys, of which the first n_real (default all) are the real cells; min_depth the floor of the
+    depth; n_time: the model's number of time indices, the length of every series (None: the first series' length).
+    The factors compile per block in spec order of the blocks: the limitations (decay, then source) first, then the
+    inhibitions (decay, then source), each mapping in its order.  The series compile ordered by (target, column); a
+    constant the series replaces (temperature_c, the equilibrium) is set to the series' first value."""
     names = list(constituents)
     index = {n: k for k, n in enumerate(names)}
     K = len(names)
@@ -294,6 +402,15 @@ def compile_kinetics(spec: Mapping[str, Mapping], constituents: Sequence[str],
     equilibrium, kind = np.zeros(K), np.zeros(K, np.int32)
     factors = []                     # (process, column, factor column, kind, half-saturation)
     per_depth = {key: np.zeros(K, np.int32) for key in _DEPTH_KEYS}
+    series = {}                      # (target, column) -> values
+
+    def add_series(target, column, value, what):
+        nonlocal n_time
+        a = _series(value, what, n_time)
+        n_time = a.shape[0] if n_time is None else n_time
+        series[(target, column)] = a
+        return a
+
     for name, block in spec.items():
         if name not in index:
             raise ValueError(f"kinetics given for {name!r}, which is not a constituent of the model")
@@ -320,8 +437,14 @@ def compile_kinetics(spec: Mapping[str, Mapping], constituents: Sequence[str],
         source_theta[k] = float(block.get("source_theta", 1.0))
         exchange[k] = float(block.get("exchange_per_day", 0.0))
         exchange_theta[k] = float(block.get("exchange_theta", 1.0))
+        for key, target in _SCALE_KEYS.items():
+            if key in block:
+                add_series(target, k, block[key], f"{key} of {name!r}")
         eq = block.get("equilibrium")
-        if isinstance(eq, str):
+        if eq is not None and not isinstance(eq, str) and _is_series(eq):
+            a = add_series(FORCE_EQUILIBRIUM, k, eq, f"equilibrium of {name!r}")
+            equilibrium[k] = a[0] if len(a) else 0.0
+        elif isinstance(eq, str):
             if eq != OXYGEN_SATURATION:
                 raise ValueError(f"kinetics of {name!r}: equilibrium must be a number or {OXYGEN_SATURATION!r}, got {eq!r}")
             kind[k] = 1
@@ -342,8 +465,16 @@ def compile_kinetics(spec: Mapping[str, Mapping], constituents: Sequence[str],
         if temperature not in index:
             raise ValueError(f"temperature constituent {temperature!r} is not a constituent of the model")
         temperature_k, temperature_c = index[temperature], 20.0
+    elif _is_series(temperature):
+        a = add_series(FORCE_TEMPERATURE, -1, temperature, "temperature")
+        temperature_k, temperature_c = -1, float(a[0]) if len(a) else 20.0
     else:
         temperature_k, temperature_c = -1, float(temperature)
+    force = [None] * 3
+    if series:
+        keys = sorted(series)
+        force = [np.array([g for g, _ in keys], np.int32), np.array([k for _, k in keys], np.int32),
+                 np.stack([series[key] for key in keys])]
     lim = [None] * 5
     if factors:
         cols = list(zip(*factors))
@@ -356,6 +487,26 @@ def compile_kinetics(spec: Mapping[str, Mapping], constituents: Sequence[str],
              exchange_per_day=exchange, exchange_theta=exchange_theta, equilibrium=equilibrium, equilibrium_kind=kind,
              limit_process=lim[0], limit_column=lim[1], limit_factor_column=lim[2], limit_kind=lim[3],
              limit_half_saturation=lim[4], decay_per_depth=depth[0], source_per_depth=depth[1],
-             exchange_per_depth=depth[2], cell_area=None if area is None else area[:n_real], min_depth=float(min_depth))
+             exchange_per_depth=depth[2], cell_area=None if area is None else area[:n_real], min_depth=float(min_depth),
+             forcing_target=force[0], forcing_column=force[1], forcing_values=force[2], n_time=n_time)
     return Kinetics(decay, theta, yields, temperature_k, temperature_c, topological_order(yields), source, source_theta,
-                    exchange, exchange_theta, equilibrium, kind, *lim, *depth, area, float(min_depth))
+                    exchange, exchange_theta, equilibrium, kind, *lim, *depth, area, float(min_depth), *force)
+
+
+def read_csv_series(spec: Optional[Mapping[str, Mapping]], temperature, time):
+    """(spec, temperature) with every series given as {"csv": path} -- a spec key of SERIES_KEYS or the temperature --
+    replaced by the file's `Value` column put onto the model datetimes `time` as the boundary conditions are
+    (io.ras.series_on_model_times).  Everything else is returned as given."""
+    from .io.ras import read_series_csv
+
+    def load(value, what):
+        if not isinstance(value, Mapping):
+            return value
+        if set(value) != {"csv"}:
+            raise ValueError(f"{what}: a series in a file is given as {{csv: path}}, got keys {sorted(value)}")
+        return read_series_csv(value["csv"], time)
+
+    if spec is not None:
+        spec = {name: ({key: load(v, f"{key} of {name!r}") if key in SERIES_KEYS else v for key, v in block.items()}
+                       if isinstance(block, Mapping) else block) for name, block in spec.items()}
+    return spec, load(temperature, "temperature")

@@ -415,3 +415,50 @@ def make_kinetics_depth(kin: dict, src: Optional[dict] = None, *, seed: int = 0,
     if src is not None:
         src = dict(src, source_per_day=source, exchange_per_day=exchange)
     return kin, src, flags
+
+
+def diurnal_light(time_seconds, *, period: float = 86400.0, phase: float = 0.0) -> np.ndarray:
+    """Relative light I(t) / I_max in [0, 1]: a sine clipped at zero, so dark half of every `period` (seconds), brightest
+    a quarter period after the sun rises at time `phase`."""
+    t = np.asarray(time_seconds, np.float64)
+    return np.maximum(np.sin(2.0 * np.pi * (t - phase) / period), 0.0)
+
+
+def make_kinetics_forcing(kin: dict, src: Optional[dict], time_seconds, *, seed: int = 0, period: float = 86400.0) -> dict:
+    """Seeded diurnal forcing for a network of make_kinetics (kin) and make_kinetics_sources (src, or None) over the model
+    times time_seconds (T,), in the manner of a river on a sunny day with a `period`-second cycle: light L(t)
+    (diurnal_light, a seeded sunrise) drives the positive sources (photosynthesis-like, source scale L) and the decay of
+    every reacting k = 2 mod 3 (solar die-off, scale (k_dark + a L) / (k_dark + a) with k_dark / a in 0.1..1); every
+    exchange rate follows a seeded wind factor in 0.5..1.5; every constant equilibrium swings by +-20 % (equilibrium
+    temperature-like, lagging the light); at a constant temperature the temperature swings by 2..5 deg C around it.
+    Returns a dict of TransportBackend.set_kinetics_forcing arguments (target, column, values (n, T))."""
+    rng = np.random.default_rng(seed + 198491317)
+    t = np.asarray(time_seconds, np.float64)
+    light = diurnal_light(t, period=period, phase=period * rng.uniform(0.15, 0.35))
+    decay = np.asarray(kin["decay_per_day"], np.float64)
+    K = len(decay)
+    zero = np.zeros(K)
+    source = np.asarray(zero if src is None or src.get("source_per_day") is None else src["source_per_day"], np.float64)
+    exchange = np.asarray(zero if src is None or src.get("exchange_per_day") is None else src["exchange_per_day"], np.float64)
+    kind = np.zeros(K, np.int32) if src is None or src.get("equilibrium_kind") is None else np.asarray(src["equilibrium_kind"])
+    equilibrium = zero if src is None or src.get("equilibrium") is None else np.asarray(src["equilibrium"], np.float64)
+    rows = []                                    # (target, column, values)
+    if kin["temperature_k"] < 0:
+        swing = 2.0 + 3.0 * rng.random()
+        rows.append((0, -1, kin["temperature_c"] + swing * np.sin(2.0 * np.pi * (t / period - 0.4))))
+    for k in range(K):
+        if exchange[k] > 0 and kind[k] == 0:
+            rows.append((1, k, equilibrium[k] * (1.0 + 0.2 * np.sin(2.0 * np.pi * (t / period - 0.45)))))
+    for k in range(K):
+        if decay[k] > 0 and k % 3 == 2:
+            dark = 0.1 + 0.9 * rng.random()
+            rows.append((2, k, (dark + light) / (dark + 1.0)))
+    for k in range(K):
+        if source[k] > 0:
+            rows.append((3, k, light.copy()))
+    for k in range(K):
+        if exchange[k] > 0:
+            rows.append((4, k, 1.0 + 0.5 * np.sin(2.0 * np.pi * (t / period * rng.uniform(1.0, 3.0) + rng.random()))))
+    cols = list(zip(*rows)) if rows else [(), (), ()]
+    return dict(target=np.array(cols[0], np.int32), column=np.array(cols[1], np.int32),
+                values=np.array(cols[2], np.float64).reshape(len(rows), len(t)))

@@ -122,6 +122,9 @@ class ClearwaterRiverine:
         if not flow_field_file_path or not isinstance(constituent_dict, dict):
             raise TypeError("Missing a `config_filepath` or a `constituent_dict` and `flow_field_file_path` to run the model.")
         plan = ras.read_ras_plan(flow_field_file_path, datetime_range)
+        if kinetics is not None or temperature is not None:       # series given as {csv: path}, onto the model times
+            from .kinetics import read_csv_series
+            kinetics, temperature = read_csv_series(kinetics, temperature, plan.time)
         if verbose:
             print("Populating Model Mesh...")
         inputs, units = {}, {}
@@ -294,8 +297,9 @@ class ClearwaterRiverine:
         transport: first-order decay and yields, then zero-order sources and relaxation toward an equilibrium such as
         reaeration toward oxygen saturation, each optionally scaled by Monod limitation and inhibition factors such as
         oxygen limitation of BOD oxidation, and processes given per unit depth such as settling, areal sediment oxygen
-        demand or a surface transfer velocity, which act through each cell's depth V / cell_area (kinetics.py: spec format;
-        temperature is a constituent name or a constant in deg C).  None switches kinetics off.  History rows are not
+        demand or a surface transfer velocity, which act through each cell's depth V / cell_area, and series of one value
+        per time index that scale a rate or replace an equilibrium, such as light on photosynthesis or wind on reaeration
+        (kinetics.py: spec format; temperature is a constituent name, a constant in deg C or a series of them).  None switches kinetics off.  History rows are not
         rewritten: the reaction of step t shows in row t + 1."""
         from .kinetics import compile_kinetics
         if spec is None:
@@ -303,7 +307,7 @@ class ClearwaterRiverine:
             self.kinetics = None
             return
         kin = compile_kinetics(spec, self.constituents, temperature, cell_area=self.cell_area, min_depth=self.min_depth,
-                               n_real=self.mesh.attrs[NUMBER_OF_REAL_CELLS] + 1)
+                               n_real=self.mesh.attrs[NUMBER_OF_REAL_CELLS] + 1, n_time=len(self.mesh["time"]))
         self.backend.set_kinetics(kin.decay_per_day, kin.theta, kin.yields, kin.temperature_k, kin.temperature_c)
         if kin.has_sources:
             self.backend.set_kinetics_sources(**kin.sources_arguments())
@@ -311,6 +315,8 @@ class ClearwaterRiverine:
             self.backend.set_kinetics_limits(**kin.limits_arguments())
         if kin.has_depth:
             self.backend.set_kinetics_depth(**kin.depth_arguments())
+        if kin.has_forcing:
+            self.backend.set_kinetics_forcing(**kin.forcing_arguments())
         self.kinetics = kin
 
     def sync(self):

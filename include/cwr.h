@@ -293,6 +293,34 @@ int cwr_set_kinetics_limits(cwr_handle* h, int n, const int* process, const int*
  * same call. */
 int cwr_set_kinetics_depth(cwr_handle* h, const double* cell_area, double min_depth, const int* decay_per_depth,
                            const int* source_per_depth, const int* exchange_per_depth);
+/* Time-varying forcing of the kinetics and sources set last (see above): n series of n_time values each, values (n,
+ * n_time) row-major, one per model time index; step t uses entry t (the index of vol[t] and dt[t]), held over the step.
+ * Series i has target[i] and column[i]:
+ *     CWR_FORCE_TEMPERATURE     column -1: replaces temperature_c (only while temperature_k == -1); O2sat(T) follows it
+ *     CWR_FORCE_EQUILIBRIUM     replaces the constant equilibrium of column k (exchange > 0, equilibrium kind 0)
+ *     CWR_FORCE_DECAY_SCALE     multiplies the decay rate of column k
+ *     CWR_FORCE_SOURCE_SCALE    multiplies the source of column k
+ *     CWR_FORCE_EXCHANGE_SCALE  multiplies the exchange rate of column k
+ * A scale f multiplies the per-day rate (rate * f[t] in fp64) before anything else acts on it: the theta^(T - 20)
+ * correction, the depth, the Monod factors and the cap, the exact per-step solutions.  A scale of 1, or a series equal to
+ * the constant it replaces, gives the bits of the unforced step.  Scales are >= 0, so a sink stays a sink and the
+ * non-negativity guarantee above holds; under an equilibrium series it holds where the series is >= 0 (not checked).
+ * n == 0 = forcing off.  Acts only while kinetics is set; cwr_set_kinetics and cwr_set_kinetics_sources clear it; it,
+ * cwr_set_kinetics_limits and cwr_set_kinetics_depth do not clear each other.  Stream-ordered upload.  CWR_EINVAL when
+ * kinetics is not set, for n < 0, n_time other than the handle's, a NULL array with n > 0, an unknown target, a column
+ * out of range or a temperature series with a column other than -1, the same (target, column) twice, a non-finite
+ * value, a negative scale, a scale on a process whose rate is 0, a temperature series while a temperature constituent
+ * is set, or an equilibrium series on a column without exchange or one that relaxes toward O2sat.  The reaction mass
+ * includes the forced rates.  Domain decomposition: every rank makes the same call. */
+enum {
+    CWR_FORCE_TEMPERATURE = 0,
+    CWR_FORCE_EQUILIBRIUM = 1,
+    CWR_FORCE_DECAY_SCALE = 2,
+    CWR_FORCE_SOURCE_SCALE = 3,
+    CWR_FORCE_EXCHANGE_SCALE = 4
+};
+int cwr_set_kinetics_forcing(cwr_handle* h, int n, int n_time, const int* target, const int* column,
+                             const double* values);
 /* Reaction mass of constituent k, sum over the steps taken of sum_i V[t]_i (c~'_ik - c~_ik), reduced on the device in a fixed
  * order (the same bits every run): a running sum since cwr_create, 0 while kinetics was never set.  Domain decomposition:
  * the partial sum over the rows the rank owns (as cwr_mass_totals_at). */

@@ -10,8 +10,9 @@ tests/test_gpu_parity.py) and (b) a single-GPU run of the same library on rank 0
 boundary flux sums are checked as sums of the per-rank partial values.  --kinetics: the same with a first-order
 network (synthetic.make_kinetics) reacted on the device, in every other case with sources and exchange as well
 (synthetic.make_kinetics_sources), in every fourth with Monod factors (synthetic.make_kinetics_limits) and, in the cases
-with sources 1 and 3 mod 4, with depth-scaled processes over the plan areas (synthetic.make_kinetics_depth), the oracle
-being oracle.kinetics_depth.KineticsRiverine, and the ranks' reaction masses summed against the single-GPU ones.  Prints one JSON line per case on
+with sources 1 and 3 mod 4, with depth-scaled processes over the plan areas (synthetic.make_kinetics_depth) and, in every
+case with sources, with time-varying forcing (synthetic.make_kinetics_forcing), the oracle being
+oracle.kinetics_forcing.KineticsRiverine, and the ranks' reaction masses summed against the single-GPU ones.  Prints one JSON line per case on
 rank 0; exit code 0 only if every check passed on every rank.
 """
 from __future__ import annotations
@@ -43,7 +44,8 @@ def main():
     from clearwater_riverine_b200 import TransportBackend, synthetic
     from clearwater_riverine_b200.domain import DomainDecomposedBackend, merge_owned
     from oracle import reference_step as ref
-    from oracle.kinetics_depth import KineticsRiverine, depth_terms
+    from oracle.kinetics_depth import depth_terms
+    from oracle.kinetics_forcing import KineticsRiverine, forcing_terms
     from oracle.kinetics_limits import limit_terms
 
     rank, world, local = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"]), int(os.environ["LOCAL_RANK"])
@@ -62,7 +64,7 @@ def main():
         adv, _, _, cdiff, dt = ref.derive_coefficients(plan.face_flow, plan.edge_velocity, plan.face_x, plan.face_y,
                                                        plan.f1, plan.f2, D, plan.time_seconds)
         inputs = synthetic.make_inputs(plan, K, seed=40 + ci)
-        kin = src = lim = dep = None
+        kin = src = lim = dep = frc = None
         if args.kinetics:
             inputs, kin = synthetic.make_kinetics(inputs, seed=40 + ci)
             if ci % 2:
@@ -72,6 +74,8 @@ def main():
             if ci % 2 and ci < 4:
                 kin, src, flags = synthetic.make_kinetics_depth(kin, src, seed=40 + ci)
                 dep = dict(cell_area=plan.cell_area, min_depth=0.05, **flags)
+            if ci % 2:
+                frc = synthetic.make_kinetics_forcing(kin, src, plan.time_seconds, seed=40 + ci, period=6 * 30.0)
         be = DomainDecomposedBackend(plan.f1, plan.f2, plan.n_face, T, K, D, rank, world, device=local, **opts)
         be.set_hydro(0, adv, cdiff, plan.edge_velocity, plan.volume, dt)
         info = be.attach()
@@ -85,6 +89,8 @@ def main():
             be.set_kinetics_limits(**lim)
         if dep is not None:
             be.set_kinetics_depth(**dep)
+        if frc is not None:
+            be.set_kinetics_forcing(**frc)
         single = oracle = None
         if rank == 0:
             single = TransportBackend(plan.f1, plan.f2, plan.n_face, T, K, D, device=local, solver_path=1,
@@ -100,6 +106,8 @@ def main():
                 single.set_kinetics_limits(**lim)
             if dep is not None:
                 single.set_kinetics_depth(**dep)
+            if frc is not None:
+                single.set_kinetics_forcing(**frc)
             if not args.no_oracle:
                 mesh = ref.HydroMesh(plan.f1, plan.f2, plan.n_face, adv, cdiff, plan.edge_velocity, plan.volume, dt, D)
                 named = {f"c{k}": inputs[k] for k in range(K)}
@@ -108,7 +116,8 @@ def main():
                 else:
                     temperature = f"c{kin['temperature_k']}" if kin["temperature_k"] >= 0 else kin["temperature_c"]
                     oracle = KineticsRiverine(mesh, named, kin["decay_per_day"], kin["theta"], kin["yields"], temperature,
-                                              **(src or {}), **limit_terms(**(lim or {})), **depth_terms(**(dep or {})))
+                                              **(src or {}), **limit_terms(**(lim or {})), **depth_terms(**(dep or {})),
+                                              **forcing_terms(**(frc or {})))
         worst_oracle = worst_single = 0.0
         iters = []
         status = 0
@@ -154,6 +163,7 @@ def main():
                 line["sources"] = src is not None
                 line["limits"] = lim is not None
                 line["depth"] = dep is not None
+                line["forcing"] = frc is not None
             single.close()
         flag = torch.tensor([1 if ok else 0], device="cuda")
         dist.all_reduce(flag, op=dist.ReduceOp.MIN)

@@ -21,6 +21,10 @@ temperature constituent and at a constant temperature (--limits-only: this leg a
 With depth-scaled processes (cwr_set_kinetics_depth), 1M x 16: the network with its sources and the flags of
 synthetic.make_kinetics_depth over the plan areas against the same network without the flags, alternately on the same
 handle, with the temperature constituent and at a constant temperature (--depth-only: this leg alone).
+With time-varying forcing (cwr_set_kinetics_forcing), 1M x 16: the network with its sources and the diurnal series of
+synthetic.make_kinetics_forcing (light-scaled sources and die-off, wind-scaled exchange, moving equilibria and, at a
+constant temperature, a temperature series) against the same network unforced, alternately on the same handle, with the
+temperature constituent and at a constant temperature (--forcing-only: this leg alone).
 --parent-root DIR: the kinetics-only, the sources-only and the sources-with-factors network timed in this tree's build
 and in DIR's (another checkout with its library built), one process per measurement, alternating, --parent-rounds times each; every process also reports the spread of
 its own repetitions.
@@ -220,6 +224,61 @@ def depth_leg(torch, res, reps, scale):
     be.close()
 
 
+def alternate_forcing(torch, be, kin, src, frc, step, reps):
+    """The network with its sources, unforced and forced, alternately, reps times each: medians and ranges of the step
+    time (ms, CUDA events) and of the CWR_FAM_RHS family time (ms per step, in separate profiled steps)."""
+    out = {"step_ms": ([], []), "rhs_family_ms": ([], [])}
+    for _ in range(reps):
+        for i, forced in enumerate((False, True)):
+            be.set_kinetics(**kin)
+            be.set_kinetics_sources(**src)
+            if forced:
+                be.set_kinetics_forcing(**frc)
+            step()
+            out["step_ms"][i].append(timed(torch, be, step, 5))
+            be.profile(1)
+            for _ in range(5):
+                step()
+            out["rhs_family_ms"][i].append(be.profile(-1)["rhs"][0] / 5)
+            be.profile(0)
+    res = {}
+    for key, v in out.items():
+        for i, name in enumerate(("unforced", "forced")):
+            res[f"{key}_{name}"] = float(np.median(v[i]))
+            res[f"{key}_{name}_range"] = [float(min(v[i])), float(max(v[i]))]
+    return res
+
+
+def forcing_leg(torch, res, reps, scale):
+    """1M x 16 with sources: unforced and forced, with the temperature constituent and at a constant one."""
+    import bench
+    from clearwater_riverine_b200 import synthetic
+    plan, K = bench.workload_plan("1m16", 14, seed=0, scale=scale)
+    inputs, kin = synthetic.make_kinetics(synthetic.make_inputs(plan, K, seed=0), seed=0, decay_range=(0.05, 2.0))
+    src = synthetic.make_kinetics_sources(kin, seed=0, rate_range=(0.05, 2.0))
+    be = build(plan, inputs, torch)
+    for t in range(3):
+        be.step(t)
+    step = lambda: be.step(3)
+    be.profile(1)
+    for _ in range(10):
+        step()
+    fam_off = be.profile(-1)["rhs"][0] / 10
+    be.profile(0)
+    kin_const = dict(kin, temperature_k=-1, temperature_c=24.0)
+    for key, k in (("1m16_forcing", kin), ("1m16_forcing_constant_temperature", kin_const)):
+        frc = synthetic.make_kinetics_forcing(k, src, plan.time_seconds, seed=0)
+        r = alternate_forcing(torch, be, k, src, frc, step, reps)
+        r["k_react_ms_unforced"] = r["rhs_family_ms_unforced"] - fam_off
+        r["k_react_ms_forced"] = r["rhs_family_ms_forced"] - fam_off
+        r["k_react_added_ms"] = r["rhs_family_ms_forced"] - r["rhs_family_ms_unforced"]
+        r["step_added_ms"] = r["step_ms_forced"] - r["step_ms_unforced"]
+        r["series_per_target"] = {name: int(np.sum(frc["target"] == g)) for g, name in
+                                  enumerate(("temperature", "equilibrium", "decay_scale", "source_scale", "exchange_scale"))}
+        res[key] = r
+    be.close()
+
+
 def regression_child(reps, scale):
     """One process of --parent-root: kinetics off, the kinetics-only, the sources-only and the sources-with-factors 1M x 16
     network (temperature constituent) on one handle; medians and spreads (min, max) of the step time and of k_react's time (CWR_FAM_RHS
@@ -322,6 +381,7 @@ def main():
     ap.add_argument("--out", default=None)
     ap.add_argument("--limits-only", action="store_true", help="only the Monod-factor leg (and --parent-root)")
     ap.add_argument("--depth-only", action="store_true", help="only the depth leg (and --parent-root)")
+    ap.add_argument("--forcing-only", action="store_true", help="only the forcing leg (and --parent-root)")
     ap.add_argument("--parent-root", default=None,
                     help="another checkout with its library built: the no-factor networks timed in both builds, alternately")
     ap.add_argument("--parent-rounds", type=int, default=3)
@@ -337,8 +397,9 @@ def main():
     if not torch.cuda.is_available():
         raise SystemExit("kinetics_bench needs a CUDA device")
     res = {"gpu": gpu_name_and_power()}
-    if args.limits_only or args.depth_only:
-        (limits_leg if args.limits_only else depth_leg)(torch, res, args.reps, args.scale)
+    if args.limits_only or args.depth_only or args.forcing_only:
+        leg = limits_leg if args.limits_only else depth_leg if args.depth_only else forcing_leg
+        leg(torch, res, args.reps, args.scale)
         if args.parent_root:
             res["no_factor_paths_vs_parent"] = parent_comparison(args.parent_root, args.parent_rounds, max(3, args.reps // 3),
                                                                  args.scale)
@@ -415,6 +476,7 @@ def main():
         be.close()
     limits_leg(torch, res, args.reps, args.scale)
     depth_leg(torch, res, args.reps, args.scale)
+    forcing_leg(torch, res, args.reps, args.scale)
     if args.parent_root:
         res["no_factor_paths_vs_parent"] = parent_comparison(args.parent_root, args.parent_rounds, max(3, args.reps // 3),
                                                              args.scale)
