@@ -75,17 +75,25 @@ def test_1m_x16_against_the_oracles_own_matrix_and_right_hand_sides():
     solve would take ~50 s per column): (1) the GPU's LHS and RHS equal the oracle's; (2) the TRUE residual of every GPU
     column, formed with the ORACLE's A and b, is below 1e-12 ||b||; (3) one column equals an independent CPU solve of the
     oracle's system (scipy BiCGSTAB + Jacobi to 1e-13) within rtol 1e-9."""
+    import bench
+    plan, K = bench.workload_plan("1m16", 3, seed=2)
+    assert plan.n_real == 1_000_000 and K == 16
+    check_against_the_oracles_system(plan, K)
+
+
+def check_against_the_oracles_system(plan, K, **want_options):
+    """Two steps of plan (3 time slices, K constituents) at default options with the flow hint and raw hydrodynamics, as
+    bench.py runs them, checked after the second step against the oracle's own A and b (see the test above).
+    want_options: options the backend must have resolved to (the path the caller wrote its case for)."""
     import scipy.sparse as sp
     import scipy.sparse.linalg as spla
-    import bench
     from clearwater_riverine_b200 import TransportBackend, synthetic
-    T = 3
-    plan, K = bench.workload_plan("1m16", T, seed=2)
-    n = plan.n_real
-    assert n == 1_000_000 and K == 16
+    T = plan.n_time
     inputs = synthetic.make_inputs(plan, K, seed=2)
     mesh = _oracle_mesh(plan)
     be = TransportBackend(plan.f1, plan.f2, plan.n_face, T, K, D, flow_hint=plan.face_flow.mean(axis=0))
+    for key, val in want_options.items():
+        assert getattr(be.options, key) == val, (key, getattr(be.options, key), val)
     be.set_geometry(plan.face_x, plan.face_y)
     be.set_hydro_raw(0, plan.face_flow, plan.edge_velocity, plan.volume, mesh.dt)
     for k in range(K):
@@ -164,20 +172,25 @@ def test_device_mass_balance_matches_the_oracles(case):
     faces = {str(nm): np.array([f]) for nm, f in zip(g["bc_names"], g["bc_faces"])}
     for c in names:
         want = ref.mass_balance(mesh, g[f"conc_{c}"], g[f"totflux_{c}"], g["face_flow"], faces)
-        got = model.mass_balance(c, faces)
-        assert abs(got["Mass_end"] - want["Mass_end"]) <= 1e-9 * abs(want["Mass_end"])
-        assert abs(got["Mass_start"] - want["Mass_start"]) <= 1e-12 * abs(want["Mass_start"])
-        assert abs(got["Vol_end"] - want["Vol_end"]) <= 1e-6 * abs(want["Vol_end"])          # (the oracle sums float32 volumes)
-        scale_m = max(abs(want["bcTotalMassInAll"]), abs(want["bcTotalMassOutAll"]), 1e-300)
-        scale_v = max(abs(want["bcTotalVolInAll"]), abs(want["bcTotalVolOutAll"]), 1e-300)
-        for key, w in want.items():
-            if key in ("Vol_start", "Vol_end", "Mass_start", "Mass_end", "error_vol", "vol_end_calc"):
-                continue
-            tol = 1e-9 * (scale_v if "vol" in key.lower() else scale_m)
-            if key in ("mass_end_calc", "error_mass"):
-                tol = 1e-9 * max(scale_m, abs(want["Mass_start"]))
-            assert abs(got[key] - w) <= tol, (c, key, got[key], w)
+        mass_balance_close(model.mass_balance(c, faces), want, c)
     model.finalize()
+
+
+def mass_balance_close(got, want, what):
+    """ClearwaterRiverine.mass_balance() against ref.mass_balance: Mass_end within 1e-9 relative, the boundary sums within
+    1e-9 of the largest boundary total."""
+    assert abs(got["Mass_end"] - want["Mass_end"]) <= 1e-9 * abs(want["Mass_end"])
+    assert abs(got["Mass_start"] - want["Mass_start"]) <= 1e-12 * abs(want["Mass_start"])
+    assert abs(got["Vol_end"] - want["Vol_end"]) <= 1e-6 * abs(want["Vol_end"])          # (the oracle sums float32 volumes)
+    scale_m = max(abs(want["bcTotalMassInAll"]), abs(want["bcTotalMassOutAll"]), 1e-300)
+    scale_v = max(abs(want["bcTotalVolInAll"]), abs(want["bcTotalVolOutAll"]), 1e-300)
+    for key, w in want.items():
+        if key in ("Vol_start", "Vol_end", "Mass_start", "Mass_end", "error_vol", "vol_end_calc"):
+            continue
+        tol = 1e-9 * (scale_v if "vol" in key.lower() else scale_m)
+        if key in ("mass_end_calc", "error_mass"):
+            tol = 1e-9 * max(scale_m, abs(want["Mass_start"]))
+        assert abs(got[key] - w) <= tol, (what, key, got[key], w)
 
 
 class _Var:

@@ -5,15 +5,35 @@ import pytest
 
 from clearwater_riverine_b200 import synthetic
 from clearwater_riverine_b200.backend import order_cells
+from tests.polygon_mesh import merge_cells, row_lengths
 
 
 def colours_of(new_of_old, color_ptr):
     return np.searchsorted(color_ptr, new_of_old, side="right") - 1
 
 
-@pytest.mark.parametrize("n_colors,hinted", [(0, False), (5, False), (8, True), (16, True), (64, True)])
-def test_order_is_a_permutation_and_colours_separate_neighbours(n_colors, hinted):
-    plan = synthetic.make_plan(37, 23, 6, tri_fraction=0.2, dry_fraction=0.02, seed=3)
+def _quads():
+    return synthetic.make_plan(37, 23, 6, tri_fraction=0.2, dry_fraction=0.02, seed=3)
+
+
+def _polygons(sizes, n_groups):
+    """The quad plan with groups of cells merged into polygons: rows of up to 8 (sizes 2, 3) or 10 (with 4) neighbours."""
+    return lambda: merge_cells(_quads(), sizes, n_groups, seed=3)
+
+
+_ORDER_CASES = [(_quads, nc, h) for nc, h in [(0, False), (5, False), (8, True), (16, True), (64, True)]]
+_ORDER_IDS = [f"{nc}-{h}" for _, nc, h in _ORDER_CASES]
+for _name, _factory in (("w8", _polygons((2, 3), 80)), ("w12", _polygons((2, 4), 70))):
+    for _nc, _h in [(0, False), (5, False), (8, True), (16, True)]:
+        _ORDER_CASES.append((_factory, _nc, _h))
+        _ORDER_IDS.append(f"{_name}-{_nc}-{_h}")
+
+
+@pytest.mark.parametrize("make_plan,n_colors,hinted", _ORDER_CASES, ids=_ORDER_IDS)
+def test_order_is_a_permutation_and_colours_separate_neighbours(make_plan, n_colors, hinted):
+    """Quad / triangle meshes and polygon meshes (ELL widths 8 and 12): a colour request below the largest degree + 1
+    is raised to it."""
+    plan = make_plan()
     n = plan.n_real
     hint = plan.face_flow.mean(0) if hinted else None
     p, cptr, n_levels = order_cells(plan.f1, plan.f2, plan.n_face, True, n_colors, hint)
@@ -22,7 +42,7 @@ def test_order_is_a_permutation_and_colours_separate_neighbours(n_colors, hinted
     if n_colors == 0:
         assert len(cptr) == 2
         return
-    assert len(cptr) - 1 >= min(n_colors, 5)
+    assert len(cptr) - 1 >= max(min(n_colors, 64), int(row_lengths(plan).max()) + 1)
     col = colours_of(p, cptr)
     internal = plan.f2 < n
     assert np.all(col[plan.f1[internal]] != col[plan.f2[internal]]), "coupled rows share a colour"

@@ -8,19 +8,36 @@ import scipy.sparse as sp
 
 from clearwater_riverine_b200 import synthetic
 from clearwater_riverine_b200.backend import strip_layout
+from tests.polygon_mesh import merge_cells, row_lengths
 
 
 def _plan(seed=3):
     return synthetic.make_plan(37, 29, 6, tri_fraction=0.2, dry_fraction=0.02, seed=seed)
 
 
-@pytest.mark.parametrize("n_parts,n_strips,n_colors", [(1, 1, 8), (1, 7, 8), (1, 24, 12), (2, 5, 9), (4, 3, 8)])
-def test_strips_partition_the_rows_and_list_their_neighbours(n_parts, n_strips, n_colors):
-    plan = _plan()
+def _polygons(sizes, n_groups):
+    """_plan() with groups of cells merged into polygons: rows of up to 8 (sizes 2, 3) or 10 (with 4) neighbours."""
+    return lambda: merge_cells(_plan(), sizes, n_groups, seed=4)
+
+
+_STRIP_CASES = [(_plan, *c) for c in [(1, 1, 8), (1, 7, 8), (1, 24, 12), (2, 5, 9), (4, 3, 8)]]
+_STRIP_IDS = ["-".join(map(str, c[1:])) for c in _STRIP_CASES]
+for _name, _factory in (("w8", _polygons((2, 3), 90)), ("w12", _polygons((2, 4), 80))):
+    for _c in [(1, 7, 8), (1, 24, 5), (2, 5, 9), (4, 3, 8)]:
+        _STRIP_CASES.append((_factory, *_c))
+        _STRIP_IDS.append(_name + "-" + "-".join(map(str, _c)))
+
+
+@pytest.mark.parametrize("make_plan,n_parts,n_strips,n_colors", _STRIP_CASES, ids=_STRIP_IDS)
+def test_strips_partition_the_rows_and_list_their_neighbours(make_plan, n_parts, n_strips, n_colors):
+    """Quad / triangle meshes and polygon meshes (ELL widths 8 and 12; colour requests below the largest degree + 1 are
+    raised to it)."""
+    plan = make_plan()
     n = plan.n_real
     L = strip_layout(plan.f1, plan.f2, plan.n_face, n_colors, plan.face_flow.mean(0), n_strips, n_parts)
     p, cptr, nc = L["new_of_old"], L["strip_cptr"], L["n_colors"]
     NS = n_parts * n_strips
+    assert nc >= max(n_colors, int(row_lengths(plan).max()) + 1)
     assert np.array_equal(np.sort(p), np.arange(n))
     # strips tile [0, n) contiguously, colours tile every strip, strips have equal sizes (+-1 per part)
     assert cptr[0, 0] == 0 and cptr[-1, -1] == n
